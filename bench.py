@@ -2,6 +2,7 @@
 """bench.py -- full pdf_update + resample + opt_setting cycles per second.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c4|c1|c2|c3|c5|sweeper]
+                    [--dump-outputs DIR]
 
 Default workload c4 (BASELINE.json configs[3], fits one B200): synthetic Lorentzian cloud, 1e8 particles x
 3 parameters, 1e5 settings, n_draws = 30, resample forced every cycle (resample_threshold > 1).
@@ -18,8 +19,15 @@ Rabi on the 101 x 101 grid), c5 the 4096 batched lock-in engines.  A "step" is o
              timed on the host: c1-c3 at their full size; c4 measured at 1e6 and 1e7 particles and extrapolated
              to 1e8 with the fitted exponent (labelled).  Falls back to the numpy port (oracle/) only when the
              reference is not installed.
+  --dump-outputs DIR   (one GPU) after the timed steps, what the timed path handed its caller in its last step, as
+             DIR/<name>.npy in float64, 64 MB at most: c1-c4 the chosen setting, the utility of every setting and the
+             particles and weights at a fixed, seeded sample of at most 2^20 particles; c5 every instance's choice and
+             moments and the clouds of 8 fixed instances; sweeper the posterior moments and a sample of the cloud.
+             The inputs depend on the arguments only, so two builds run with the same arguments can be compared output
+             for output.
 """
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -64,6 +72,7 @@ class ClockSampler:
             self.proc = subprocess.Popen(['nvidia-smi', '-i', str(self.index), f'--query-gpu={self.Q}',
                                           '--format=csv,noheader,nounits', '-lms', '200'],
                                          stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.kill)         # (a no-op once stopped; ends the sampler if the run fails)
             self.thread = threading.Thread(target=self._read, daemon=True)
             self.thread.start()
         except Exception:
@@ -78,6 +87,7 @@ class ClockSampler:
             return {'sm_mhz': None, 'sm_max_mhz': None, 'reasons': ['nvidia-smi unavailable']}
         time.sleep(0.25)
         self.proc.terminate()
+        self.proc.wait()
         sm, mx, reasons = [], None, set()
         for r in self.rows:
             try:
@@ -91,6 +101,69 @@ class ClockSampler:
                 pass
         return {'sm_mhz': float(np.median(sm)) if sm else None, 'sm_max_mhz': mx, 'reasons': sorted(reasons),
                 'samples': len(sm)}
+
+
+DUMP_BYTES = 64 << 20        # --dump-outputs writes at most this much in all
+DUMP_ROW = 1 << 20           # entries of the longest dumped row; a longer one is sampled
+
+
+def _sample(n, m=DUMP_ROW):
+    """A fixed, seeded, sorted sample of m of the indices 0..n-1 (all of them when n <= m)."""
+    return np.arange(n) if n <= m else np.sort(np.random.default_rng(0).choice(n, m, replace=False))
+
+
+def _cloud_sample(eng, max_bytes):
+    """The cloud's particles and normalised weights at a fixed sample of the particle indices, within max_bytes.
+    Both are gathered on the device, and nothing of the engine's state changes (the measurements after a dump see the
+    engine the timed steps left)."""
+    import ctypes
+    import torch
+    particles = eng.particles_dev                       # (waits for an enqueued cycle)
+    m = int(min(DUMP_ROW, max_bytes // (8 * (eng.n_dims + 1))))
+    idx = torch.from_numpy(_sample(eng.n_particles, m)).to(particles.device)
+    w = torch.empty(eng.n_particles, dtype=torch.float64, device=particles.device)
+    eng._check(eng._lib.obe_normalized_weights(eng._cs(), ctypes.c_void_p(w.data_ptr()), eng._stream()))
+    return {'particles': particles[:, idx].cpu().numpy(), 'weights': w[idx].cpu().numpy()}
+
+
+def _write_dump(out_dir, arrays):
+    arrays = {name: np.asarray(a, dtype=np.float64) for name, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        raise RuntimeError(f'--dump-outputs: {total} bytes exceed the {DUMP_BYTES}-byte budget')
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
+def dump_cycle(eng, out_dir):
+    """--dump-outputs of an OptBayesExpt cycle (c1-c4): the chosen setting and its utility, the utility of every setting
+    (a fixed sample of DUMP_ROW settings when there are more) and a sample of the resampled cloud."""
+    import torch
+    best = eng.best_index_dev.cpu()
+    index = int(best[0])
+    utility = eng._utility_dev
+    out = {'chosen_index': [index], 'chosen_utility': best[1:2].view(torch.float64).numpy(),
+           'chosen_setting': eng.allsettings[:, index]}
+    if utility.numel() > DUMP_ROW:
+        cols = _sample(utility.numel())
+        out['utility_index'] = cols
+        utility = utility[torch.from_numpy(cols).to(utility.device)]
+    out['utility'] = utility.cpu().numpy()
+    out.update(_cloud_sample(eng, DUMP_BYTES - sum(8 * np.size(a) for a in out.values())))
+    _write_dump(out_dir, out)
+
+
+def dump_batched(eng, out_dir, n_instances=8):
+    """--dump-outputs of the batched cycle (c5): every instance's chosen setting, resample flag and posterior moments,
+    and the whole clouds of a fixed sample of instances."""
+    idx = eng.last_setting_index
+    inst = _sample(eng.n_instances, n_instances)
+    _write_dump(out_dir, {'chosen_index': idx, 'chosen_setting': eng.allsettings[:, idx],
+                          'just_resampled': eng.just_resampled, 'mean': eng.mean(), 'covariance': eng.covariance(),
+                          'n_eff': eng.n_eff(), 'instances': inst,
+                          'particles': np.stack([eng.particles(b) for b in inst]),
+                          'weights': np.stack([eng.particle_weights(b) for b in inst])})
 
 
 # -------------------------------------------------------------------------------------------------
@@ -243,6 +316,8 @@ def bench_small(args):
     b1.record()
     torch.cuda.synchronize()
     ms_warm = b0.elapsed_time(b1) / args.steps
+    if args.dump_outputs:
+        dump_cycle(eng, args.dump_outputs)
 
     # ---- end to end through pdf_update / opt_setting, closed loop: forced and natural resampling
     def closed_loop(threshold, steps):
@@ -365,6 +440,8 @@ def bench_c5(args, rank, world):
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / args.steps
+    if args.dump_outputs:
+        dump_batched(eng, args.dump_outputs)
     # per-phase split of the same cycle (events between the phases; outside the timed region)
     pe = [[torch.cuda.Event(enable_timing=True) for _ in range(4)] for _ in range(args.steps)]
     for t in range(args.steps):
@@ -458,6 +535,10 @@ def bench_sweeper(args):
                 times.append(time.perf_counter() - t0)
                 n_res += eng._epoch - e0
         out[mode] = (float(np.mean(times)), n_res / max(1, args.steps))
+        if args.dump_outputs and mode == 'fused':
+            # what the last timed sweep left: the posterior cloud (a sample of it) and its moments
+            _write_dump(args.dump_outputs, {'mean': eng.mean(), 'covariance': eng.covariance(),
+                                            **_cloud_sample(eng, DUMP_BYTES // 2)})
         del eng
         torch.cuda.empty_cache()
     t_f, r_f = out['fused']
@@ -562,10 +643,16 @@ def main():
                          'sweeper: the sweeper demo\'s multi-point inference (1 GPU)')
     ap.add_argument('--no-multinomial', action='store_true', help='c4: skip the like-for-like multinomial line')
     ap.add_argument('--no-invariance', action='store_true', help='multi-GPU: skip the G-invariance side check')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='one GPU: write the outputs of the last timed step to DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be >= 1 and --warmup >= 0')
     n_total = int(args.particles)
     rank = int(os.environ.get('RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
+    if args.dump_outputs and (args.impl != 'ours' or world > 1):
+        ap.error('--dump-outputs covers the GPU path on one GPU (--impl ours, no torchrun)')
     if args.impl == 'reference':
         return reference_line(args) if rank == 0 else None
     if args.workload == 'c5':
@@ -644,7 +731,7 @@ def main():
         barrier()
     settle()
     for t in range(3):
-        eng.run_cycle_async(fixed[t])
+        eng.run_cycle_async(fixed[t % len(fixed)])
     barrier()
     t_host0 = time.perf_counter()
     e_start.record()
@@ -656,6 +743,8 @@ def main():
     host_enqueue_ms = (time.perf_counter() - t_host0) * 1e3 / args.steps
     barrier()
     ms_total = e_start.elapsed_time(e_stop)
+    if args.dump_outputs:
+        dump_cycle(eng, args.dump_outputs)
     # ---------------- end to end through the reference-shaped API, closed loop -------------------
     eng.eager_select = True              # the resample inside pdf_update starts the selection opt_setting() asks for
     eng.async_update = True              # forced resampling: the decision does not need N_eff, pdf_update does not sync
@@ -721,7 +810,7 @@ def main():
     eng.early_select = False
     sv = [[torch.cuda.Event(enable_timing=True) for _ in range(5)] for _ in range(args.steps)]
     for t in range(2):
-        eng.run_cycle_async(fixed[t])
+        eng.run_cycle_async(fixed[t % len(fixed)])
     barrier()
     s_start, s_stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     s_start.record()
@@ -760,7 +849,7 @@ def main():
     if world == 1:
         n0, n1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         for t in range(3):
-            eng.run_cycle_async(fixed[t], resample=False, select=True)
+            eng.run_cycle_async(fixed[t % len(fixed)], resample=False, select=True)
         n0.record()
         for t in range(args.steps):
             eng.run_cycle_async(fixed[args.warmup + t], resample=False, select=True)
@@ -772,7 +861,7 @@ def main():
     # ---------------- the long-run figure: > 1 s of back-to-back cycles (the power cap has bitten by then) ----------
     n_sus = int(min(2000, max(50, 1.2 / (ms_step * 1e-3))))
     for t in range(3):
-        eng.run_cycle_async(fixed[t])
+        eng.run_cycle_async(fixed[t % len(fixed)])
     barrier()
     u0, u1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     u0.record()
@@ -805,7 +894,7 @@ def main():
         eng.resampling = 'multinomial_device'
         k_m = max(3, min(10, args.steps))
         for t in range(2):
-            eng.run_cycle_async(fixed[t])
+            eng.run_cycle_async(fixed[t % len(fixed)])
         m0, m1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         m0.record()
         for t in range(k_m):

@@ -1,15 +1,17 @@
 """Pin the oracle against the UNMODIFIED reference and write tests/golden/*.npz.
 
-TEST INFRASTRUCTURE.  Runs only in the build container (it needs /root/reference,
-which does not exist on the GPU box).  It imports the reference from a scratch
-copy (numba writes a cache next to the source it imports), seeds the reference's
-instance Generator (``obe.rng``, particlepdf.py:142-145) and runs each scenario
+TEST INFRASTRUCTURE.  Needs a source tree of the reference (usnistgov/optbayesexpt
+v1.2.0, given with --reference); the tests only read what it writes.  It imports
+the reference from a scratch copy (numba writes a cache next to the source it
+imports), seeds the reference's instance Generator (``obe.rng``, particlepdf.py:142-145) and runs each scenario
 in lock-step with ``oracle.obe_oracle.OracleOBE`` seeded identically.  Every
 step must agree (indices exactly, floats to 1e-12) or the script exits non-zero;
 the reference's own trajectory is what gets written to tests/golden/.
 
-    python oracle/pin_against_reference.py            # check + (re)write goldens
-    python oracle/pin_against_reference.py --check    # check only
+    python oracle/pin_against_reference.py --reference SRC            # check + (re)write goldens
+    python oracle/pin_against_reference.py --reference SRC --check    # check only
+
+What is written is cut down by shrink() so that every golden file stays well under 1 MB.
 """
 import argparse
 import os
@@ -29,10 +31,9 @@ from oracle.scenarios import SCENARIOS, build_inputs, simulate_measurement  # no
 GOLDEN = os.path.join(ROOT, 'tests', 'golden')
 
 
-def import_reference():
-    src = '/root/reference'
-    if not os.path.isdir(src):
-        raise SystemExit('reference tree not present; goldens can only be made in the build container')
+def import_reference(src):
+    if not os.path.isdir(os.path.join(src, 'optbayesexpt')):
+        raise SystemExit(f'no reference source tree at {src}')
     scratch = os.path.join(tempfile.gettempdir(), 'obe_refcopy')
     if os.path.isdir(scratch):
         shutil.rmtree(scratch)
@@ -267,6 +268,28 @@ def run_sweeper_lockstep():
     return out
 
 
+#: keys of a run_lockstep() record that are recorded for diagnosis only: neither tests/test_oracle.py nor
+#: tests/test_gpu_parity.py reads them.  (The sweeper record is stored whole: tests/test_gpu_sweeper.py reads its std.)
+DIAGNOSTIC_KEYS = ('std', 'n_eff', 'first_resample_step', 'pre_resample_weights', 'pre_resample_particles',
+                   'post_resample_particles', 'worst_weight_rel')
+#: a utility row longer than this is stored at a fixed, seeded sample of the settings (utility_columns)
+MAX_UTILITY_COLUMNS = 4096
+
+
+def shrink(out):
+    """A scenario's golden record as stored: the diagnostic keys dropped, and a long utility row (c3's 101 x 101 grid)
+    sampled at MAX_UTILITY_COLUMNS fixed settings that include every chosen one.  The chosen indices themselves
+    are still checked against the whole grid (set_index)."""
+    keep = {k: v for k, v in out.items() if k not in DIAGNOSTIC_KEYS}
+    util = keep.get('utility')
+    if util is not None and util.shape[1] > MAX_UTILITY_COLUMNS:
+        cols = np.random.default_rng(0).choice(util.shape[1], MAX_UTILITY_COLUMNS, replace=False)
+        cols = np.unique(np.concatenate((cols, keep['set_index']))).astype(np.int64)
+        keep['utility'] = util[:, cols]
+        keep['utility_columns'] = cols
+    return keep
+
+
 def check_equivalences():
     """The numpy identities the oracle relies on (SURVEY 8c), re-verified against this numpy."""
     rng = np.random.default_rng(7)
@@ -321,10 +344,11 @@ def check_entropy_utilities(ref):
 
 def main():
     ap = argparse.ArgumentParser()
+    ap.add_argument('--reference', required=True, help='source tree of usnistgov/optbayesexpt v1.2.0')
     ap.add_argument('--check', action='store_true')
     ap.add_argument('--only', default=None)
     args = ap.parse_args()
-    ref = import_reference()
+    ref = import_reference(args.reference)
     check_equivalences()
     check_entropy_utilities(ref)
     os.makedirs(GOLDEN, exist_ok=True)
@@ -335,7 +359,7 @@ def main():
         print(f"{sc['name']}: lock-step OK over {sc['n_cycles']} cycles, "
               f"{int(out['resampled'].sum())} resamples, worst weight rel diff {out['worst_weight_rel']:.2e}")
         if not args.check:
-            keep = {k: v for k, v in out.items()}
+            keep = shrink(out)
             if not sc.get('store_prior', True):
                 keep.pop('prior')
                 keep.pop('pre_resample_particles', None)

@@ -666,13 +666,14 @@ def test_golden_trajectory(obe, sc):
     eng, inp = _engine(obe, sc, pickiness=sc.get('pickiness', 15))
     nch = orc.MODELS[sc['model']][4]
     tol = sc.get('traj_rtol', 1e-9)
+    cols = g['utility_columns'] if 'utility_columns' in g.files else slice(None)   # (a large grid is sampled)
     seen = False
     with warnings.catch_warnings():
         warnings.simplefilter('ignore', RuntimeWarning)
         for t in range(sc['n_cycles']):
             setting = eng.good_setting() if sc['selection'] == 'good' else eng.opt_setting()
             assert eng.last_setting_index == g['set_index'][t], f'setting index differs at cycle {t}'
-            assert_allclose(eng._utility_dev.cpu().numpy(), g['utility'][t], rtol=tol if seen else 1e-12,
+            assert_allclose(eng._utility_dev.cpu().numpy()[cols], g['utility'][t], rtol=tol if seen else 1e-12,
                             err_msg=f'utility t={t}')
             y, sig = g['y_meas'][t], g['sigma_meas'][t]
             rec = (setting, tuple(y) if nch > 1 else float(y[0]), tuple(sig) if nch > 1 else float(sig[0]))

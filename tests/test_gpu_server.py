@@ -1,7 +1,7 @@
-"""SURVEY 8(f) row 3: the reference's own TCP front end (``OBE_Server``, optbayesexpt/obe_server.py:118-315, wire format
-obe_socket.py:12-25,88-129) driving the GPU engine.  The server class is the UNMODIFIED reference's (imported from
-baseline/_ref, which travels to the GPU box; /root/reference in the build container); only the engine it is told to
-make (``make_obe``) is ours.  The client speaks the reference's protocol (10-digit length + JSON) over loopback:
+"""SURVEY 8(f) row 3: the reference's TCP front end (``OBE_Server``, optbayesexpt/obe_server.py:118-315, wire format
+obe_socket.py:12-25,88-129) driving the GPU engine.  The server class is the UNMODIFIED reference's when it is installed
+in baseline/_ref (baseline/install_reference.sh), else its restatement in oracle/obe_server.py; only the engine it is
+told to make (``make_obe``) is ours.  The client speaks the reference's protocol (10-digit length + JSON) over loopback:
 optset / goodset / newdat / getmean / getstd / getcov / getset / getcon / getpar / getwgt / ready / done.
 Only getpar / getwgt may bring the cloud back to the host."""
 import os
@@ -19,14 +19,15 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def _reference():
-    for path in (os.path.join(ROOT, 'baseline', '_ref'), '/root/reference'):
-        if os.path.isdir(os.path.join(path, 'optbayesexpt')):
-            if path not in sys.path:
-                sys.path.insert(0, path)
-            warnings.simplefilter('ignore', SyntaxWarning)
-            import optbayesexpt
-            return optbayesexpt
-    pytest.skip('the reference package is not installed (baseline/install_reference.sh)')
+    path = os.path.join(ROOT, 'baseline', '_ref')
+    if os.path.isdir(os.path.join(path, 'optbayesexpt')):
+        if path not in sys.path:
+            sys.path.insert(0, path)
+        warnings.simplefilter('ignore', SyntaxWarning)
+        import optbayesexpt
+        return optbayesexpt
+    from oracle import obe_server
+    return obe_server
 
 
 def _free_port():

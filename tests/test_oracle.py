@@ -163,6 +163,7 @@ def test_oracle_replays_reference_golden(sc):
                         cost_of_changing_setting=sc.get('cost_of_changing_setting'),
                         rng=np.random.default_rng(sc['seed_rng']))
     tol = sc.get('traj_rtol', 1e-9)
+    cols = g['utility_columns'] if 'utility_columns' in g.files else slice(None)   # (a large grid is sampled)
     seen = False
     import warnings
     with warnings.catch_warnings():
@@ -170,7 +171,7 @@ def test_oracle_replays_reference_golden(sc):
         for t in range(sc['n_cycles']):
             setting = eng.good_setting() if sc['selection'] == 'good' else eng.opt_setting()
             assert eng.last_setting_index == g['set_index'][t], f't={t}'
-            assert_allclose(eng.last_utility, g['utility'][t], rtol=tol if seen else 1e-12)
+            assert_allclose(eng.last_utility[cols], g['utility'][t], rtol=tol if seen else 1e-12)
             y, sig = g['y_meas'][t], g['sigma_meas'][t]
             rec = (setting, tuple(y) if nch > 1 else float(y[0]), tuple(sig) if nch > 1 else float(sig[0]))
             eng.pdf_update(rec)
@@ -181,6 +182,17 @@ def test_oracle_replays_reference_golden(sc):
             assert_allclose(eng.mean(), g['mean'][t], rtol=tol if seen else 1e-12)
     assert_allclose(eng.particle_weights, g['final_weights'], rtol=max(tol, 1e-9),
                     atol=1e-15 * g['final_weights'].max())
+
+
+def test_golden_shrink_keeps_what_the_replays_read():
+    """oracle/pin_against_reference.py stores every scenario record through shrink(): it must keep each key that the
+    replays here and in tests/test_gpu_parity.py read."""
+    from oracle.pin_against_reference import shrink
+    read = {'prior', 'set_index', 'utility', 'y_meas', 'sigma_meas', 'resampled', 'first_ancestors', 'mean', 'cov',
+            'final_weights', 'final_particles'}
+    for sc in SCENARIOS:
+        g = np.load(os.path.join(GOLDEN, sc['name'] + '.npz'))
+        assert read <= set(g.files) and read <= set(shrink({k: g[k] for k in g.files})), sc['name']
 
 
 # ---- sweeper workload (demos/sweeper/obe_sweeper.py), SURVEY 8(f) row 2 ------------------------------
