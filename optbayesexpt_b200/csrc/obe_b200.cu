@@ -1459,7 +1459,7 @@ __global__ void __launch_bounds__(OBE_THREADS, OBE_MOVE_BLOCKS(D)) k_sys_move(co
 #define OBE_WR_PREFETCH 1   /* B2 prefetches the next group's ancestor lines into L2 while this group is computed */
 #endif
 
-struct WrUnit { long long og_al, o_al, base; int q_emit_end, A, lastrel, pad; };
+struct WrUnit { long long og_al, o_al, base; int q_emit_end, A, lastrel, rr; };
 
 // ---- the comb arithmetic of one work unit, shared by the streaming kernel and the early-select pick kernel (so the
 // ancestor of a slot is the same bits wherever it is computed)
@@ -1626,6 +1626,13 @@ __global__ void __launch_bounds__(OBE_THREADS, OBE_WR_BLOCKS(D)) k_sys_resample_
         {
             const double wuni = c.wuni_in;
             const double* __restrict__ wt = c.w_in + base;
+            // the whole tile's weights (16 KB) are requested into L2 at once: the segment walk below keeps only one
+            // 2 KB segment in flight, so without this every segment paid its own HBM latency
+            if (wuni <= 0.0) {
+#pragma unroll 1
+                for (int i = lane * 16; i < cnt_tile; i += 32 * 16)      // one 128-byte line per lane and step
+                    asm volatile("prefetch.global.L2 [%0];" ::"l"(wt + i));
+            }
             const WrComb cw = wr_comb_of(c, c.prefix[k], chunk0, A, n_chunk, lastrel);
             double wb = 0.0;                  // canonical sum of the totals of the segments before this one
             int carry_end = A;                // end slot of the last particle walked so far
@@ -1690,6 +1697,7 @@ __global__ void __launch_bounds__(OBE_THREADS, OBE_WR_BLOCKS(D)) k_sys_resample_
                 w.o_al = chunk0 - A - c.slot_begin;                   // its position in this shard's output (multiple of 4)
                 w.base = base;
                 w.q_emit_end = A + n_emit; w.A = A; w.lastrel = lastrel;
+                w.rr = (int)(c.slot_begin & 3);                       // launch-uniform
             }
             __syncwarp();
             const volatile WrUnit& vu = wu[warp];
@@ -1697,9 +1705,6 @@ __global__ void __launch_bounds__(OBE_THREADS, OBE_WR_BLOCKS(D)) k_sys_resample_
             // Groups are aligned to the shard's OUTPUT, so every full group stores whole 32-byte sectors whatever
             // the shard's first global slot is; a shard with slot_begin % 4 != 0 draws the normals of its groups from
             // one more Philox call (jitter_group4_w) -- the normals of a slot do not depend on the grouping.
-            const int rr = (int)(c.slot_begin & 3);                   // launch-uniform
-            const double* __restrict__ pin = c.pin + base;
-            const long long ld_in = c.ld_in, ld_out = c.ld_out;
 #if OBE_WR_SPLIT
             // B1: marks -> ancestors (index + 1) in place: max-scan over the chunk, the carry in a register
             {
@@ -1735,6 +1740,8 @@ __global__ void __launch_bounds__(OBE_THREADS, OBE_WR_BLOCKS(D)) k_sys_resample_
             auto emit = [&](auto full_tag, const int emit_pos) {
                 constexpr bool FULL = decltype(full_tag)::value;
                 const int q0 = emit_pos + lane * 4;
+                const double* __restrict__ pin = vc.pin + vu.base;
+                const long long ld_in = vc.ld_in;
                 unsigned int* rp = reinterpret_cast<unsigned int*>(marks + q0);
                 const uint2 raw = *reinterpret_cast<const uint2*>(rp);
                 *reinterpret_cast<uint2*>(rp) = make_uint2(0u, 0u);
@@ -1788,7 +1795,7 @@ __global__ void __launch_bounds__(OBE_THREADS, OBE_WR_BLOCKS(D)) k_sys_resample_
                     for (int j = 0; j < D; ++j) xv[u][j] = __ldg(pin + j * ld_in + rel[u]);
                 }
                 if (vc.jitter) {
-                    switch (rr) {
+                    switch (vu.rr) {
                         case 0: jitter_group4_w<D, 0>(xv, vu.og_al + q0, vc.seed, vc.epoch, sF, sMean, vc.a_param, vc.scale,
                                                       vc.z_out, vu.o_al + q0, ok); break;
                         case 1: jitter_group4_w<D, 1>(xv, vu.og_al + q0, vc.seed, vc.epoch, sF, sMean, vc.a_param, vc.scale,
@@ -1802,6 +1809,7 @@ __global__ void __launch_bounds__(OBE_THREADS, OBE_WR_BLOCKS(D)) k_sys_resample_
                 const long long o0 = vu.o_al + q0;
                 double* __restrict__ pout = vc.pout;
                 double* __restrict__ w_out = vc.w_out;
+                const long long ld_out = vc.ld_out;
                 if (FULL || all) {
 #pragma unroll
                     for (int j = 0; j < D; ++j) {
