@@ -93,6 +93,25 @@ int obe_model_builtin(const char* name, int n_params, obe_model_t* out);
 int obe_model_compile(const char* cuda_source, const char* entry, int n_settings, int n_params,
                       int n_model_params, int n_constants, int n_channels, obe_model_t* out,
                       char* log, size_t log_len);
+/* A model whose update uses a non-Gaussian measurement likelihood, compiled by NVRTC for sm_100a.
+ * The model is the built-in `builtin_name`, or (builtin_name == NULL) `model_source` / `model_entry`
+ * with the dimensions of obe_model_compile.  `likelihood`:
+ *   "poisson"   record (setting, k_c): y_c is the expected count lambda_c,
+ *               log L = sum_c xlogy(k_c, lambda_c) - lambda_c - lgamma(k_c + 1)
+ *   "binomial"  record (setting, k_c, n_c): y_c is the success probability p_c,
+ *               log L = sum_c lgamma(n+1) - lgamma(k+1) - lgamma(n-k+1) + xlogy(k, p) + xlog1py(n-k, -p)
+ *   "user"      `likelihood_source` defines
+ *               __device__ double <likelihood_entry>(const double* y_model, const double* y_meas,
+ *                                                    const double* aux, int n_channels)
+ *               returning log L of the record (y_meas = its second element, aux = its third).
+ * The weight factor is exp(choke * log L).  obe_update / obe_cycle / obe_update_from_y_model take such a
+ * handle: y_meas carries the counts (the measured values), sigma the third element of the record
+ * (trial counts, aux; may be NULL for Poisson), noise_index must be NULL.  The batched and multi-point
+ * entries refuse it. */
+int obe_model_compile_likelihood(const char* builtin_name, const char* model_source, const char* model_entry,
+                                 int n_settings, int n_params, int n_model_params, int n_constants,
+                                 int n_channels, const char* likelihood, const char* likelihood_source,
+                                 const char* likelihood_entry, obe_model_t* out, char* log, size_t log_len);
 int obe_model_info(obe_model_t m, int* n_settings, int* n_model_params, int* n_constants,
                    int* n_channels, int* n_params);
 void obe_model_free(obe_model_t m);
@@ -117,6 +136,12 @@ int obe_update_from_y(const obe_cloud_t* c, const double* y_model_dev, int64_t l
                       const double* y_meas, const double* sigma, const int32_t* noise_index,
                       int n_lik_channels, int use_choke, double choke, const double* pivot,
                       void* stream);
+/* obe_update_from_y with the likelihood of the model handle m (obe_update_from_y itself for a
+ * Gaussian handle). */
+int obe_update_from_y_model(obe_model_t m, const obe_cloud_t* c, const double* y_model_dev, int64_t ld_y,
+                            int n_channels, const double* y_meas, const double* sigma,
+                            const int32_t* noise_index, int n_lik_channels, int use_choke, double choke,
+                            const double* pivot, void* stream);
 /* ParticlePDF.bayesian_update(likelihood) (particlepdf.py:216-231): likelihood supplied, (n). */
 int obe_update_from_likelihood(const obe_cloud_t* c, const double* likelihood_dev,
                                const double* pivot, void* stream);

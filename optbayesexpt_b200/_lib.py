@@ -93,12 +93,17 @@ SIGNATURES = {
     'obe_model_builtin': (C.c_int, [C.c_char_p, C.c_int, C.POINTER(_VP)]),
     'obe_model_compile': (C.c_int, [C.c_char_p, C.c_char_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                     C.POINTER(_VP), C.c_char_p, C.c_size_t]),
+    'obe_model_compile_likelihood': (C.c_int, [C.c_char_p, C.c_char_p, C.c_char_p, C.c_int, C.c_int, C.c_int, C.c_int,
+                                               C.c_int, C.c_char_p, C.c_char_p, C.c_char_p, C.POINTER(_VP),
+                                               C.c_char_p, C.c_size_t]),
     'obe_model_info': (C.c_int, [_VP] + [C.POINTER(C.c_int)] * 5),
     'obe_model_free': (None, [_VP]),
     'obe_set_uniform': (C.c_int, [_PCLOUD, _VP]),
     'obe_update': (C.c_int, [_VP, _PCLOUD, _PD, _PD, _PD, _PD, _PI32, C.c_int, C.c_int, C.c_double, _PD, _VP]),
     'obe_update_from_y': (C.c_int, [_PCLOUD, _VP, C.c_int64, C.c_int, _PD, _PD, _PI32, C.c_int, C.c_int,
                                     C.c_double, _PD, _VP]),
+    'obe_update_from_y_model': (C.c_int, [_VP, _PCLOUD, _VP, C.c_int64, C.c_int, _PD, _PD, _PI32, C.c_int, C.c_int,
+                                          C.c_double, _PD, _VP]),
     'obe_update_from_likelihood': (C.c_int, [_PCLOUD, _VP, _PD, _VP]),
     'obe_refresh': (C.c_int, [_PCLOUD, C.c_uint32, C.c_uint32, _PI32, C.c_int, _PD, C.c_int, _VP]),
     'obe_fetch_stats': (C.c_int, [_PCLOUD, _PD, _VP]),

@@ -16,7 +16,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from .models import DeviceModel, builtin
+from .models import DeviceModel, builtin, non_gaussian
 
 
 class BatchedOptBayesExpt:
@@ -31,6 +31,9 @@ class BatchedOptBayesExpt:
             measurement_model = builtin(measurement_model)
         if not isinstance(measurement_model, DeviceModel):
             raise TypeError('measurement_model must be a DeviceModel; there is no CPU fallback')
+        if non_gaussian(measurement_model):
+            raise ValueError('BatchedOptBayesExpt supports the Gaussian likelihood only; use OptBayesExpt for '
+                             'a Poisson, binomial or cuda_likelihood model')
         self.model_function = measurement_model
         from .models import resolve_device
         dev = resolve_device(device)

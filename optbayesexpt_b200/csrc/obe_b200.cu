@@ -17,6 +17,7 @@
 #include <stdio.h>
 #include <string.h>
 #include <atomic>
+#include <cmath>
 #include <string>
 #include <type_traits>
 #include <vector>
@@ -141,11 +142,13 @@ static cudaError_t set_max_smem(const void* f, size_t smem) {
     if (e == cudaSuccess && dev >= 0 && n_cached < 96) cache[n_cached++] = Ent{f, smem, dev};
     return e;
 }
-static int launch_update_kernel(const void* f, int d, int src, const ObeUpdateArgs& a, int grid, cudaStream_t st) {
+// q: the per-record data of a non-Gaussian likelihood, the second argument of its update kernels
+static int launch_update_kernel(const void* f, int d, int src, const ObeUpdateArgs& a, int grid, cudaStream_t st,
+                                const ObeLikParams* q = nullptr) {
     const size_t smem = update_smem_bytes(d, src);
     cudaError_t e = set_max_smem(f, smem);
     if (e != cudaSuccess) return obe_fail("cudaFuncSetAttribute(max dynamic smem): %s%s", cudaGetErrorString(e));
-    void* params[1] = {const_cast<ObeUpdateArgs*>(&a)};
+    void* params[2] = {const_cast<ObeUpdateArgs*>(&a), const_cast<ObeLikParams*>(q)};
     e = cudaLaunchKernel(f, dim3(grid), dim3(OBE_UPDATE_THREADS), params, smem, st);
     if (e != cudaSuccess) return obe_fail("launch update kernel: %s%s", cudaGetErrorString(e));
     return 0;
@@ -2460,7 +2463,13 @@ struct obe_model {
     const void* f_bsim;
     const void* f_multi;    // multi-point (sweep) update
     cudaLibrary_t lib;
+    int lik;                // OBE_LIK_*: the measurement likelihood of the update kernels
+    const void* f_update_y; // non-Gaussian handles: the update from a supplied y_model (OBE_SRC_Y)
 };
+#define OBE_LIK_GAUSS 0
+#define OBE_LIK_POISSON 1
+#define OBE_LIK_BINOMIAL 2
+#define OBE_LIK_USER 3
 
 template <class M, int D>
 static void fill_model(obe_model* m) {
@@ -2548,6 +2557,68 @@ static const char* k_src_models =
 #include "obe_models_src.inc"
     ;
 
+// NVRTC: source -> sm_100a cubin; the compiler log goes to `log` and, on failure, into the error message
+static int nvrtc_cubin(const std::string& src, const char* name, std::vector<char>& cubin, char* log, size_t log_len) {
+    nvrtcProgram prog;
+    const char* headers[2] = {k_src_device, k_src_models};
+    const char* names[2] = {"obe_device.cuh", "obe_models.cuh"};
+    nvrtcResult r = g_nvrtc.create(&prog, src.c_str(), name, 2, headers, names);
+    if (r != NVRTC_SUCCESS) return obe_fail("nvrtcCreateProgram: %s%s", g_nvrtc.errstr(r));
+    const char* opts[] = {"--gpu-architecture=sm_100a", "-std=c++17", "-lineinfo"};
+    r = g_nvrtc.compile(prog, 3, opts);
+    size_t lsz = 0;
+    g_nvrtc.log_size(prog, &lsz);
+    std::vector<char> lbuf(lsz + 1, 0);
+    if (lsz > 1) g_nvrtc.log(prog, lbuf.data());
+    if (log && log_len) {
+        strncpy(log, lbuf.data(), log_len - 1);
+        log[log_len - 1] = 0;
+    }
+    if (r != NVRTC_SUCCESS) {
+        g_nvrtc.destroy(&prog);
+        return obe_fail("NVRTC compile failed: %s\n%s", g_nvrtc.errstr(r), lbuf.data());
+    }
+    size_t csz = 0;
+    g_nvrtc.cubin_size(prog, &csz);
+    cubin.resize(csz);
+    g_nvrtc.cubin(prog, cubin.data());
+    g_nvrtc.destroy(&prog);
+    return 0;
+}
+// loads the cubin into m->lib and looks up `n` kernels; on failure frees m
+static int load_kernels(obe_model* m, const std::vector<char>& cubin, const char* const* names, const void** k, int n) {
+    cudaError_t e = cudaLibraryLoadData(&m->lib, cubin.data(), nullptr, nullptr, 0, nullptr, nullptr, 0);
+    if (e != cudaSuccess) { delete m; return obe_fail("cudaLibraryLoadData: %s%s", cudaGetErrorString(e)); }
+    for (int i = 0; i < n; ++i) {
+        cudaKernel_t kk;
+        e = cudaLibraryGetKernel(&kk, m->lib, names[i]);
+        if (e != cudaSuccess) {
+            cudaLibraryUnload(m->lib);
+            delete m;
+            return obe_fail("cudaLibraryGetKernel(%s): %s", names[i], cudaGetErrorString(e));
+        }
+        k[i] = (const void*)kk;
+    }
+    return 0;
+}
+
+template <class M>
+static const char* builtin_dims(const char* name, obe_model* m) {
+    m->ns = M::NS; m->np_model = M::NP; m->ncons = M::NCONS; m->nch = M::NCH;
+    return name;
+}
+// the functor struct of a built-in model (NULL for an unknown name), and its dimensions into m
+static const char* builtin_struct(const std::string& s, obe_model* m) {
+    if (s == "lorentzian_hwhm") return builtin_dims<ObeLorentzianHWHM>("ObeLorentzianHWHM", m);
+    if (s == "lorentzian_fwhm") return builtin_dims<ObeLorentzianFWHM>("ObeLorentzianFWHM", m);
+    if (s == "lorentzian_4p") return builtin_dims<ObeLorentzian4P>("ObeLorentzian4P", m);
+    if (s == "lorentzian_dip") return builtin_dims<ObeLorentzianDip>("ObeLorentzianDip", m);
+    if (s == "line") return builtin_dims<ObeLine>("ObeLine", m);
+    if (s == "rabi") return builtin_dims<ObeRabi>("ObeRabi", m);
+    if (s == "lockin_coil") return builtin_dims<ObeLockinCoil>("ObeLockinCoil", m);
+    return nullptr;
+}
+
 // ---------------------------------------------------------------------------------------------
 // C ABI
 // ---------------------------------------------------------------------------------------------
@@ -2631,50 +2702,89 @@ int obe_model_compile(const char* cuda_source, const char* entry, int n_settings
     std::string src = "#include \"obe_device.cuh\"\n#include \"obe_models.cuh\"\n";
     src += cuda_source;
     src += tail;
-    nvrtcProgram prog;
-    const char* headers[2] = {k_src_device, k_src_models};
-    const char* names[2] = {"obe_device.cuh", "obe_models.cuh"};
-    nvrtcResult r = g_nvrtc.create(&prog, src.c_str(), "obe_user_model.cu", 2, headers, names);
-    if (r != NVRTC_SUCCESS) return obe_fail("nvrtcCreateProgram: %s%s", g_nvrtc.errstr(r));
-    const char* opts[] = {"--gpu-architecture=sm_100a", "-std=c++17", "-lineinfo"};
-    r = g_nvrtc.compile(prog, 3, opts);
-    size_t lsz = 0;
-    g_nvrtc.log_size(prog, &lsz);
-    std::vector<char> lbuf(lsz + 1, 0);
-    if (lsz > 1) g_nvrtc.log(prog, lbuf.data());
-    if (log && log_len) {
-        strncpy(log, lbuf.data(), log_len - 1);
-        log[log_len - 1] = 0;
-    }
-    if (r != NVRTC_SUCCESS) {
-        g_nvrtc.destroy(&prog);
-        return obe_fail("NVRTC compile failed: %s\n%s", g_nvrtc.errstr(r), lbuf.data());
-    }
-    size_t csz = 0;
-    g_nvrtc.cubin_size(prog, &csz);
-    std::vector<char> cubin(csz);
-    g_nvrtc.cubin(prog, cubin.data());
-    g_nvrtc.destroy(&prog);
+    std::vector<char> cubin;
+    if (nvrtc_cubin(src, "obe_user_model.cu", cubin, log, log_len)) return -1;
     obe_model* m = new obe_model();
     m->ns = n_settings; m->np_model = n_model_params; m->ncons = n_constants; m->nch = n_channels;
     m->d = n_params; m->user = true;
-    cudaError_t e = cudaLibraryLoadData(&m->lib, cubin.data(), nullptr, nullptr, 0, nullptr, nullptr, 0);
-    if (e != cudaSuccess) { delete m; return obe_fail("cudaLibraryLoadData: %s%s", cudaGetErrorString(e)); }
-    cudaKernel_t k[8];
+    const void* k[8];
     const char* kn[8] = {"obe_k_update_user", "obe_k_evalp_user", "obe_k_utility_user", "obe_k_evals_user",
                          "obe_k_bupdate_user", "obe_k_bselect_user", "obe_k_bsim_user", "obe_k_multi_user"};
-    for (int i = 0; i < 8; ++i) {
-        e = cudaLibraryGetKernel(&k[i], m->lib, kn[i]);
-        if (e != cudaSuccess) {
-            cudaLibraryUnload(m->lib);
-            delete m;
-            return obe_fail("cudaLibraryGetKernel(%s): %s", kn[i], cudaGetErrorString(e));
-        }
+    if (load_kernels(m, cubin, kn, k, 8)) return -1;
+    m->f_update = k[0]; m->f_evalp = k[1];
+    m->f_utility = k[2]; m->f_evals = k[3];
+    m->f_bupdate = k[4]; m->f_bselect = k[5]; m->f_bsim = k[6];
+    m->f_multi = k[7];
+    *out = m;
+    return 0;
+}
+
+int obe_model_compile_likelihood(const char* builtin_name, const char* model_source, const char* model_entry,
+                                 int n_settings, int n_params, int n_model_params, int n_constants, int n_channels,
+                                 const char* likelihood, const char* likelihood_source, const char* likelihood_entry,
+                                 obe_model_t* out, char* log, size_t log_len) {
+    if (log && log_len) log[0] = 0;
+    if (!out || !likelihood || (!builtin_name && (!model_source || !model_entry)))
+        return obe_fail("null argument%s%s");
+    const std::string lk(likelihood);
+    int kind;
+    if (lk == "poisson") kind = OBE_LIK_POISSON;
+    else if (lk == "binomial") kind = OBE_LIK_BINOMIAL;
+    else if (lk == "user") kind = OBE_LIK_USER;
+    else return obe_fail("unknown likelihood '%s' (poisson, binomial or user)%s", likelihood);
+    if (kind == OBE_LIK_USER && (!likelihood_source || !likelihood_entry))
+        return obe_fail("a user likelihood needs its source and entry%s%s");
+    obe_model tmp = {};
+    std::string model_def;
+    if (builtin_name) {
+        const char* st = builtin_struct(builtin_name, &tmp);
+        if (!st) return obe_fail("unknown built-in model '%s'%s", builtin_name);
+        model_def = std::string("typedef ") + st + " ObeLikModel;\n";
+    } else {
+        if (n_model_params < 0 || n_channels < 1 || n_channels > OBE_MAX_CH || n_settings < 0 ||
+            n_settings > OBE_MAX_SET || n_constants < 0 || n_constants > OBE_MAX_CONS)
+            return obe_fail("model dimensions out of range%s%s");
+        tmp.ns = n_settings; tmp.np_model = n_model_params; tmp.ncons = n_constants; tmp.nch = n_channels;
+        char def[1024];
+        snprintf(def, sizeof(def),
+                 "\nstruct ObeLikModel {\n"
+                 "    enum { NS = %d, NP = %d, NCONS = %d, NCH = %d };\n"
+                 "    __device__ static __forceinline__ void eval(const double* s, const double* p, const double* c, double* y) {\n"
+                 "        %s(s, p, c, y);\n    }\n};\n",
+                 n_settings, n_model_params, n_constants, n_channels, model_entry);
+        model_def = std::string(model_source) + def;
     }
-    m->f_update = (const void*)k[0]; m->f_evalp = (const void*)k[1];
-    m->f_utility = (const void*)k[2]; m->f_evals = (const void*)k[3];
-    m->f_bupdate = (const void*)k[4]; m->f_bselect = (const void*)k[5]; m->f_bsim = (const void*)k[6];
-    m->f_multi = (const void*)k[7];
+    if (n_params < 1 || n_params > OBE_MAX_DIMS || tmp.np_model > n_params)
+        return obe_fail("n_params out of range (the model's parameters .. 8)%s%s");
+    if (load_nvrtc()) return -1;
+    std::string src = "#include \"obe_device.cuh\"\n#include \"obe_models.cuh\"\n";
+    src += model_def;
+    const char* lik_type = kind == OBE_LIK_POISSON ? "ObePoissonLik" : (kind == OBE_LIK_BINOMIAL ? "ObeBinomialLik" : "ObeUserLik");
+    if (kind == OBE_LIK_USER) {
+        src += likelihood_source;
+        src += "\nstruct ObeUserPmf {\n"
+               "    static constexpr bool NONPOS = false;\n"
+               "    template <int NY>\n"
+               "    __device__ static __forceinline__ double loglik(const double (&y)[NY], const double* ym,\n"
+               "                                                    const ObeLikParams& q, int n) {\n"
+               "        return ";
+        src += likelihood_entry;
+        src += "(y, ym, q.aux, n);\n    }\n};\ntypedef ObeLogLik<ObeUserPmf> ObeUserLik;\n";
+    }
+    char tail[512];
+    snprintf(tail, sizeof(tail),
+             "OBE_DEFINE_LIK_KERNELS(ObeLikModel, %s, %d)\n"
+             "OBE_DEFINE_GRID_KERNELS(ObeLikModel, lik)\n", lik_type, n_params);
+    src += tail;
+    std::vector<char> cubin;
+    if (nvrtc_cubin(src, "obe_likelihood_model.cu", cubin, log, log_len)) return -1;
+    obe_model* m = new obe_model(tmp);
+    m->d = n_params; m->user = true; m->lik = kind;
+    const void* k[5];
+    const char* kn[5] = {"obe_k_update_lik", "obe_k_updatey_lik", "obe_k_evalp_lik", "obe_k_utility_lik",
+                         "obe_k_evals_lik"};
+    if (load_kernels(m, cubin, kn, k, 5)) return -1;
+    m->f_update = k[0]; m->f_update_y = k[1]; m->f_evalp = k[2]; m->f_utility = k[3]; m->f_evals = k[4];
     *out = m;
     return 0;
 }
@@ -2750,6 +2860,36 @@ static int fill_likelihood_args(ObeUpdateArgs& a, int d, int nch_avail, const do
     return 0;
 }
 
+// The record of a non-Gaussian likelihood: y_meas[c] = the counts (the measured values for a user likelihood),
+// aux[c] = the record's third element (binomial trial counts; anything a user likelihood reads; NULL for Poisson).
+// The log-factorial terms of the counting pmfs are per-record constants, computed here once.
+static int fill_lik_record(ObeUpdateArgs& a, ObeLikParams& q, int kind, int nch_avail, const double* y_meas,
+                           const double* aux, const int32_t* noise_index, int n_lik, int use_choke, double choke) {
+    if (n_lik < 0 || n_lik > nch_avail || n_lik > OBE_MAX_CH) return obe_fail("n_lik_channels out of range%s%s");
+    if (!y_meas) return obe_fail("y_meas is null%s%s");
+    if (noise_index) return obe_fail("a noise parameter needs the Gaussian likelihood%s%s");
+    if (!aux && kind != OBE_LIK_POISSON) return obe_fail("this likelihood needs the record's third element%s%s");
+    memset(&q, 0, sizeof(q));
+    a.n_lik_channels = n_lik;
+    for (int cidx = 0; cidx < n_lik; ++cidx) {
+        const double k = y_meas[cidx];
+        a.y_meas[cidx] = k;
+        q.aux[cidx] = aux ? aux[cidx] : 0.0;
+        if (kind == OBE_LIK_POISSON) {
+            if (!(std::isfinite(k) && k >= 0.0 && k == std::floor(k)))
+                return obe_fail("Poisson counts must be finite non-negative integers%s%s");
+            q.lconst[cidx] = std::lgamma(k + 1.0);
+        } else if (kind == OBE_LIK_BINOMIAL) {
+            const double nt = aux[cidx];
+            if (!(std::isfinite(k) && std::isfinite(nt) && k >= 0.0 && k <= nt && k == std::floor(k) && nt == std::floor(nt)))
+                return obe_fail("binomial records need integers 0 <= k <= n_trials%s%s");
+            q.lconst[cidx] = (std::lgamma(nt + 1.0) - std::lgamma(k + 1.0)) - std::lgamma(nt - k + 1.0);
+        }
+    }
+    a.use_choke = use_choke; a.choke = choke;
+    return 0;
+}
+
 int obe_set_uniform(const obe_cloud_t* c, void* stream) {
     if (check_cloud(c)) return -1;
     cudaStream_t st = (cudaStream_t)stream;
@@ -2789,6 +2929,12 @@ int obe_update(obe_model_t m, const obe_cloud_t* c, const double* setting, const
     a.scale_in = 1; a.write_weights = 1;
     for (int j = 0; j < m->ns; ++j) a.setting[j] = setting[j];
     for (int j = 0; j < m->ncons; ++j) a.cons[j] = constants[j];
+    if (m->lik != OBE_LIK_GAUSS) {
+        ObeLikParams q;
+        if (fill_lik_record(a, q, m->lik, m->nch, y_meas, sigma, noise_index, n_lik_channels, use_choke, choke)) return -1;
+        if (launch_update_kernel(m->f_update, c->d, OBE_SRC_MODEL, a, update_grid(c), (cudaStream_t)stream, &q)) return -1;
+        return finish_update(c, 1, (cudaStream_t)stream);
+    }
     if (fill_likelihood_args(a, c->d, m->nch, y_meas, sigma, noise_index, n_lik_channels, use_choke, choke)) return -1;
     cudaStream_t st = (cudaStream_t)stream;
     if (launch_update_kernel(m->f_update, c->d, OBE_SRC_MODEL, a, update_grid(c), st)) return -1;
@@ -2807,6 +2953,27 @@ int obe_update_from_y(const obe_cloud_t* c, const double* y_model_dev, int64_t l
     if (fill_likelihood_args(a, c->d, n_channels, y_meas, sigma, noise_index, n_lik_channels, use_choke, choke)) return -1;
     cudaStream_t st = (cudaStream_t)stream;
     if (launch_generic<OBE_SRC_Y>(c->d, a, update_grid(c), st)) return -1;
+    return finish_update(c, 1, st);
+}
+
+int obe_update_from_y_model(obe_model_t m, const obe_cloud_t* c, const double* y_model_dev, int64_t ld_y,
+                            int n_channels, const double* y_meas, const double* sigma, const int32_t* noise_index,
+                            int n_lik_channels, int use_choke, double choke, const double* pivot, void* stream) {
+    if (!m) return obe_fail("null model%s%s");
+    if (m->lik == OBE_LIK_GAUSS)
+        return obe_update_from_y(c, y_model_dev, ld_y, n_channels, y_meas, sigma, noise_index, n_lik_channels, use_choke,
+                                 choke, pivot, stream);
+    if (check_cloud(c)) return -1;
+    if (m->d != c->d) return obe_fail("model was built for a different n_params%s%s");
+    if (!y_model_dev || (ld_y & 1) || ((uintptr_t)y_model_dev & 15)) return obe_fail("y_model must be 16-byte aligned with even ld%s%s");
+    ObeUpdateArgs a;
+    base_update_args(c, a, pivot);
+    a.scale_in = 1; a.write_weights = 1;
+    a.y_model = y_model_dev; a.ld_y = ld_y;
+    ObeLikParams q;
+    if (fill_lik_record(a, q, m->lik, n_channels, y_meas, sigma, noise_index, n_lik_channels, use_choke, choke)) return -1;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (launch_update_kernel(m->f_update_y, c->d, OBE_SRC_Y, a, update_grid(c), st, &q)) return -1;
     return finish_update(c, 1, st);
 }
 
@@ -3604,6 +3771,8 @@ int obe_update_multi(obe_model_t m, const obe_cloud_t* c, double* weights_out_de
                      const double* lik_scale, int use_choke, double choke, double threshold, int64_t n_total,
                      double* sums_dev, double* result_dev, void* stream) {
     if (!m || !weights_out_dev || !records_dev || !sums_dev || !result_dev) return obe_fail("null argument%s%s");
+    if (m->lik != OBE_LIK_GAUSS)
+        return obe_fail("obe_update_multi: the model handle has a non-Gaussian likelihood (only the single-cloud update takes one)%s%s");
     if (check_cloud(c)) return -1;
     if (m->d != c->d) return obe_fail("model was built for a different n_params%s%s");
     if (n_points < 1 || n_points > OBE_MULTI_MAX) return obe_fail("multi-point update takes 1..128 points per call%s%s");
@@ -3634,6 +3803,8 @@ int obe_batch_simulate(obe_model_t m, const obe_batch_t* b, const double* settin
                        const double* noise_level, const double* noise_level_dev, uint64_t seed, uint32_t cycle,
                        int write_sigma, void* stream) {
     if (!m || !b || !settings_dev || !true_params_dev) return obe_fail("null argument%s%s");
+    if (m->lik != OBE_LIK_GAUSS)
+        return obe_fail("obe_batch_simulate: the model handle has a non-Gaussian likelihood (only the single-cloud update takes one)%s%s");
     if (!noise_level && !noise_level_dev) return obe_fail("simulate: need a noise level%s%s");
     if (ld_true < b->n_inst) return obe_fail("simulate: ld_true < n_inst%s%s");
     if (obe_sms() <= 0) return obe_fail("no CUDA device: this library has no CPU fallback%s%s");
@@ -3791,6 +3962,8 @@ int obe_batch_update(obe_model_t m, const obe_batch_t* b, const double* settings
                      const double* constants, const int32_t* noise_index, int n_lik_channels, int use_choke,
                      double choke, double resample_threshold, int force_resample, void* stream) {
     if (!m) return obe_fail("null model%s%s");
+    if (m->lik != OBE_LIK_GAUSS)
+        return obe_fail("obe_batch_update: the model handle has a non-Gaussian likelihood (only the single-cloud update takes one)%s%s");
     if (check_batch(b)) return -1;
     if (m->d != b->d) return obe_fail("model was built for a different n_params%s%s");
     if (use_last && !settings_dev) return obe_fail("use_last needs the setting grid%s%s");
@@ -3841,6 +4014,8 @@ int obe_batch_select(obe_model_t m, const obe_batch_t* b, const double* settings
                      const double* constants, int k, const double* var_noise, double cost_change, uint64_t uniform_seed,
                      uint32_t cycle, int method, int log_form, double* utility_dev, void* stream) {
     if (!m || !settings_dev) return obe_fail("null argument%s%s");
+    if (m->lik != OBE_LIK_GAUSS)
+        return obe_fail("obe_batch_select: the model handle has a non-Gaussian likelihood (only the single-cloud update takes one)%s%s");
     if (check_batch(b)) return -1;
     if (k < 1 || k > OBE_MAX_DRAWS) return obe_fail("n_draws must be 1..128 for batched engines%s%s");
     ObeBSelectArgs a;

@@ -417,12 +417,103 @@ __device__ __forceinline__ void obe_pick_rows(const double (&p)[NE][D], int ni, 
     for (int e = 0; e < NE; ++e) out[e] = dflt;
 }
 
+// ---- measurement likelihoods of the update pass --------------------------------------------------------------
+// A likelihood maps the model outputs y[e][c] of NE particles and the record (r_y[c]: the measured values) to the
+// factor lik[e] each weight is multiplied by, choke included.  The zip truncation of obe_base.py:453-455 is
+// a.n_lik_channels.
+
+// Gaussian noise with a known sigma, or sigma as a particle row (a.n_noise > 0).  The default.  Its code stays
+// inline in obe_update_vec: moved into a functor, ptxas allocated registers differently for one pre-instantiated
+// update kernel (k_update_generic<1, OBE_SRC_Y>, 90 -> 88), and the existing kernels are meant to stay as they are.
+struct ObeGaussLik {
+    static constexpr bool GAUSS = true;
+};
+
+// Per-record data of the log-likelihoods, computed on the host: aux[c] is the record's third element (trial counts
+// of a binomial, anything a user likelihood wants), lconst[c] the log-factorial terms of a counting pmf.
+struct ObeLikParams {
+    double aux[OBE_MAX_CH];
+    double lconst[OBE_MAX_CH];
+};
+
+// xlogy(k, x) = 0 for k == 0 (even at x == 0), k log x otherwise (scipy.special.xlogy)
+__device__ __forceinline__ double obe_xlogy(double k, double x) { return k == 0.0 ? 0.0 : k * log(x); }
+__device__ __forceinline__ double obe_xlog1py(double k, double x) { return k == 0.0 ? 0.0 : k * log1p(x); }
+
+// Poisson counts: r_y[c] = k_c >= 0, y_c = expected count lambda_c, lconst[c] = lgamma(k_c + 1)
+// (scipy.stats.poisson.logpmf).  lambda < 0 / NaN / +inf give NaN (weight 0, like nan_to_num of scipy's nan).
+struct ObePoissonPmf {
+    static constexpr bool NONPOS = true;
+    template <int NY>
+    __device__ static __forceinline__ double loglik(const double (&y)[NY], const double* k, const ObeLikParams& q, int n) {
+        double ll = 0.0;
+#pragma unroll
+        for (int c = 0; c < NY; ++c) {
+            if (c < n) {
+                const double lam = y[c];
+                const double lc = (obe_xlogy(k[c], lam) - lam) - q.lconst[c];
+                ll += (lam >= 0.0) ? lc : __longlong_as_double(0x7ff8000000000000ll);
+            }
+        }
+        return ll;
+    }
+};
+
+// Binomial: r_y[c] = k_c successes of aux[c] = n_c trials, y_c = success probability p_c,
+// lconst[c] = lgamma(n+1) - lgamma(k+1) - lgamma(n-k+1) (scipy.stats.binom.logpmf).  p outside [0, 1] gives NaN.
+struct ObeBinomialPmf {
+    static constexpr bool NONPOS = true;
+    template <int NY>
+    __device__ static __forceinline__ double loglik(const double (&y)[NY], const double* k, const ObeLikParams& q, int n) {
+        double ll = 0.0;
+#pragma unroll
+        for (int c = 0; c < NY; ++c) {
+            if (c < n) {
+                const double pr = y[c];
+                const double lc = (q.lconst[c] + obe_xlogy(k[c], pr)) + obe_xlog1py(q.aux[c] - k[c], -pr);
+                ll += (pr >= 0.0 && pr <= 1.0) ? lc : __longlong_as_double(0x7ff8000000000000ll);
+            }
+        }
+        return ll;
+    }
+};
+
+// A likelihood given as its logarithm per particle: lik = exp(choke * log L), choke = 1 without one.  A pmf has
+// log L <= 0 (NONPOS): rounding-level positive sums are clamped to 0 and the lean exp of the Gaussian applies (NaN
+// and -inf give 0).  Otherwise (a user likelihood) log L may be positive and goes through the full-range exp.
+template <class Pmf>
+struct ObeLogLik {
+    static constexpr bool GAUSS = false;
+    ObeLikParams q;
+    template <int D, int NE, int NY>
+    __device__ __forceinline__ void operator()(const ObeUpdateArgs& a, const double (&)[NE][D],
+                                               const double (&y)[NE][NY], const double* r_y, const double*,
+                                               double (&lik)[NE]) const {
+        double ll[NE];
+#pragma unroll
+        for (int e = 0; e < NE; ++e) {
+            ll[e] = Pmf::loglik(y[e], r_y, q, a.n_lik_channels);
+            if (Pmf::NONPOS) ll[e] = ll[e] > 0.0 ? 0.0 : ll[e];
+            if (a.use_choke) ll[e] *= a.choke;
+        }
+        if (Pmf::NONPOS) {
+            obe_exp_nonpos_vec<NE>(ll, lik);
+        } else {
+#pragma unroll
+            for (int e = 0; e < NE; ++e) lik[e] = exp(ll[e]);
+        }
+    }
+};
+typedef ObeLogLik<ObePoissonPmf> ObePoissonLik;
+typedef ObeLogLik<ObeBinomialPmf> ObeBinomialLik;
+
 // ALLV: every element of the stage is a live particle (all stages but the ragged last one): the valid[] selects vanish.
-template <class Model, int D, int SRC, int NE, bool BATCHED, bool ALLV = false>
+template <class Model, int D, int SRC, int NE, bool BATCHED, bool ALLV = false, class Lik = ObeGaussLik>
 __device__ __forceinline__ void obe_update_vec(const ObeUpdateArgs& a, const double (&p)[NE][D],
                                                const double (&w_in)[NE], const double (&yg)[NE][OBE_MAX_CH],
                                                const double (&lik_given)[NE], const bool (&valid)[NE], double invS,
-                                               ObeAcc<D>& acc, const double* rec, double (&t)[NE]) {
+                                               ObeAcc<D>& acc, const double* rec, double (&t)[NE],
+                                               const Lik& likf = Lik()) {
     const double* r_set = BATCHED ? rec + OBE_REC_SET : a.setting;
     const double* r_y = BATCHED ? rec + OBE_REC_Y : a.y_meas;
     const double* r_isig = BATCHED ? rec + OBE_REC_ISIG : a.inv_sigma;
@@ -448,52 +539,56 @@ __device__ __forceinline__ void obe_update_vec(const ObeUpdateArgs& a, const dou
                 }
                 lik[e] = 1.0;
             }
-            // prod_c exp(-((y_c - y_meas_c)/sigma_c)**2 / 2) / sigma_c  (obe_base.py:264-271, 453-455) as ONE
-            // exponential of the summed arguments times the product of the reciprocals: the division by sigma
-            // is a multiplication by its reciprocal (host's 1/sigma, or one refined rcp per particle for a
-            // noise parameter, shared by the channels that name the same row).  For one channel this is the
-            // same sequence of operations as exp(arg) * (1/sigma).
-            const bool noise = a.n_noise > 0;
-            double argsum[NE], isprod[NE], inv_prev[NE];
+            if constexpr (Lik::GAUSS) {
+                // prod_c exp(-((y_c - y_meas_c)/sigma_c)**2 / 2) / sigma_c  (obe_base.py:264-271, 453-455) as ONE
+                // exponential of the summed arguments times the product of the reciprocals: the division by sigma
+                // is a multiplication by its reciprocal (host's 1/sigma, or one refined rcp per particle for a
+                // noise parameter, shared by the channels that name the same row).  For one channel this is the
+                // same sequence of operations as exp(arg) * (1/sigma).
+                const bool noise = a.n_noise > 0;
+                double argsum[NE], isprod[NE], inv_prev[NE];
 #pragma unroll
-            for (int e = 0; e < NE; ++e) { argsum[e] = 0.0; isprod[e] = 1.0; inv_prev[e] = 1.0; }
-            int ni_prev = -2;
+                for (int e = 0; e < NE; ++e) { argsum[e] = 0.0; isprod[e] = 1.0; inv_prev[e] = 1.0; }
+                int ni_prev = -2;
 #pragma unroll
-            for (int c = 0; c < NY; ++c) {
-                if (c < a.n_lik_channels) {
-                    const int ni = a.noise_idx[c];
-                    double inv_sig[NE];
-                    if (!noise) {
+                for (int c = 0; c < NY; ++c) {
+                    if (c < a.n_lik_channels) {
+                        const int ni = a.noise_idx[c];
+                        double inv_sig[NE];
+                        if (!noise) {
 #pragma unroll
-                        for (int e = 0; e < NE; ++e) inv_sig[e] = r_isig[c];
-                    } else if (ni == ni_prev) {
+                            for (int e = 0; e < NE; ++e) inv_sig[e] = r_isig[c];
+                        } else if (ni == ni_prev) {
 #pragma unroll
-                        for (int e = 0; e < NE; ++e) inv_sig[e] = inv_prev[e];
-                    } else {
-                        double sig[NE];
-                        obe_pick_rows<D, NE>(p, ni, sig, 1.0);
+                            for (int e = 0; e < NE; ++e) inv_sig[e] = inv_prev[e];
+                        } else {
+                            double sig[NE];
+                            obe_pick_rows<D, NE>(p, ni, sig, 1.0);
 #pragma unroll
-                        for (int e = 0; e < NE; ++e) inv_sig[e] = obe_rcp_fast(sig[e]);
+                            for (int e = 0; e < NE; ++e) inv_sig[e] = obe_rcp_fast(sig[e]);
+                        }
+#pragma unroll
+                        for (int e = 0; e < NE; ++e) {
+                            const double q = (y[e][c] - r_y[c]) * inv_sig[e];
+                            argsum[e] = fma(-0.5 * q, q, argsum[e]);
+                            isprod[e] *= inv_sig[e];
+                            inv_prev[e] = inv_sig[e];
+                        }
+                        ni_prev = ni;
                     }
-#pragma unroll
-                    for (int e = 0; e < NE; ++e) {
-                        const double q = (y[e][c] - r_y[c]) * inv_sig[e];
-                        argsum[e] = fma(-0.5 * q, q, argsum[e]);
-                        isprod[e] *= inv_sig[e];
-                        inv_prev[e] = inv_sig[e];
-                    }
-                    ni_prev = ni;
                 }
-            }
-            {
-                double ex[NE];
-                obe_exp_nonpos_vec<NE>(argsum, ex);
+                {
+                    double ex[NE];
+                    obe_exp_nonpos_vec<NE>(argsum, ex);
 #pragma unroll
-                for (int e = 0; e < NE; ++e) lik[e] = ex[e] * isprod[e];
-            }
-            if (a.use_choke) {
+                    for (int e = 0; e < NE; ++e) lik[e] = ex[e] * isprod[e];
+                }
+                if (a.use_choke) {
 #pragma unroll
-                for (int e = 0; e < NE; ++e) lik[e] = pow(lik[e], a.choke);
+                    for (int e = 0; e < NE; ++e) lik[e] = pow(lik[e], a.choke);
+                }
+            } else {
+                likf(a, p, y, r_y, r_isig, lik);
             }
         }
         // t = nan_to_num(w * lik); w = w_in * invS needs no second nan_to_num (stored weights are finite and
@@ -694,8 +789,8 @@ struct ObeUpdateRows {
     static constexpr int NROWS = 1 + D + (SRC == OBE_SRC_Y ? OBE_MAX_CH : 0) + (SRC == OBE_SRC_LIK ? 1 : 0);
 };
 
-template <class Model, int D, int SRC>
-__device__ void obe_update_body(const ObeUpdateArgs& a) {
+template <class Model, int D, int SRC, class Lik = ObeGaussLik>
+__device__ void obe_update_body(const ObeUpdateArgs& a, const Lik& likf = Lik()) {
     constexpr int NROWS = ObeUpdateRows<D, SRC>::NROWS;
     using ST = ObeStage<NROWS>;
     constexpr int SE = ST::ELEMS, NST = ST::NSTAGES, SUB = ST::SUB, EPT = ST::EPT;
@@ -845,7 +940,7 @@ __device__ void obe_update_body(const ObeUpdateArgs& a) {
                     for (int c = 0; c < OBE_MAX_CH; ++c) yge[e][c] = (SRC == OBE_SRC_Y) ? yv[SRC == OBE_SRC_Y ? c : 0][e] : 0.0;
                     lke[e] = (SRC == OBE_SRC_LIK) ? lv[e] : 1.0;
                 }
-                obe_update_vec<Model, D, SRC, EPT, false>(a, pe, wv, yge, lke, valid, invS, acc, nullptr, te);
+                obe_update_vec<Model, D, SRC, EPT, false, false, Lik>(a, pe, wv, yge, lke, valid, invS, acc, nullptr, te, likf);
 #pragma unroll
                 for (int e = 0; e < EPT; ++e) tsum += te[e];
                 if (write_weights) {
@@ -1999,6 +2094,21 @@ struct ObeNoModel {
     }                                                                                                          \
     extern "C" __global__ void __launch_bounds__(OBE_THREADS) obe_k_bsim_##SUFFIX(const ObeBSimArgs a) {         \
         obe_bsimulate_body<MODEL>(a);                                                                          \
+    }
+
+// A model with a non-Gaussian likelihood LIK (compiled by NVRTC per handle): the model-evaluating update, the update
+// from a supplied y_model, and the model evaluation over the cloud.  No batched or multi-point kernels.
+#define OBE_DEFINE_LIK_KERNELS(MODEL, LIK, D)                                                                  \
+    extern "C" __global__ void __launch_bounds__(OBE_UPDATE_THREADS, 1) obe_k_update_lik(const ObeUpdateArgs a, \
+                                                                                         const ObeLikParams q) { \
+        obe_update_body<MODEL, D, OBE_SRC_MODEL, LIK>(a, LIK{q});                                               \
+    }                                                                                                          \
+    extern "C" __global__ void __launch_bounds__(OBE_UPDATE_THREADS, 1) obe_k_updatey_lik(const ObeUpdateArgs a, \
+                                                                                          const ObeLikParams q) { \
+        obe_update_body<ObeNoModel, D, OBE_SRC_Y, LIK>(a, LIK{q});                                              \
+    }                                                                                                          \
+    extern "C" __global__ void __launch_bounds__(OBE_THREADS) obe_k_evalp_lik(const ObeEvalArgs a) {           \
+        obe_eval_params_body<MODEL, D>(a);                                                                     \
     }
 
 #define OBE_DEFINE_GRID_KERNELS(MODEL, SUFFIX)                                                             \

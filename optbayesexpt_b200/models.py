@@ -33,7 +33,8 @@ class DeviceModel:
     parameters the model itself reads, e.g. a trailing noise parameter).
     """
 
-    def __init__(self, name, n_settings, n_model_params, n_constants, n_channels, source=None, entry=None):
+    def __init__(self, name, n_settings, n_model_params, n_constants, n_channels, source=None, entry=None,
+                 likelihood='gaussian'):
         self.name = name
         self.n_settings = n_settings
         self.n_model_params = n_model_params
@@ -41,8 +42,28 @@ class DeviceModel:
         self.n_channels = n_channels
         self.source = source
         self.entry = entry
+        #: measurement likelihood of the update kernels: 'gaussian', 'poisson', 'binomial' or a CudaLikelihood
+        self.likelihood = likelihood
         self._handles = {}
+        self._variants = {}
         self.compile_log = ''
+
+    def with_likelihood(self, likelihood):
+        """The same model with another measurement likelihood ('gaussian', 'poisson', 'binomial' or
+        :func:`cuda_likelihood`).  A non-Gaussian model is compiled by NVRTC on first use."""
+        if isinstance(likelihood, str):
+            if likelihood not in LIKELIHOODS:
+                raise ValueError(f'unknown likelihood_model {likelihood!r}; have {list(LIKELIHOODS)} or cuda_likelihood(...)')
+        elif not isinstance(likelihood, CudaLikelihood):
+            raise TypeError('likelihood_model must be one of '
+                            f'{list(LIKELIHOODS)} or optbayesexpt_b200.cuda_likelihood(source, entry)')
+        if likelihood == self.likelihood:
+            return self
+        if likelihood not in self._variants:        # (one NVRTC compile per likelihood and n_params)
+            self._variants[likelihood] = DeviceModel(self.name, self.n_settings, self.n_model_params,
+                                                     self.n_constants, self.n_channels, source=self.source,
+                                                     entry=self.entry, likelihood=likelihood)
+        return self._variants[likelihood]
 
     def handle(self, n_params):
         """obe_model_t for a cloud with ``n_params`` rows."""
@@ -52,7 +73,20 @@ class DeviceModel:
         if n_params < self.n_model_params:
             raise ValueError(f'model {self.name} reads {self.n_model_params} parameters, cloud has {n_params}')
         h = C.c_void_p()
-        if self.source is None:
+        if self.likelihood != 'gaussian':
+            log = C.create_string_buffer(1 << 16)
+            user = isinstance(self.likelihood, CudaLikelihood)
+            rc = lib.obe_model_compile_likelihood(
+                self.name.encode() if self.source is None else None,
+                None if self.source is None else self.source.encode(),
+                None if self.source is None else self.entry.encode(),
+                self.n_settings, n_params, self.n_model_params, self.n_constants, self.n_channels,
+                b'user' if user else self.likelihood.encode(),
+                self.likelihood.source.encode() if user else None,
+                self.likelihood.entry.encode() if user else None, C.byref(h), log, len(log))
+            self.compile_log = log.value.decode(errors='replace')
+            _lib.check(rc)
+        elif self.source is None:
             _lib.check(lib.obe_model_builtin(self.name.encode(), n_params, C.byref(h)))
         else:
             log = C.create_string_buffer(1 << 16)
@@ -114,8 +148,50 @@ class DeviceModel:
 
     def __repr__(self):
         kind = 'builtin' if self.source is None else 'nvrtc'
+        lik = '' if self.likelihood == 'gaussian' else f', likelihood={self.likelihood!r}'
         return (f'DeviceModel({self.name!r}, {kind}, settings={self.n_settings}, params={self.n_model_params}, '
-                f'constants={self.n_constants}, channels={self.n_channels})')
+                f'constants={self.n_constants}, channels={self.n_channels}{lik})')
+
+
+#: the measurement likelihoods of the update kernel, by name (a user likelihood is a :func:`cuda_likelihood`)
+LIKELIHOODS = ('gaussian', 'poisson', 'binomial')
+
+
+class CudaLikelihood:
+    """A measurement likelihood as CUDA source: see :func:`cuda_likelihood`."""
+
+    def __init__(self, source, entry):
+        self.source = source
+        self.entry = entry
+
+    def __eq__(self, other):
+        return isinstance(other, CudaLikelihood) and (self.source, self.entry) == (other.source, other.entry)
+
+    def __hash__(self):
+        return hash((self.source, self.entry))
+
+    def __repr__(self):
+        return f'cuda_likelihood(entry={self.entry!r})'
+
+
+def non_gaussian(measurement_model, likelihood_model=None):
+    """True when an engine built from these arguments would use a non-Gaussian likelihood."""
+    if likelihood_model is not None:
+        return likelihood_model != 'gaussian'
+    return isinstance(measurement_model, DeviceModel) and measurement_model.likelihood != 'gaussian'
+
+
+def cuda_likelihood(source, entry):
+    """User measurement likelihood for ``OptBayesExpt(..., likelihood_model=...)``, compiled by NVRTC with the model.
+
+    ``source`` must define ``__device__ double <entry>(const double* y_model, const double* y_meas,
+    const double* aux, int n_channels)`` returning the LOG-likelihood of the record for one particle:
+    ``y_model`` are the model outputs, ``y_meas`` the record's second element and ``aux`` its third (a noise
+    level, trial counts, anything per channel), both cut to ``n_channels`` entries.  The weight factor is
+    ``exp(choke * log L)``; log L may be positive.  This replaces overriding ``likelihood`` in Python, which
+    cannot run inside the update kernel.
+    """
+    return CudaLikelihood(source, entry)
 
 
 def builtin(name):

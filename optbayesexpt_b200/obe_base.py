@@ -53,16 +53,40 @@ class OptBayesExpt(ParticlePDF):
 
     ``measurement_model`` must be a :class:`~optbayesexpt_b200.models.DeviceModel` (or the name
     of a built-in): a Python callable cannot run inside a kernel and there is no CPU path.
+
+    ``likelihood_model`` selects the measurement likelihood of the update (the reference's
+    ``likelihood`` method, obe_base.py:418-461), evaluated inside the update kernel:
+
+    - ``'gaussian'`` (the default): records ``(setting, y_meas, sigma)``;
+    - ``'poisson'``: records ``(setting, counts)`` or ``(setting, counts, ignored)``, the model output is the
+      expected count;
+    - ``'binomial'``: records ``(setting, k, n_trials)``, the model output is the success probability;
+    - :func:`~optbayesexpt_b200.models.cuda_likelihood`: a log-likelihood in CUDA, records
+      ``(setting, y_meas, aux)``.
+
+    The design half is the same for every likelihood: the utility divides by ``yvar_noise_model()``, so
+    for counting data ``default_noise_std`` sets the noise scale of the utility (e.g. about sqrt of a typical
+    count).  Overriding ``likelihood`` in Python raises ``TypeError``: it could not run inside the kernel.
     """
 
     def __init__(self, measurement_model, setting_values, parameter_samples, constants,
                  n_draws=DEFAULT_N_DRAWS, choke=None, use_jit=True, utility_method='variance_approx',
-                 selection_method='optimal', pickiness=15, default_noise_std=1.0, **kwargs):
+                 selection_method='optimal', pickiness=15, default_noise_std=1.0, likelihood_model=None, **kwargs):
         if isinstance(measurement_model, str):
             measurement_model = builtin(measurement_model)
         if not isinstance(measurement_model, DeviceModel):
             raise TypeError('measurement_model must be a DeviceModel (optbayesexpt_b200.models.builtin(...) or '
                             'cuda_source(...)): a Python callable cannot run on the GPU and there is no CPU fallback')
+        if type(self).likelihood is not OptBayesExpt.likelihood:
+            raise TypeError(f'{type(self).__name__} overrides likelihood() in Python, which the update kernel cannot '
+                            'run: pass likelihood_model=\'poisson\' | \'binomial\' | '
+                            'optbayesexpt_b200.cuda_likelihood(source, entry) instead')
+        if likelihood_model is not None:
+            measurement_model = measurement_model.with_likelihood(likelihood_model)
+        #: 'gaussian', 'poisson', 'binomial' or a CudaLikelihood
+        self.likelihood_model = measurement_model.likelihood
+        if self.likelihood_model != 'gaussian':
+            self._likelihood_spec = self._counting_spec if isinstance(self.likelihood_model, str) else self._aux_spec
         ParticlePDF.__init__(self, parameter_samples, use_jit=use_jit, **kwargs)
         torch = self._torch
         self.model_function = measurement_model
@@ -287,6 +311,43 @@ class OptBayesExpt(ParticlePDF):
         n_lik = min(self.n_channels, len(y_meas), len(sigma))
         return y_meas[:n_lik], sigma[:n_lik], None, n_lik
 
+    def _counting_spec(self, measurement_record):
+        """Poisson (setting, counts[, ignored]) / binomial (setting, k, n_trials) records: (k[C], n_trials[C] |
+        None, None, n_lik), checked here so that a bad record raises before anything is enqueued."""
+        k = measurement_record[1]
+        if type(k) is float:                     # the common single-channel record, without numpy
+            if self.likelihood_model == 'poisson':
+                n = k
+            else:
+                n = measurement_record[2] if len(measurement_record) > 2 else None
+            if type(n) is float and 0.0 <= k <= n < math.inf and k == math.floor(k) and n == math.floor(n):
+                return (k,), (None if self.likelihood_model == 'poisson' else (n,)), None, 1
+        k = np.atleast_1d(np.asarray(measurement_record[1], dtype=np.float64))
+        n_lik = min(self.n_channels, len(k))
+        if self.likelihood_model == 'poisson':
+            k = k[:n_lik]
+            if not (np.all(np.isfinite(k)) and np.all(k >= 0) and np.all(k == np.floor(k))):
+                raise ValueError(f'Poisson counts must be finite non-negative integers, got {k}')
+            return k, None, None, n_lik
+        if len(measurement_record) < 3:
+            raise ValueError('a binomial record is (setting, k, n_trials)')
+        n = np.atleast_1d(np.asarray(measurement_record[2], dtype=np.float64))
+        n_lik = min(n_lik, len(n))
+        k, n = k[:n_lik], n[:n_lik]
+        if not (np.all(np.isfinite(k)) and np.all(np.isfinite(n)) and np.all(k >= 0) and np.all(k <= n)
+                and np.all(k == np.floor(k)) and np.all(n == np.floor(n))):
+            raise ValueError(f'binomial records need integers 0 <= k <= n_trials, got k={k}, n_trials={n}')
+        return k, n, None, n_lik
+
+    def _aux_spec(self, measurement_record):
+        """cuda_likelihood records (setting, y_meas, aux): (y_meas[C], aux[C], None, n_lik)."""
+        if len(measurement_record) < 3:
+            raise ValueError('a cuda_likelihood record is (setting, y_meas, aux)')
+        y_meas = np.atleast_1d(np.asarray(measurement_record[1], dtype=np.float64))
+        aux = np.atleast_1d(np.asarray(measurement_record[2], dtype=np.float64))
+        n_lik = min(self.n_channels, len(y_meas), len(aux))
+        return y_meas[:n_lik], aux[:n_lik], None, n_lik
+
     def pdf_update(self, measurement_record, y_model_data=None):
         """Bayesian update of the cloud from one measurement (obe_base.py:340-399).
 
@@ -328,11 +389,12 @@ class OptBayesExpt(ParticlePDF):
                     src = torch.as_tensor(np.ascontiguousarray(
                         np.asarray(y_model_data, dtype=np.float64).reshape(self.n_channels, -1)))
                 y[:, :self.n_particles].copy_(src[:, :self.n_particles])
-            self._check(self._lib.obe_update_from_y(self._cs(), C.c_void_p(y.data_ptr()), self._buf.ld,
-                                                    self.n_channels, _lib.darr(y_meas, _lib.MAX_CHANNELS),
-                                                    None if sigma is None else _lib.darr(sigma, _lib.MAX_CHANNELS),
-                                                    _lib.iarr(noise_index), n_lik, use_choke, choke, pivot,
-                                                    self._stream()))
+            self._check(self._lib.obe_update_from_y_model(self._model, self._cs(), C.c_void_p(y.data_ptr()),
+                                                          self._buf.ld, self.n_channels,
+                                                          _lib.darr(y_meas, _lib.MAX_CHANNELS),
+                                                          None if sigma is None else _lib.darr(sigma, _lib.MAX_CHANNELS),
+                                                          _lib.iarr(noise_index), n_lik, use_choke, choke, pivot,
+                                                          self._stream()))
         self._after_update()
         if self.just_resampled:
             self.enforce_parameter_constraints()
@@ -820,7 +882,8 @@ class OptBayesExpt(ParticlePDF):
             self._apply_constraint_masks(mask_le=le, mask_lt=lt, sync=False)
 
     def likelihood(self, y_model, measurement_record):
-        """Likelihood of the record for every particle (obe_base.py:418-461), on the device."""
+        """Likelihood of the record for every particle (obe_base.py:418-461), on the device, with the
+        ``likelihood_model`` of the engine (choke included)."""
         torch = self._torch
         y_meas, sigma, noise_index, n_lik = self._likelihood_spec(measurement_record)
         tmp = self._buf.empty_like(share_particles=True)
@@ -830,12 +893,13 @@ class OptBayesExpt(ParticlePDF):
         y[:, :self.n_particles].copy_(torch.as_tensor(
             np.ascontiguousarray(np.asarray(y_model, dtype=np.float64).reshape(self.n_channels, -1))))
         use_choke = 0 if self.choke is None else 1
-        self._check(self._lib.obe_update_from_y(C.byref(tmp.struct()), C.c_void_p(y.data_ptr()), self._buf.ld,
-                                                self.n_channels, _lib.darr(y_meas, _lib.MAX_CHANNELS),
-                                                None if sigma is None else _lib.darr(sigma, _lib.MAX_CHANNELS),
-                                                _lib.iarr(noise_index), n_lik, use_choke,
-                                                0.0 if self.choke is None else float(self.choke),
-                                                _lib.darr(self._pivot, _lib.MAX_PARAMS), self._stream()))
+        self._check(self._lib.obe_update_from_y_model(self._model, C.byref(tmp.struct()), C.c_void_p(y.data_ptr()),
+                                                      self._buf.ld, self.n_channels,
+                                                      _lib.darr(y_meas, _lib.MAX_CHANNELS),
+                                                      None if sigma is None else _lib.darr(sigma, _lib.MAX_CHANNELS),
+                                                      _lib.iarr(noise_index), n_lik, use_choke,
+                                                      0.0 if self.choke is None else float(self.choke),
+                                                      _lib.darr(self._pivot, _lib.MAX_PARAMS), self._stream()))
         return tmp.weights[:self.n_particles].cpu().numpy()
 
     # ------------------------------------------------------------------------------------------

@@ -8,6 +8,7 @@ pass, and the positivity constraint is applied as a bit mask by the refresh kern
 import numpy as np
 
 from .obe_base import OptBayesExpt
+from .models import non_gaussian as _non_gaussian
 
 
 class OptBayesExptNoiseParameter(OptBayesExpt):
@@ -15,6 +16,9 @@ class OptBayesExptNoiseParameter(OptBayesExpt):
 
     def __init__(self, measurement_model, setting_values, parameter_samples, constants,
                  noise_parameter_index=None, **kwargs):
+        if _non_gaussian(measurement_model, kwargs.get('likelihood_model')):
+            raise ValueError('a noise parameter is the sigma of the Gaussian likelihood: '
+                             f'{type(self).__name__} takes no other likelihood_model')
         OptBayesExpt.__init__(self, measurement_model, setting_values, parameter_samples, constants, **kwargs)
         self.noise_parameter_index = np.atleast_1d(noise_parameter_index)
         if noise_parameter_index is None or len(self.noise_parameter_index) != self.n_channels:

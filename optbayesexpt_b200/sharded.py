@@ -20,6 +20,7 @@ import os
 import numpy as np
 
 from . import _lib
+from .models import non_gaussian
 from .obe_base import OptBayesExpt
 
 
@@ -260,6 +261,9 @@ class ShardedOptBayesExpt(OptBayesExpt):
     def __init__(self, measurement_model, setting_values, parameter_samples, constants, group=None,
                  slack=0.25, seed=0, peer_exchange=None, **kwargs):
         import torch
+        if non_gaussian(measurement_model, kwargs.get('likelihood_model')):
+            raise ValueError('ShardedOptBayesExpt supports the Gaussian likelihood only; use OptBayesExpt for '
+                             'likelihood_model=\'poisson\' | \'binomial\' | cuda_likelihood(...)')
         self._comm = Comm(group)
         if peer_exchange is None:
             # default: on for a real multi-GPU job (nccl backend), off otherwise; OBE_PEER_EXCHANGE=0/1 overrides
