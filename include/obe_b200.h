@@ -161,6 +161,38 @@ int obe_materialize_weights(const obe_cloud_t* c, void* stream);
 /* Normalised weights (t * INVS, nan_to_num) into out_dev (n). particle_weights getter. */
 int obe_normalized_weights(const obe_cloud_t* c, double* out_dev, void* stream);
 
+/* ---- posterior summaries: quantiles and marginal histograms (csrc/obe_summary.cuh) ---------- */
+/* Read-only: the cloud, its weights and stats are not written.  Mass is u64 fixed point: a particle of
+ * normalised weight w (as obe_normalized_weights) carries wq = rint(w * 2^62); particles with wq == 0 are left
+ * out everywhere.  Integer sums make every result independent of the grid and of the run.  Each call ends
+ * with one stream synchronisation (the read of its small result into HOST memory).  params: host array of
+ * n_params (1..8) parameter rows.  Errors: parameter out of range, bad levels / bins / edges, an empty
+ * posterior (sum of wq == 0) and normalised weights that sum to 4 or more (sum of wq >= 2^64).  scratch_dev: device memory of the size the matching query returns. */
+size_t obe_quantile_scratch_bytes(int n_params, int n_q);
+size_t obe_histogram_scratch_bytes(int n_params, int bins);
+size_t obe_histogram2d_scratch_bytes(int bins_x, int bins_y);
+/* Streaming passes over the cloud that this thread's last summary call made (range pass included). */
+int obe_summary_passes(void);
+/* out[r * n_q + i]: the smallest coordinate x* of row params[r] with sum{wq : x <= x*} >= max(1, ceil(q_i W)),
+ * W = sum wq (exact).  q: n_q (1..16) levels in [0, 1].  q = 0 gives the minimum and q = 1 the maximum of the
+ * positive-weight particles; a zero answer is +0.0. */
+int obe_quantile(const obe_cloud_t* c, const int32_t* params, int n_params, const double* q, int n_q,
+                 void* scratch_dev, double* out, void* stream);
+/* lo_out / hi_out[r]: min / max coordinate of the positive-weight particles of row params[r] (the automatic
+ * histogram range).  scratch_dev: obe_histogram_scratch_bytes(n_params, 1) bytes. */
+int obe_summary_range(const obe_cloud_t* c, const int32_t* params, int n_params, void* scratch_dev, double* lo_out,
+                      double* hi_out, void* stream);
+/* Weighted 1-D histograms with np.histogram's uniform-bin rule.  edges: host (n_params, bins + 1), each row
+ * non-decreasing, finite, edges[0] < edges[bins]; bins 1..4096.  mass_out / count_out (count_out may be NULL):
+ * host (n_params, bins) u64 sums of wq and particle counts. */
+int obe_histogram(const obe_cloud_t* c, const int32_t* params, int n_params, const double* edges, int bins,
+                  void* scratch_dev, uint64_t* mass_out, uint64_t* count_out, void* stream);
+/* Joint histogram of rows param_x, param_y with np.histogram2d's rule; mass_out / count_out: host
+ * (bins_x, bins_y), bins_x * bins_y <= 65536. */
+int obe_histogram2d(const obe_cloud_t* c, int param_x, int param_y, const double* xedges, int bins_x,
+                    const double* yedges, int bins_y, void* scratch_dev, uint64_t* mass_out, uint64_t* count_out,
+                    void* stream);
+
 /* ---- weighted draws: Generator.choice(p=w) (particlepdf.py:330-331) ---------------------- */
 /* Canonical normalised CDF of the weights into cdf_dev (n). */
 int obe_cdf(const obe_cloud_t* c, double* cdf_dev, void* stream);

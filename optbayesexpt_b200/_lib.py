@@ -109,6 +109,16 @@ SIGNATURES = {
     'obe_fetch_stats': (C.c_int, [_PCLOUD, _PD, _VP]),
     'obe_materialize_weights': (C.c_int, [_PCLOUD, _VP]),
     'obe_normalized_weights': (C.c_int, [_PCLOUD, _VP, _VP]),
+    'obe_summary_passes': (C.c_int, []),
+    'obe_quantile_scratch_bytes': (C.c_size_t, [C.c_int, C.c_int]),
+    'obe_histogram_scratch_bytes': (C.c_size_t, [C.c_int, C.c_int]),
+    'obe_histogram2d_scratch_bytes': (C.c_size_t, [C.c_int, C.c_int]),
+    'obe_quantile': (C.c_int, [_PCLOUD, _PI32, C.c_int, _PD, C.c_int, _VP, _PD, _VP]),
+    'obe_summary_range': (C.c_int, [_PCLOUD, _PI32, C.c_int, _VP, _PD, _PD, _VP]),
+    'obe_histogram': (C.c_int, [_PCLOUD, _PI32, C.c_int, _PD, C.c_int, _VP, C.POINTER(C.c_uint64),
+                                C.POINTER(C.c_uint64), _VP]),
+    'obe_histogram2d': (C.c_int, [_PCLOUD, C.c_int, C.c_int, _PD, C.c_int, _PD, C.c_int, _VP,
+                                  C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), _VP]),
     'obe_cdf': (C.c_int, [_PCLOUD, _VP, _VP]),
     'obe_search': (C.c_int, [_PCLOUD, _VP, _VP, C.c_int64, _VP, _VP]),
     'obe_draw': (C.c_int, [_PCLOUD, _PD, C.c_int, _VP, _VP, _VP]),

@@ -12,7 +12,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 LIB = os.path.join(HERE, 'libobe_b200.so')
-SOURCES = ['obe_b200.cu', 'obe_device.cuh', 'obe_models.cuh']
+SOURCES = ['obe_b200.cu', 'obe_device.cuh', 'obe_models.cuh', 'obe_summary.cuh']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '-std=c++17',
               '-shared', '-Xcompiler', '-fPIC', '-cudart', 'static']
 

@@ -4040,3 +4040,5 @@ int obe_batch_select(obe_model_t m, const obe_batch_t* b, const double* settings
 }
 
 }  // extern "C"
+
+#include "obe_summary.cuh"

@@ -9,6 +9,8 @@ Differences a user can see (all deliberate, see DESIGN.md):
   * ``particles`` / ``particle_weights`` return READ-ONLY numpy mirrors downloaded on demand
     (assign a new array to change them; in-place edits would silently miss the device copy, so
     they raise instead).  ``particles_dev`` / ``weights_dev`` give the torch tensors, zero-copy.
+  * ``quantile`` / ``histogram`` / ``histogram2d`` summarise the posterior on the device
+    (summaries.py); only their small results reach the host.
   * ``resampling='systematic'`` (default) uses the fused systematic-comb kernel with Philox
     normals on the device; ``resampling='multinomial'`` reproduces the reference's
     ``Generator.choice`` + ``multivariate_normal`` exactly, consuming ``self.rng`` in the same
@@ -21,9 +23,10 @@ import numpy as np
 
 from . import _lib
 from .models import ParticleBuffers
+from .summaries import SummaryMixin
 
 
-class ParticlePDF:
+class ParticlePDF(SummaryMixin):
     """Weighted-particle probability distribution (particlepdf.py:12-145)."""
 
     def __init__(self, prior, a_param=0.98, resample_threshold=0.5, auto_resample=True, scale=True,

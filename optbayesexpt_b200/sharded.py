@@ -244,6 +244,10 @@ def gstats_from_plan(plan_host, d, world):
                 noise=g[_lib.ST_NOISE:_lib.ST_NOISE + 4].copy(), pivot=g[_lib.ST_PIVOT:_lib.ST_PIVOT + d].copy())
 
 
+_SUMMARY_REFUSAL = ('{} of a sharded cloud is not implemented yet (it needs an all-reduce of the fixed-point bins '
+                    'across shards); gather the cloud or use an unsharded engine')
+
+
 class ShardedOptBayesExpt(OptBayesExpt):
     """OptBayesExpt over a cloud sharded across the ranks of a process group.
 
@@ -416,6 +420,17 @@ class ShardedOptBayesExpt(OptBayesExpt):
     def n_eff(self):
         self._fetch_plan()
         return float(self._gmom[3])
+
+    # The inherited summaries would answer for this rank's shard alone.  The sharded version is one integer
+    # all-reduce of the fixed-point bins per pass (DESIGN.md §7); until it exists they refuse.
+    def quantile(self, q, params=None):
+        raise NotImplementedError(_SUMMARY_REFUSAL.format('quantile'))
+
+    def histogram(self, bins, range=None, params=None, return_counts=False):
+        raise NotImplementedError(_SUMMARY_REFUSAL.format('histogram'))
+
+    def histogram2d(self, i, j, bins, range=None, return_counts=False):
+        raise NotImplementedError(_SUMMARY_REFUSAL.format('histogram2d'))
 
     def resample_test(self):
         import warnings
