@@ -112,6 +112,23 @@ int obe_model_compile_likelihood(const char* builtin_name, const char* model_sou
                                  int n_settings, int n_params, int n_model_params, int n_constants,
                                  int n_channels, const char* likelihood, const char* likelihood_source,
                                  const char* likelihood_entry, obe_model_t* out, char* log, size_t log_len);
+/* The handle of obe_model_compile_likelihood whose utility kernel is likelihood-aware: the noise variance of
+ * setting s and channel c is the likelihood's own, averaged over the K draws,
+ *   v_c = (sum_k nu(y_kc, a_c)) / K  (summed sequentially over k),
+ *   poisson:  nu = y                (v_c is the mean of the K outputs),
+ *   binomial: nu = y (1 - y), then v_c /= a_c   (a_c: the planned trial count),
+ *   user:     nu = <noise_var_entry>(y, a_c), a `__device__ double f(double y_model, double aux)` defined in
+ *             `likelihood_source` (required for "user").
+ * Term of channel c: r_c = 0 where the spread is 0, else spread / v_c (+inf where v_c = 0); spread is var_p
+ * (variance), (max - min)^2 (max-min) or exp(2H)/(2 pi e) (pseudo).  A setting where some draw's output is
+ * invalid for the likelihood (poisson: lambda < 0 or not finite; binomial: p outside [0, 1] or NaN; user: nu
+ * negative or NaN) gets utility exactly 0.  obe_utility / obe_cycle read their var_noise[c] as a_c for such a
+ * handle and refuse the full-KLD method.  Everything else is what the plain likelihood handle does. */
+int obe_model_compile_likelihood_design(const char* builtin_name, const char* model_source, const char* model_entry,
+                                        int n_settings, int n_params, int n_model_params, int n_constants,
+                                        int n_channels, const char* likelihood, const char* likelihood_source,
+                                        const char* likelihood_entry, const char* noise_var_entry, obe_model_t* out,
+                                        char* log, size_t log_len);
 int obe_model_info(obe_model_t m, int* n_settings, int* n_model_params, int* n_constants,
                    int* n_channels, int* n_params);
 void obe_model_free(obe_model_t m);

@@ -96,6 +96,9 @@ SIGNATURES = {
     'obe_model_compile_likelihood': (C.c_int, [C.c_char_p, C.c_char_p, C.c_char_p, C.c_int, C.c_int, C.c_int, C.c_int,
                                                C.c_int, C.c_char_p, C.c_char_p, C.c_char_p, C.POINTER(_VP),
                                                C.c_char_p, C.c_size_t]),
+    'obe_model_compile_likelihood_design': (C.c_int, [C.c_char_p, C.c_char_p, C.c_char_p, C.c_int, C.c_int, C.c_int,
+                                                      C.c_int, C.c_int, C.c_char_p, C.c_char_p, C.c_char_p,
+                                                      C.c_char_p, C.POINTER(_VP), C.c_char_p, C.c_size_t]),
     'obe_model_info': (C.c_int, [_VP] + [C.POINTER(C.c_int)] * 5),
     'obe_model_free': (None, [_VP]),
     'obe_set_uniform': (C.c_int, [_PCLOUD, _VP]),

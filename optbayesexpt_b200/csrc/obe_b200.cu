@@ -2465,6 +2465,7 @@ struct obe_model {
     cudaLibrary_t lib;
     int lik;                // OBE_LIK_*: the measurement likelihood of the update kernels
     const void* f_update_y; // non-Gaussian handles: the update from a supplied y_model (OBE_SRC_Y)
+    int design;             // f_utility is the likelihood-aware utility: obe_utility reads var_noise[c] as the aux a_c
 };
 #define OBE_LIK_GAUSS 0
 #define OBE_LIK_POISSON 1
@@ -2719,10 +2720,13 @@ int obe_model_compile(const char* cuda_source, const char* entry, int n_settings
     return 0;
 }
 
-int obe_model_compile_likelihood(const char* builtin_name, const char* model_source, const char* model_entry,
-                                 int n_settings, int n_params, int n_model_params, int n_constants, int n_channels,
-                                 const char* likelihood, const char* likelihood_source, const char* likelihood_entry,
-                                 obe_model_t* out, char* log, size_t log_len) {
+// A non-Gaussian handle.  noise_var_entry == NULL: the plain likelihood handle, whose utility is today's
+// (var_noise[c] the noise variance).  design != 0: the same update kernels, and the likelihood-aware utility
+// (obe_k_utility_design: var_noise[c] is the design aux a_c; noise_var_entry names a user likelihood's variance).
+static int compile_likelihood(const char* builtin_name, const char* model_source, const char* model_entry,
+                              int n_settings, int n_params, int n_model_params, int n_constants, int n_channels,
+                              const char* likelihood, const char* likelihood_source, const char* likelihood_entry,
+                              int design, const char* noise_var_entry, obe_model_t* out, char* log, size_t log_len) {
     if (log && log_len) log[0] = 0;
     if (!out || !likelihood || (!builtin_name && (!model_source || !model_entry)))
         return obe_fail("null argument%s%s");
@@ -2734,6 +2738,8 @@ int obe_model_compile_likelihood(const char* builtin_name, const char* model_sou
     else return obe_fail("unknown likelihood '%s' (poisson, binomial or user)%s", likelihood);
     if (kind == OBE_LIK_USER && (!likelihood_source || !likelihood_entry))
         return obe_fail("a user likelihood needs its source and entry%s%s");
+    if (design && kind == OBE_LIK_USER && !noise_var_entry)
+        return obe_fail("a likelihood-aware design with a user likelihood needs its noise_var entry%s%s");
     obe_model tmp = {};
     std::string model_def;
     if (builtin_name) {
@@ -2770,23 +2776,60 @@ int obe_model_compile_likelihood(const char* builtin_name, const char* model_sou
                "        return ";
         src += likelihood_entry;
         src += "(y, ym, q.aux, n);\n    }\n};\ntypedef ObeLogLik<ObeUserPmf> ObeUserLik;\n";
+        if (design) {
+            src += "struct ObeUserNoise {\n"
+                   "    static constexpr bool LIK = true;\n"
+                   "    static constexpr bool NU_IS_Y = false;\n"
+                   "    __device__ static __forceinline__ double nu(double y, double a) { return ";
+            src += noise_var_entry;
+            src += "(y, a); }\n"
+                   "    __device__ static __forceinline__ bool ok(double, double v) { return v >= 0.0; }\n"
+                   "    __device__ static __forceinline__ double finish(double m, double) { return m; }\n};\n";
+        }
     }
+    const char* noise_type = kind == OBE_LIK_POISSON ? "ObePoissonNoise"
+                             : (kind == OBE_LIK_BINOMIAL ? "ObeBinomialNoise" : "ObeUserNoise");
     char tail[512];
-    snprintf(tail, sizeof(tail),
-             "OBE_DEFINE_LIK_KERNELS(ObeLikModel, %s, %d)\n"
-             "OBE_DEFINE_GRID_KERNELS(ObeLikModel, lik)\n", lik_type, n_params);
+    if (design)
+        snprintf(tail, sizeof(tail),
+                 "OBE_DEFINE_LIK_KERNELS(ObeLikModel, %s, %d)\n"
+                 "OBE_DEFINE_DESIGN_KERNELS(ObeLikModel, %s)\n", lik_type, n_params, noise_type);
+    else
+        snprintf(tail, sizeof(tail),
+                 "OBE_DEFINE_LIK_KERNELS(ObeLikModel, %s, %d)\n"
+                 "OBE_DEFINE_GRID_KERNELS(ObeLikModel, lik)\n", lik_type, n_params);
     src += tail;
     std::vector<char> cubin;
     if (nvrtc_cubin(src, "obe_likelihood_model.cu", cubin, log, log_len)) return -1;
     obe_model* m = new obe_model(tmp);
-    m->d = n_params; m->user = true; m->lik = kind;
+    m->d = n_params; m->user = true; m->lik = kind; m->design = design ? 1 : 0;
     const void* k[5];
     const char* kn[5] = {"obe_k_update_lik", "obe_k_updatey_lik", "obe_k_evalp_lik", "obe_k_utility_lik",
                          "obe_k_evals_lik"};
+    if (design) { kn[3] = "obe_k_utility_design"; kn[4] = "obe_k_evals_design"; }
     if (load_kernels(m, cubin, kn, k, 5)) return -1;
     m->f_update = k[0]; m->f_update_y = k[1]; m->f_evalp = k[2]; m->f_utility = k[3]; m->f_evals = k[4];
     *out = m;
     return 0;
+}
+
+int obe_model_compile_likelihood(const char* builtin_name, const char* model_source, const char* model_entry,
+                                 int n_settings, int n_params, int n_model_params, int n_constants, int n_channels,
+                                 const char* likelihood, const char* likelihood_source, const char* likelihood_entry,
+                                 obe_model_t* out, char* log, size_t log_len) {
+    return compile_likelihood(builtin_name, model_source, model_entry, n_settings, n_params, n_model_params,
+                              n_constants, n_channels, likelihood, likelihood_source, likelihood_entry, 0, nullptr, out,
+                              log, log_len);
+}
+
+int obe_model_compile_likelihood_design(const char* builtin_name, const char* model_source, const char* model_entry,
+                                        int n_settings, int n_params, int n_model_params, int n_constants,
+                                        int n_channels, const char* likelihood, const char* likelihood_source,
+                                        const char* likelihood_entry, const char* noise_var_entry, obe_model_t* out,
+                                        char* log, size_t log_len) {
+    return compile_likelihood(builtin_name, model_source, model_entry, n_settings, n_params, n_model_params,
+                              n_constants, n_channels, likelihood, likelihood_source, likelihood_entry, 1,
+                              noise_var_entry, out, log, log_len);
 }
 
 int obe_model_info(obe_model_t m, int* ns, int* npm, int* nc, int* nch, int* np) {
@@ -3707,6 +3750,9 @@ int obe_utility(obe_model_t m, const double* draws_dev, int k, const double* set
     if (method < 0 || method > 3) return obe_fail("unknown utility method%s%s");
     if (method >= 2 && (k < 3 || k > OBE_MAX_DRAWS)) return obe_fail("entropy utilities need 3 <= n_draws <= 128%s%s");
     if (method == 3 && (!kld_noise_dev || m->nch != 1)) return obe_fail("full KLD utility: single-channel models, noise required%s%s");
+    if (method == 3 && m->design)
+        return obe_fail("full KLD utility: its noise samples are Gaussian; a likelihood-aware design handle has none%s%s");
+    if (m->design && !var_noise) return obe_fail("a likelihood-aware design handle needs the design aux in var_noise%s%s");
     if (!var_noise && !stats_dev) return obe_fail("need var_noise or stats%s%s");
     if (k < 1) return obe_fail("n_draws must be >= 1%s%s");
     if (obe_sms() <= 0) return obe_fail("no CUDA device: this library has no CPU fallback%s%s");

@@ -1478,7 +1478,40 @@ __device__ __forceinline__ void obe_block_argmax(double& best, long long& besti,
     }
 }
 
-template <class Model>
+// ---- noise variance of the design half ---------------------------------------------------------------------------
+// The utility divides the spread of the K model curves at a setting by a noise variance.  ObeFixedNoise (the default,
+// every pre-instantiated kernel): the constant var_noise[c], or the noise-parameter estimate.  A likelihood policy
+// (design_noise='likelihood', NVRTC modules only) uses the likelihood's own variance averaged over the K draws,
+// v_c = finish((sum_k nu(y_kc, a_c)) / K, a_c), summed sequentially over k, with a_c = var_noise[c] read as the design
+// aux; r_c = 0 where the spread is 0, spread / v_c otherwise (+inf where v_c = 0).  A setting where some draw's output
+// is invalid for the likelihood (ok() false) gets utility 0.
+struct ObeFixedNoise {
+    static constexpr bool LIK = false;
+    static constexpr bool NU_IS_Y = false;
+};
+// Poisson: variance lambda.  nu = y, so v_c is the mean of the variance pass itself.  lambda < 0 / NaN / inf invalid.
+struct ObePoissonNoise {
+    static constexpr bool LIK = true;
+    static constexpr bool NU_IS_Y = true;
+    __device__ static __forceinline__ double nu(double y, double) { return y; }
+    __device__ static __forceinline__ bool ok(double y, double) { return y >= 0.0 && y <= 1.7976931348623157e308; }
+    __device__ static __forceinline__ double finish(double m, double) { return m; }
+};
+// Binomial in probability units: variance p (1 - p) / n, n = a_c the planned trials.  p outside [0, 1] / NaN invalid.
+struct ObeBinomialNoise {
+    static constexpr bool LIK = true;
+    static constexpr bool NU_IS_Y = false;
+    __device__ static __forceinline__ double nu(double y, double) { return obe_mul(y, obe_sub(1.0, y)); }
+    __device__ static __forceinline__ bool ok(double y, double) { return y >= 0.0 && y <= 1.0; }
+    __device__ static __forceinline__ double finish(double m, double a) { return obe_div(m, a); }
+};
+// (a user likelihood's policy, nu = its noise_var(y, a), negative or NaN invalid, is generated with its source by
+// obe_model_compile_likelihood_design)
+__device__ __forceinline__ double obe_design_ratio(double spread, double v) {
+    return spread == 0.0 ? 0.0 : obe_div(spread, v);
+}
+
+template <class Model, class Noise = ObeFixedNoise>
 __device__ void obe_utility_body(const ObeUtilityArgs& a) {
     extern __shared__ double obe_smem[];
     double* sdraw = obe_smem;  // [K][NP]
@@ -1537,20 +1570,35 @@ __device__ void obe_utility_body(const ObeUtilityArgs& a) {
             __syncwarp();
             if (valid && g == 0) {
                 double u = 0.0;
+                bool ok = true;
 #pragma unroll
                 for (int c = 0; c < Model::NCH; ++c) {
                     const double* yc = yv + c * K;
-                    double mean = 0.0, ss = 0.0;
-                    for (int k = 0; k < K; ++k) mean = obe_add(mean, yc[k]);
+                    double mean = 0.0, ss = 0.0, nus = 0.0;
+                    for (int k = 0; k < K; ++k) {
+                        mean = obe_add(mean, yc[k]);
+                        if constexpr (Noise::LIK) {        // the first lane sums nu beside the mean
+                            const double nu = Noise::nu(yc[k], var_n[c]);
+                            if constexpr (!Noise::NU_IS_Y) nus = obe_add(nus, nu);
+                            ok = ok & Noise::ok(yc[k], nu);
+                        }
+                    }
                     mean = obe_div(mean, kd);
                     for (int k = 0; k < K; ++k) {
                         const double dlt = obe_sub(yc[k], mean);
                         ss = obe_add(ss, obe_mul(dlt, dlt));
                     }
-                    const double r = obe_div(obe_div(ss, kd), var_n[c]);
+                    double r;
+                    if constexpr (Noise::LIK) {
+                        const double v = Noise::finish(Noise::NU_IS_Y ? mean : obe_div(nus, kd), var_n[c]);
+                        r = obe_design_ratio(obe_div(ss, kd), v);
+                    } else {
+                        r = obe_div(obe_div(ss, kd), var_n[c]);
+                    }
                     u = obe_add(u, a.log_form ? log(obe_add(1.0, r)) : r);
                 }
                 if (a.cost) u = obe_div(u, a.cost[s]);
+                if constexpr (Noise::LIK) u = ok ? u : 0.0;
                 a.utility[s] = u;
                 const bool unan = (u != u), bnan = (best != best);
                 if (!have || (!bnan && (unan || u > best))) { best = u; besti = s; have = true; }
@@ -1565,6 +1613,12 @@ __device__ void obe_utility_body(const ObeUtilityArgs& a) {
         for (int j = 0; j < Model::NS; ++j) st[j] = a.settings[j * a.lds + s];
         double y[Model::NCH];
         double u = 0.0;
+        bool ok = true;                                  // (likelihood noise: every draw's output is valid here)
+        double nus[Noise::LIK ? Model::NCH : 1];         // (likelihood noise: sum_k nu(y_kc, a_c))
+        if constexpr (Noise::LIK) {
+#pragma unroll
+            for (int c = 0; c < Model::NCH; ++c) nus[c] = 0.0;
+        }
         if (a.method == 0) {
             double mean[Model::NCH], ss[Model::NCH];
 #pragma unroll
@@ -1580,6 +1634,11 @@ __device__ void obe_utility_body(const ObeUtilityArgs& a) {
                 for (int c = 0; c < Model::NCH; ++c) {
                     mean[c] = obe_add(mean[c], y[c]);
                     if (a.cache) ycol[(k * Model::NCH + c) * blockDim.x] = y[c];
+                    if constexpr (Noise::LIK) {        // nu is summed in pass 1
+                        const double nu = Noise::nu(y[c], var_n[c]);
+                        if constexpr (!Noise::NU_IS_Y) nus[c] = obe_add(nus[c], nu);
+                        ok = ok & Noise::ok(y[c], nu);
+                    }
                 }
             }
 #pragma unroll
@@ -1600,7 +1659,13 @@ __device__ void obe_utility_body(const ObeUtilityArgs& a) {
 #pragma unroll
             for (int c = 0; c < Model::NCH; ++c) {
                 const double var_p = obe_div(ss[c], kd);
-                const double r = obe_div(var_p, var_n[c]);
+                double r;
+                if constexpr (Noise::LIK) {
+                    const double v = Noise::finish(Noise::NU_IS_Y ? mean[c] : obe_div(nus[c], kd), var_n[c]);
+                    r = obe_design_ratio(var_p, v);
+                } else {
+                    r = obe_div(var_p, var_n[c]);
+                }
                 u = obe_add(u, a.log_form ? log(obe_add(1.0, r)) : r);
             }
         } else if (a.method >= 2) {
@@ -1614,6 +1679,11 @@ __device__ void obe_utility_body(const ObeUtilityArgs& a) {
 #pragma unroll
                     for (int cc = 1; cc < Model::NCH; ++cc)
                         if (cc == c) v = y[cc];
+                    if constexpr (Noise::LIK) {
+                        const double nu = Noise::nu(v, var_n[c]);
+                        nus[c] = obe_add(nus[c], nu);
+                        ok = ok & Noise::ok(v, nu);
+                    }
                     if (a.method == 3) v = obe_add(v, a.kld_noise[k * Model::NCH + c]);
                     ys[k] = v;
                 }
@@ -1622,7 +1692,9 @@ __device__ void obe_utility_body(const ObeUtilityArgs& a) {
                 if (a.method == 2) {
                     // yvar_from_entropy: exp(2H)/(2 pi e)  (obe_base.py:516-517), then var/var_n
                     const double var_p = exp(2.0 * h) / (2.0 * 3.141592653589793 * 2.718281828459045);
-                    const double r = obe_div(var_p, var_n[c]);
+                    double r;
+                    if constexpr (Noise::LIK) r = obe_design_ratio(var_p, Noise::finish(obe_div(nus[c], kd), var_n[c]));
+                    else r = obe_div(var_p, var_n[c]);
                     u = obe_add(u, a.log_form ? log(obe_add(1.0, r)) : r);
                 } else {
                     u = exp(h - s_noise_entropy[c]) - 1.0;      // obe_base.py:717-720 (single channel)
@@ -1637,16 +1709,24 @@ __device__ void obe_utility_body(const ObeUtilityArgs& a) {
                 for (int c = 0; c < Model::NCH; ++c) {
                     mx[c] = (k == 0 || y[c] > mx[c]) ? y[c] : mx[c];
                     mn[c] = (k == 0 || y[c] < mn[c]) ? y[c] : mn[c];
+                    if constexpr (Noise::LIK) {
+                        const double nu = Noise::nu(y[c], var_n[c]);
+                        nus[c] = obe_add(nus[c], nu);
+                        ok = ok & Noise::ok(y[c], nu);
+                    }
                 }
             }
 #pragma unroll
             for (int c = 0; c < Model::NCH; ++c) {
                 const double span = obe_sub(mx[c], mn[c]);
-                const double r = obe_div(obe_mul(span, span), var_n[c]);
+                double r;
+                if constexpr (Noise::LIK) r = obe_design_ratio(obe_mul(span, span), Noise::finish(obe_div(nus[c], kd), var_n[c]));
+                else r = obe_div(obe_mul(span, span), var_n[c]);
                 u = obe_add(u, a.log_form ? log(obe_add(1.0, r)) : r);
             }
         }
         if (a.cost) u = obe_div(u, a.cost[s]);
+        if constexpr (Noise::LIK) u = ok ? u : 0.0;
         a.utility[s] = u;
         // np.argmax: first maximum, NaN counts as the maximum
         const bool unan = (u != u), bnan = (best != best);
@@ -2109,6 +2189,16 @@ struct ObeNoModel {
     }                                                                                                          \
     extern "C" __global__ void __launch_bounds__(OBE_THREADS) obe_k_evalp_lik(const ObeEvalArgs a) {           \
         obe_eval_params_body<MODEL, D>(a);                                                                     \
+    }
+
+// The utility of a likelihood-aware design (design_noise='likelihood'): var_noise[c] is the design aux a_c and NOISE
+// the likelihood's noise-variance policy.  Compiled by NVRTC per handle, beside OBE_DEFINE_LIK_KERNELS.
+#define OBE_DEFINE_DESIGN_KERNELS(MODEL, NOISE)                                                               \
+    extern "C" __global__ void __launch_bounds__(OBE_THREADS) obe_k_utility_design(const ObeUtilityArgs a) {  \
+        obe_utility_body<MODEL, NOISE>(a);                                                                    \
+    }                                                                                                         \
+    extern "C" __global__ void __launch_bounds__(OBE_THREADS) obe_k_evals_design(const ObeEvalArgs a) {       \
+        obe_eval_settings_body<MODEL>(a);                                                                     \
     }
 
 #define OBE_DEFINE_GRID_KERNELS(MODEL, SUFFIX)                                                             \

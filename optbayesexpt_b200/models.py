@@ -34,7 +34,7 @@ class DeviceModel:
     """
 
     def __init__(self, name, n_settings, n_model_params, n_constants, n_channels, source=None, entry=None,
-                 likelihood='gaussian'):
+                 likelihood='gaussian', design_noise='fixed'):
         self.name = name
         self.n_settings = n_settings
         self.n_model_params = n_model_params
@@ -44,26 +44,40 @@ class DeviceModel:
         self.entry = entry
         #: measurement likelihood of the update kernels: 'gaussian', 'poisson', 'binomial' or a CudaLikelihood
         self.likelihood = likelihood
+        #: noise variance of the utility kernel: 'fixed' (the engine's yvar_noise_model()) or 'likelihood' (the
+        #: likelihood's own variance at each setting; non-Gaussian likelihoods only)
+        self.design_noise = design_noise
         self._handles = {}
         self._variants = {}
         self.compile_log = ''
 
-    def with_likelihood(self, likelihood):
+    def with_likelihood(self, likelihood, design_noise='fixed'):
         """The same model with another measurement likelihood ('gaussian', 'poisson', 'binomial' or
-        :func:`cuda_likelihood`).  A non-Gaussian model is compiled by NVRTC on first use."""
+        :func:`cuda_likelihood`).  A non-Gaussian model is compiled by NVRTC on first use.
+
+        ``design_noise='likelihood'`` gives the variant whose utility kernel divides by the likelihood's own noise
+        variance (see ``OptBayesExpt(..., design_noise=)``); a Gaussian model has only the 'fixed' one."""
         if isinstance(likelihood, str):
             if likelihood not in LIKELIHOODS:
                 raise ValueError(f'unknown likelihood_model {likelihood!r}; have {list(LIKELIHOODS)} or cuda_likelihood(...)')
         elif not isinstance(likelihood, CudaLikelihood):
             raise TypeError('likelihood_model must be one of '
                             f'{list(LIKELIHOODS)} or optbayesexpt_b200.cuda_likelihood(source, entry)')
-        if likelihood == self.likelihood:
+        if design_noise not in DESIGN_NOISES:
+            raise ValueError(f'design_noise must be one of {list(DESIGN_NOISES)}, got {design_noise!r}')
+        if likelihood == 'gaussian':
+            design_noise = 'fixed'                  # (the Gaussian noise variance is the fixed one by definition)
+        elif design_noise == 'likelihood' and isinstance(likelihood, CudaLikelihood) and likelihood.noise_var is None:
+            raise ValueError("design_noise='likelihood' with a cuda_likelihood needs its noise_var entry: "
+                             'cuda_likelihood(source, entry, noise_var=...)')
+        if likelihood == self.likelihood and design_noise == self.design_noise:
             return self
-        if likelihood not in self._variants:        # (one NVRTC compile per likelihood and n_params)
-            self._variants[likelihood] = DeviceModel(self.name, self.n_settings, self.n_model_params,
-                                                     self.n_constants, self.n_channels, source=self.source,
-                                                     entry=self.entry, likelihood=likelihood)
-        return self._variants[likelihood]
+        key = (likelihood, design_noise)
+        if key not in self._variants:               # (one NVRTC compile per variant and n_params)
+            self._variants[key] = DeviceModel(self.name, self.n_settings, self.n_model_params, self.n_constants,
+                                              self.n_channels, source=self.source, entry=self.entry,
+                                              likelihood=likelihood, design_noise=design_noise)
+        return self._variants[key]
 
     def handle(self, n_params):
         """obe_model_t for a cloud with ``n_params`` rows."""
@@ -76,14 +90,18 @@ class DeviceModel:
         if self.likelihood != 'gaussian':
             log = C.create_string_buffer(1 << 16)
             user = isinstance(self.likelihood, CudaLikelihood)
-            rc = lib.obe_model_compile_likelihood(
-                self.name.encode() if self.source is None else None,
-                None if self.source is None else self.source.encode(),
-                None if self.source is None else self.entry.encode(),
-                self.n_settings, n_params, self.n_model_params, self.n_constants, self.n_channels,
-                b'user' if user else self.likelihood.encode(),
-                self.likelihood.source.encode() if user else None,
-                self.likelihood.entry.encode() if user else None, C.byref(h), log, len(log))
+            args = (self.name.encode() if self.source is None else None,
+                    None if self.source is None else self.source.encode(),
+                    None if self.source is None else self.entry.encode(),
+                    self.n_settings, n_params, self.n_model_params, self.n_constants, self.n_channels,
+                    b'user' if user else self.likelihood.encode(),
+                    self.likelihood.source.encode() if user else None,
+                    self.likelihood.entry.encode() if user else None)
+            if self.design_noise == 'likelihood':
+                nv = self.likelihood.noise_var.encode() if user else None
+                rc = lib.obe_model_compile_likelihood_design(*args, nv, C.byref(h), log, len(log))
+            else:
+                rc = lib.obe_model_compile_likelihood(*args, C.byref(h), log, len(log))
             self.compile_log = log.value.decode(errors='replace')
             _lib.check(rc)
         elif self.source is None:
@@ -149,29 +167,36 @@ class DeviceModel:
     def __repr__(self):
         kind = 'builtin' if self.source is None else 'nvrtc'
         lik = '' if self.likelihood == 'gaussian' else f', likelihood={self.likelihood!r}'
+        if self.design_noise != 'fixed':
+            lik += f', design_noise={self.design_noise!r}'
         return (f'DeviceModel({self.name!r}, {kind}, settings={self.n_settings}, params={self.n_model_params}, '
                 f'constants={self.n_constants}, channels={self.n_channels}{lik})')
 
 
 #: the measurement likelihoods of the update kernel, by name (a user likelihood is a :func:`cuda_likelihood`)
 LIKELIHOODS = ('gaussian', 'poisson', 'binomial')
+#: the noise variance the utility divides by: the engine's fixed one, or the likelihood's own at each setting
+DESIGN_NOISES = ('fixed', 'likelihood')
 
 
 class CudaLikelihood:
     """A measurement likelihood as CUDA source: see :func:`cuda_likelihood`."""
 
-    def __init__(self, source, entry):
+    def __init__(self, source, entry, noise_var=None):
         self.source = source
         self.entry = entry
+        self.noise_var = noise_var
 
     def __eq__(self, other):
-        return isinstance(other, CudaLikelihood) and (self.source, self.entry) == (other.source, other.entry)
+        return isinstance(other, CudaLikelihood) and \
+            (self.source, self.entry, self.noise_var) == (other.source, other.entry, other.noise_var)
 
     def __hash__(self):
-        return hash((self.source, self.entry))
+        return hash((self.source, self.entry, self.noise_var))
 
     def __repr__(self):
-        return f'cuda_likelihood(entry={self.entry!r})'
+        nv = '' if self.noise_var is None else f', noise_var={self.noise_var!r}'
+        return f'cuda_likelihood(entry={self.entry!r}{nv})'
 
 
 def non_gaussian(measurement_model, likelihood_model=None):
@@ -181,7 +206,7 @@ def non_gaussian(measurement_model, likelihood_model=None):
     return isinstance(measurement_model, DeviceModel) and measurement_model.likelihood != 'gaussian'
 
 
-def cuda_likelihood(source, entry):
+def cuda_likelihood(source, entry, noise_var=None):
     """User measurement likelihood for ``OptBayesExpt(..., likelihood_model=...)``, compiled by NVRTC with the model.
 
     ``source`` must define ``__device__ double <entry>(const double* y_model, const double* y_meas,
@@ -190,8 +215,13 @@ def cuda_likelihood(source, entry):
     level, trial counts, anything per channel), both cut to ``n_channels`` entries.  The weight factor is
     ``exp(choke * log L)``; log L may be positive.  This replaces overriding ``likelihood`` in Python, which
     cannot run inside the update kernel.
+
+    ``noise_var`` (optional) names a second function of ``source``, ``__device__ double <noise_var>(double y_model,
+    double aux)``: the variance of one channel's measurement given its model output and the design aux.  It is
+    what ``OptBayesExpt(..., design_noise='likelihood')`` divides the utility by (averaged over the draws), and
+    that mode requires it.  A negative or NaN value marks the output as impossible: the setting's utility is 0.
     """
-    return CudaLikelihood(source, entry)
+    return CudaLikelihood(source, entry, noise_var)
 
 
 def builtin(name):

@@ -14,7 +14,7 @@ import math
 import numpy as np
 
 from . import _lib
-from .models import DeviceModel, builtin
+from .models import DESIGN_NOISES, DeviceModel, builtin
 from .particlepdf import ParticlePDF
 
 DEFAULT_N_DRAWS = 30
@@ -64,14 +64,25 @@ class OptBayesExpt(ParticlePDF):
     - :func:`~optbayesexpt_b200.models.cuda_likelihood`: a log-likelihood in CUDA, records
       ``(setting, y_meas, aux)``.
 
-    The design half is the same for every likelihood: the utility divides by ``yvar_noise_model()``, so
-    for counting data ``default_noise_std`` sets the noise scale of the utility (e.g. about sqrt of a typical
-    count).  Overriding ``likelihood`` in Python raises ``TypeError``: it could not run inside the kernel.
+    ``design_noise`` selects the noise variance the utility divides the spread of the model curves by:
+
+    - ``'fixed'`` (the default): ``yvar_noise_model()``, the same at every setting; for counting data
+      ``default_noise_std`` then sets the noise scale of the utility (e.g. about sqrt of a typical count);
+    - ``'likelihood'``: the likelihood's own noise variance at each setting, averaged over the drawn parameter
+      sets -- the expected count for Poisson, p (1 - p) / n for binomial with ``n = design_aux`` the planned trials
+      of the next measurement (required), the ``noise_var`` function of a ``cuda_likelihood`` (required) at
+      ``aux = design_aux`` (default 1).  A setting where some draw's model output is impossible for the likelihood
+      gets utility 0.  On a Gaussian engine this is the fixed variance by definition.  Not with
+      ``full_kld_utility``, whose noise samples are Gaussian.
+
+    ``design_aux`` is a scalar or one value per channel, finite and > 0, and may be reassigned between cycles.
+    Overriding ``likelihood`` in Python raises ``TypeError``: it could not run inside the kernel.
     """
 
     def __init__(self, measurement_model, setting_values, parameter_samples, constants,
                  n_draws=DEFAULT_N_DRAWS, choke=None, use_jit=True, utility_method='variance_approx',
-                 selection_method='optimal', pickiness=15, default_noise_std=1.0, likelihood_model=None, **kwargs):
+                 selection_method='optimal', pickiness=15, default_noise_std=1.0, likelihood_model=None,
+                 design_noise='fixed', design_aux=None, **kwargs):
         if isinstance(measurement_model, str):
             measurement_model = builtin(measurement_model)
         if not isinstance(measurement_model, DeviceModel):
@@ -83,6 +94,22 @@ class OptBayesExpt(ParticlePDF):
                             'optbayesexpt_b200.cuda_likelihood(source, entry) instead')
         if likelihood_model is not None:
             measurement_model = measurement_model.with_likelihood(likelihood_model)
+        if design_noise not in DESIGN_NOISES:
+            raise ValueError(f'design_noise must be one of {list(DESIGN_NOISES)}, got {design_noise!r}')
+        #: 'fixed' or 'likelihood': the noise variance of the utility (see the class documentation)
+        self.design_noise = design_noise
+        # the likelihood-aware utility kernel runs only for a non-Gaussian likelihood
+        self._design_lik = design_noise == 'likelihood' and measurement_model.likelihood != 'gaussian'
+        if self._design_lik:
+            if utility_method == 'full_kld_utility':
+                raise ValueError("design_noise='likelihood' does not apply to full_kld_utility: its noise samples "
+                                 'are Gaussian draws')
+            if measurement_model.likelihood == 'binomial' and design_aux is None:
+                raise ValueError("design_noise='likelihood' with a binomial likelihood needs design_aux, the planned "
+                                 'number of trials of the next measurement')
+            measurement_model = measurement_model.with_likelihood(measurement_model.likelihood, 'likelihood')
+        elif measurement_model.design_noise != 'fixed':
+            measurement_model = measurement_model.with_likelihood(measurement_model.likelihood)
         #: 'gaussian', 'poisson', 'binomial' or a CudaLikelihood
         self.likelihood_model = measurement_model.likelihood
         if self.likelihood_model != 'gaussian':
@@ -117,6 +144,7 @@ class OptBayesExpt(ParticlePDF):
         self.n_channels = measurement_model.n_channels
         self.utility_y_space = np.array([])   # never materialised on the device path
         self.default_noise_std = np.ones((self.n_channels, 1)) * default_noise_std
+        self.design_aux = design_aux
 
         utilitymethods = ['variance_approx', 'pseudo_utility', 'full_kld_utility', 'max_min']
         if utility_method == 'variance_approx':
@@ -715,7 +743,7 @@ class OptBayesExpt(ParticlePDF):
             cy.method = self._utility_code
             cy.log_form = 1 if self.utility_log_form else 0
             if not cy.noise_from_stats:
-                vn = np.asarray(self.yvar_noise_model(), dtype=np.float64).reshape(-1)
+                vn = np.asarray(self._design_var_noise(), dtype=np.float64).reshape(-1)
                 self._cy_vn[:min(len(vn), _lib.MAX_CHANNELS)] = vn[:_lib.MAX_CHANNELS]
         if self.early_select and resample and select:
             # (small clouds: same early order on the main stream -- the fork / join cost more than the overlap hides)
@@ -905,6 +933,36 @@ class OptBayesExpt(ParticlePDF):
     # ------------------------------------------------------------------------------------------
     # design half (obe_base.py:463-805)
     # ------------------------------------------------------------------------------------------
+    @property
+    def design_aux(self):
+        """Per-channel aux of the likelihood-aware utility (``design_noise='likelihood'``): the planned trials of the
+        next binomial measurement, the ``aux`` of a cuda_likelihood's ``noise_var``.  Read at every selection."""
+        return self._design_aux
+
+    @design_aux.setter
+    def design_aux(self, value):
+        if value is None:
+            if self._design_lik and self.likelihood_model == 'binomial':
+                raise ValueError("design_noise='likelihood' with a binomial likelihood needs design_aux")
+            arr = np.ones(self.n_channels)
+        else:
+            arr = np.asarray(value, dtype=np.float64).reshape(-1)
+            if arr.size == 1:
+                arr = np.full(self.n_channels, arr[0])
+            if arr.size != self.n_channels:
+                raise ValueError(f'design_aux needs a scalar or {self.n_channels} values, got {arr.size}')
+            if not (np.all(np.isfinite(arr)) and np.all(arr > 0)):
+                raise ValueError(f'design_aux must be finite and > 0, got {value!r}')
+        self._design_aux = value
+        self._design_aux_arr = arr
+
+    def _design_var_noise(self):
+        """What the utility kernel divides by: the design aux for a likelihood-aware handle (whose kernel computes
+        the noise variance itself), yvar_noise_model() otherwise."""
+        if self._design_lik:
+            return self._design_aux_arr
+        return self.yvar_noise_model()
+
     def y_var_noise_model(self):
         return self.yvar_noise_model()
 
@@ -943,7 +1001,7 @@ class OptBayesExpt(ParticlePDF):
             var_noise = None
             stats_ptr = C.c_void_p(self._buf.stats.data_ptr())
         else:
-            vn = np.asarray(self.yvar_noise_model(), dtype=np.float64)
+            vn = np.asarray(self._design_var_noise(), dtype=np.float64)
             key = vn.tobytes()
             cache = self._var_noise_cache
             if cache is None or cache[0] != key:
@@ -993,6 +1051,9 @@ class OptBayesExpt(ParticlePDF):
         """The utility of method `code` whatever ``utility_method`` the engine was built with."""
         if code == 3 and self.n_channels != 1:
             raise ValueError('full_kld_utility supports single-channel models')
+        if code == 3 and self._design_lik:
+            raise ValueError("full_kld_utility is not available with design_noise='likelihood': its noise samples "
+                             'are Gaussian draws')
         saved = self._utility_code
         self._utility_code = code
         try:
