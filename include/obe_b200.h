@@ -77,6 +77,8 @@ int obe_device_count(void);
  * which the resample plan runs on a thread-block cluster of 8 CTAs instead of one CTA (default 8192).
  * "utility_lane_fill": the variance utility uses 8/4/2 lanes per setting while n_settings * lanes stays
  * below this percentage of the resident thread count (default 50; 0 = always one thread per setting).
+ * "utility_info_blocks": > 0 caps the grid of the information-gain utility (method 4) at that many CTAs
+ * (default 0: one CTA per 8 settings, at most 8 per SM); its result does not depend on the grid.
  * Returns 0, or -1 for an unknown name. */
 int obe_set_option(const char* name, int64_t value);                 /* 0 without a usable CUDA device                */
 int64_t obe_num_tiles(int64_t n);
@@ -351,7 +353,7 @@ typedef struct obe_cycle {
     int64_t lds, n_settings;
     double var_noise[OBE_MAX_CHANNELS];
     int32_t noise_from_stats;           /* 1: var_noise is ignored, the noise sums of the live stats block are used */
-    int32_t method, log_form, pad0;
+    int32_t method, log_form, pad0;     /* method: the obe_utility code (0 variance .. 4 information gain) */
     const double* cost_dev;
     const double* kld_noise_dev;
     double* utility_dev;
@@ -409,7 +411,12 @@ int obe_draw_strided(const obe_cloud_t* c, const double* u_host, int m, double* 
  * the noise-parameter accumulators of c_stats_dev (obe_noiseparam.py:132-136); cost_dev (S) or
  * NULL (cost_estimate, obe_base.py:566-577); method 0 = variance, 1 = max-min
  * (obe_base.py:602-626), 2 = pseudo (spacing-entropy of the K outputs, obe_base.py:491-518,657-686),
- * 3 = full KLD (obe_base.py:688-720; kld_noise_dev = (K, C) noise samples, single channel);
+ * 3 = full KLD (obe_base.py:688-720; kld_noise_dev = (K, C) noise samples, single channel),
+ * 4 = information gain: the mutual information I(theta; y | s) in nats between the K draws (uniform) and the next
+ * count, exact over the union of the draws' count windows, for the design handle of a Poisson or binomial likelihood
+ * (obe_model_compile_likelihood_design), single channel, 1 <= K <= 128, var_noise[0] the design aux (binomial: the
+ * planned trials, an integer >= 1); log_form is ignored; a setting where some draw's output is invalid for the
+ * likelihood gets 0; obe_cycle_t.method = 4 runs it inside the cycle.
  * log_form=1 gives log(1 + var/sigma^2).  utility_dev (S) out; best_dev: int64 index then double
  * value (16 bytes). */
 int obe_utility(obe_model_t m, const double* draws_dev, int k, const double* settings_dev,

@@ -901,6 +901,7 @@ static cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
 static int64_t g_utility_lane_fill = 50;          /* obe_set_option("utility_lane_fill"), percent of resident threads */
 static int64_t g_plan_cluster_min_tiles = 8192;   /* obe_set_option("plan_cluster_min_tiles") */
 static int64_t g_utility_cache = 1;               /* obe_set_option("utility_cache"): park the K curves in shared memory */
+static int64_t g_utility_info_blocks = 0;         /* obe_set_option("utility_info_blocks"): > 0 caps the information-gain grid */
 static int64_t g_resample_fused = 1;              /* obe_set_option("resample_fused"): 1 = k_sys_resample_warp, 0 = ancestors + move */
 static int64_t g_resample_units_per_sm = 16;      /* obe_set_option("resample_units_per_sm"): work units per SM the chunk size aims at */
 static int64_t g_resample_reserve = 0;            /* obe_set_option("resample_reserve_ctas"): CTA slots an early-select resample leaves to the selection kernels */
@@ -2466,6 +2467,7 @@ struct obe_model {
     int lik;                // OBE_LIK_*: the measurement likelihood of the update kernels
     const void* f_update_y; // non-Gaussian handles: the update from a supplied y_model (OBE_SRC_Y)
     int design;             // f_utility is the likelihood-aware utility: obe_utility reads var_noise[c] as the aux a_c
+    const void* f_utility_info;  // Poisson / binomial design handles: the information-gain utility (method 4)
 };
 #define OBE_LIK_GAUSS 0
 #define OBE_LIK_POISSON 1
@@ -2651,6 +2653,7 @@ int obe_set_option(const char* name, int64_t value) {
     if (s == "plan_cluster_min_tiles") { g_plan_cluster_min_tiles = value < 0 ? 0 : value; return 0; }
     if (s == "utility_lane_fill") { g_utility_lane_fill = value < 0 ? 0 : value; return 0; }
     if (s == "utility_cache") { g_utility_cache = value ? 1 : 0; return 0; }
+    if (s == "utility_info_blocks") { g_utility_info_blocks = value < 0 ? 0 : value; return 0; }
     if (s == "resample_fused") { g_resample_fused = value ? 1 : 0; return 0; }
     if (s == "resample_blocks") { g_resample_blocks = value < 0 ? 0 : value; return 0; }
     if (s == "resample_reserve_ctas") { g_resample_reserve = value < 0 ? 0 : value; return 0; }
@@ -2784,7 +2787,8 @@ static int compile_likelihood(const char* builtin_name, const char* model_source
             src += noise_var_entry;
             src += "(y, a); }\n"
                    "    __device__ static __forceinline__ bool ok(double, double v) { return v >= 0.0; }\n"
-                   "    __device__ static __forceinline__ double finish(double m, double) { return m; }\n};\n";
+                   "    __device__ static __forceinline__ double finish(double m, double) { return m; }\n"
+                   "    typedef ObeNoInfo Info;\n};\n";
         }
     }
     const char* noise_type = kind == OBE_LIK_POISSON ? "ObePoissonNoise"
@@ -2803,12 +2807,15 @@ static int compile_likelihood(const char* builtin_name, const char* model_source
     if (nvrtc_cubin(src, "obe_likelihood_model.cu", cubin, log, log_len)) return -1;
     obe_model* m = new obe_model(tmp);
     m->d = n_params; m->user = true; m->lik = kind; m->design = design ? 1 : 0;
-    const void* k[5];
-    const char* kn[5] = {"obe_k_update_lik", "obe_k_updatey_lik", "obe_k_evalp_lik", "obe_k_utility_lik",
-                         "obe_k_evals_lik"};
+    const void* k[6];
+    const char* kn[6] = {"obe_k_update_lik", "obe_k_updatey_lik", "obe_k_evalp_lik", "obe_k_utility_lik",
+                         "obe_k_evals_lik", "obe_k_utility_info"};
     if (design) { kn[3] = "obe_k_utility_design"; kn[4] = "obe_k_evals_design"; }
-    if (load_kernels(m, cubin, kn, k, 5)) return -1;
+    // (the information gain needs a known support: Poisson and binomial design handles only)
+    const int nk = design && kind != OBE_LIK_USER ? 6 : 5;
+    if (load_kernels(m, cubin, kn, k, nk)) return -1;
     m->f_update = k[0]; m->f_update_y = k[1]; m->f_evalp = k[2]; m->f_utility = k[3]; m->f_evals = k[4];
+    if (nk == 6) m->f_utility_info = k[5];
     *out = m;
     return 0;
 }
@@ -3747,8 +3754,24 @@ int obe_utility(obe_model_t m, const double* draws_dev, int k, const double* set
                 void* best_dev, void* select_scratch_dev, void* stream) {
     if (!m || !draws_dev || !settings_dev || !utility_dev || !best_dev || !select_scratch_dev)
         return obe_fail("null argument%s%s");
-    if (method < 0 || method > 3) return obe_fail("unknown utility method%s%s");
-    if (method >= 2 && (k < 3 || k > OBE_MAX_DRAWS)) return obe_fail("entropy utilities need 3 <= n_draws <= 128%s%s");
+    if (method < 0 || method > 4) return obe_fail("unknown utility method%s%s");
+    if (method == 4) {
+        if (!m->design || !m->f_utility_info)
+            return obe_fail("information gain utility: needs the likelihood-aware design handle of a Poisson or "
+                            "binomial likelihood%s%s");
+        if (m->nch != 1) return obe_fail("information gain utility: single-channel models only%s%s");
+        if (k < 1 || k > OBE_MAX_DRAWS) return obe_fail("information gain utility: 1 <= n_draws <= 128%s%s");
+        if (!var_noise) return obe_fail("information gain utility: needs the design aux in var_noise%s%s");
+        if (m->lik == OBE_LIK_BINOMIAL && !(var_noise[0] >= 1.0 && var_noise[0] <= 9007199254740992.0 &&
+                                            var_noise[0] == floor(var_noise[0]))) {
+            char got[64];
+            snprintf(got, sizeof(got), "%.17g", var_noise[0]);
+            return obe_fail("information gain utility: the binomial trial count (design aux) must be an integer "
+                            ">= 1, got %s%s", got);
+        }
+    }
+    if ((method == 2 || method == 3) && (k < 3 || k > OBE_MAX_DRAWS))
+        return obe_fail("entropy utilities need 3 <= n_draws <= 128%s%s");
     if (method == 3 && (!kld_noise_dev || m->nch != 1)) return obe_fail("full KLD utility: single-channel models, noise required%s%s");
     if (method == 3 && m->design)
         return obe_fail("full KLD utility: its noise samples are Gaussian; a likelihood-aware design handle has none%s%s");
@@ -3771,6 +3794,17 @@ int obe_utility(obe_model_t m, const double* draws_dev, int k, const double* set
     for (int j = 0; j < m->ncons; ++j) a.cons[j] = constants[j];
     size_t smem = (size_t)k * (m->np_model > 0 ? m->np_model : 1) * sizeof(double);
     if (smem > 48 * 1024) return obe_fail("n_draws too large for shared memory%s%s");
+    if (method == 4) {
+        // one warp per setting, OBE_INFO_ARRAYS x K doubles of shared memory per warp beside the draws
+        smem += (size_t)(OBE_THREADS / 32) * OBE_INFO_ARRAYS * k * sizeof(double);
+        cudaError_t e = set_max_smem(m->f_utility_info, smem);
+        if (e != cudaSuccess) return obe_fail("cudaFuncSetAttribute(max dynamic smem): %s%s", cudaGetErrorString(e));
+        const int64_t per_block = OBE_THREADS / 32;
+        int64_t blocks = (n_settings + per_block - 1) / per_block;
+        if (blocks > (int64_t)obe_sms() * 8) blocks = (int64_t)obe_sms() * 8;
+        if (g_utility_info_blocks > 0 && blocks > g_utility_info_blocks) blocks = g_utility_info_blocks;
+        return launch_kernel(m->f_utility_info, (int)blocks, smem, (cudaStream_t)stream, &a, true);
+    }
     // variance utility: several lanes per setting while the grid is too small to fill the GPU anyway (the
     // one-thread-per-setting walk is pure latency there; on a large grid the idle lanes of the sequential sums
     // would cost throughput: 1e5 settings take 42 us with one lane, 60 us with eight) and the K curves of a

@@ -1485,6 +1485,9 @@ __device__ __forceinline__ void obe_block_argmax(double& best, long long& besti,
 // v_c = finish((sum_k nu(y_kc, a_c)) / K, a_c), summed sequentially over k, with a_c = var_noise[c] read as the design
 // aux; r_c = 0 where the spread is 0, spread / v_c otherwise (+inf where v_c = 0).  A setting where some draw's output
 // is invalid for the likelihood (ok() false) gets utility 0.
+struct ObePoissonInfo;   // (the pmf of a likelihood policy, for the information gain: see obe_info_gain_body)
+struct ObeBinomialInfo;
+struct ObeNoInfo;
 struct ObeFixedNoise {
     static constexpr bool LIK = false;
     static constexpr bool NU_IS_Y = false;
@@ -1496,6 +1499,7 @@ struct ObePoissonNoise {
     __device__ static __forceinline__ double nu(double y, double) { return y; }
     __device__ static __forceinline__ bool ok(double y, double) { return y >= 0.0 && y <= 1.7976931348623157e308; }
     __device__ static __forceinline__ double finish(double m, double) { return m; }
+    typedef ObePoissonInfo Info;                         // (the information gain, obe_info_gain_body)
 };
 // Binomial in probability units: variance p (1 - p) / n, n = a_c the planned trials.  p outside [0, 1] / NaN invalid.
 struct ObeBinomialNoise {
@@ -1504,6 +1508,7 @@ struct ObeBinomialNoise {
     __device__ static __forceinline__ double nu(double y, double) { return obe_mul(y, obe_sub(1.0, y)); }
     __device__ static __forceinline__ bool ok(double y, double) { return y >= 0.0 && y <= 1.0; }
     __device__ static __forceinline__ double finish(double m, double a) { return obe_div(m, a); }
+    typedef ObeBinomialInfo Info;
 };
 // (a user likelihood's policy, nu = its noise_var(y, a), negative or NaN invalid, is generated with its source by
 // obe_model_compile_likelihood_design)
@@ -1763,6 +1768,293 @@ __device__ void obe_utility_body(const ObeUtilityArgs& a) {
         *a.counter = 0u;
     }
     (void)lane; (void)warp;
+}
+
+// ---- information gain (utility method 4) ------------------------------------------------------------------------
+// The mutual information between the parameters and the next count, for theta uniform over the K draws:
+//   I(s) = (1/K) sum_k sum_y p_k(y) log(p_k(y) / pbar(y)),  p_k(y) = P(y | theta_k, s),  pbar = (1/K) sum_j p_j,
+// in nats, in [0, log K].  Exact up to the mass outside the windows (< 1e-17 per component):
+// - component k contributes the integers of [mu_k - t_k, mu_k + t_k] (clipped to the support), t = sqrt(79 var) + 27
+//   (Bernstein: the tail beyond t is below exp(-t^2 / (2 (var + t/3))) < 1e-17), t = 0 for a point mass; y runs over
+//   the union of the K windows, so a setting costs K |union| pmf terms;
+// - log-pmfs are differences from a reference draw r with an interior output (the one closest to the mean of the K
+//   outputs): delta_k(y) = log p_k(y) - log p_r(y), exact 0 for k = r and -inf off a point mass's support;
+// - with M = max_k delta_k(y) and L = log1p((1/K) sum_k expm1(delta_k - M)) (log of the mixture over e^M p_r), the
+//   term of draw k is pbar(y) phi(d_k), d_k = delta_k - M - L = log(p_k / pbar), phi(d) = d e^d - expm1(d) >= 0:
+//   sum_k pbar phi(p_k / pbar) is the KL sum at y because sum_k (pbar - p_k) = 0, and no term cancels another, so
+//   an I of 1e-12 keeps its digits;
+// - pbar(y) = exp(log p_r(y) + M + L) is the only place lgamma enters.
+// An invalid output (ok() false) gives the setting 0; K bitwise-equal outputs give exactly 0.
+// Pmf: the likelihood's support, windows, reference log-pmf and the coefficients of delta_k(y).  n: the binomial trials.
+struct ObeNoInfo {                    // (a user likelihood: its support is unknown, so no information-gain kernel body)
+    static constexpr bool EXACT = false;
+};
+// Poisson with mean x: delta_k(y) = y A_k - B_k, A_k = log1p((x_k - x_r) / x_r), B_k = x_k - x_r.
+struct ObePoissonInfo {
+    static constexpr bool EXACT = true;
+    __device__ static __forceinline__ bool ok(double x) { return x >= 0.0 && x <= OBE_DBL_MAX; }
+    __device__ static __forceinline__ bool interior(double x) { return x > 0.0; }
+    __device__ static __forceinline__ void moments(double x, double, double& mu, double& var) { mu = x; var = x; }
+    __device__ static __forceinline__ double top(double) { return OBE_DBL_MAX; }
+    __device__ static __forceinline__ void coef(double x, double xr, double, double& A, double& B) {
+        B = x - xr;
+        A = log1p(B / xr);                               // x = 0: log1p(-1) = -inf
+    }
+    __device__ static __forceinline__ double delta(double y, double, double A, double B) {
+        return y == 0.0 ? -B : fma(y, A, -B);
+    }
+    __device__ static __forceinline__ double logpmf(double y, double xr, double) {
+        return (y == 0.0 ? 0.0 : y * log(xr)) - xr - lgamma(y + 1.0);
+    }
+};
+// Binomial with n trials and success probability x: delta_k(y) = y A_k + (n - y) B_k, A_k = log1p((x_k - x_r) / x_r),
+// B_k = log1p((x_r - x_k) / (1 - x_r)); a point mass at 0 (x = 0) or n (x = 1) has A or B = -inf.
+struct ObeBinomialInfo {
+    static constexpr bool EXACT = true;
+    __device__ static __forceinline__ bool ok(double x) { return x >= 0.0 && x <= 1.0; }
+    __device__ static __forceinline__ bool interior(double x) { return x > 0.0 && x < 1.0; }
+    __device__ static __forceinline__ void moments(double x, double n, double& mu, double& var) {
+        mu = n * x;
+        var = mu * (1.0 - x);
+    }
+    __device__ static __forceinline__ double top(double n) { return n; }
+    __device__ static __forceinline__ void coef(double x, double xr, double, double& A, double& B) {
+        A = log1p((x - xr) / xr);
+        B = log1p((xr - x) / (1.0 - xr));
+    }
+    __device__ static __forceinline__ double delta(double y, double n, double A, double B) {
+        const double t = y < n ? (n - y) * B : 0.0;
+        return y > 0.0 ? fma(y, A, t) : t;
+    }
+    __device__ static __forceinline__ double logpmf(double y, double xr, double n) {
+        return ((lgamma(n + 1.0) - lgamma(y + 1.0)) - lgamma(n - y + 1.0)) + (y * log(xr) + (n - y) * log1p(-xr));
+    }
+};
+
+// expm1(x) for x <= 5 (-inf included), from the polynomial of obe_exp_nonpos: on |x| <= ln2/2 the product r p(r)
+// (no cancellation), elsewhere 2^k (1 + r p(r)) - 1, whose result is at least 0.29 in magnitude.  ~2 ulp.
+__device__ __forceinline__ double obe_expm1_lean(double x) {
+    const double xc = fmax(x, -708.0);
+    const double t = fma(xc, 1.4426950408889634, 6755399441055744.0);
+    const int k = __double2loint(t);
+    const double kf = t - 6755399441055744.0;
+    double r = fma(kf, -6.93147180369123816490e-01, xc);
+    r = fma(kf, -1.90821492927058770002e-10, r);
+    double p = obe_exp_c[0];
+#pragma unroll
+    for (int i = 1; i < 12; ++i) p = fma(p, r, obe_exp_c[i]);
+    p = fma(p, r, 1.0);                                  // (e^r - 1) / r
+    const double em = p * r;
+    if (k == 0) return em;
+    const double scale = __hiloint2double((k + 1023) << 20, 0);
+    return x < -708.0 ? -1.0 : fma(em, scale, scale - 1.0);
+}
+// phi(d) = d e^d - expm1(d) = sum_{m >= 2} (m - 1) d^m / m!  (>= 0; phi(-inf) = 1): the series through m = 13 on
+// |d| < 1/2 (relative truncation < 1e-13), where the closed form would cancel.
+__device__ __forceinline__ double obe_info_phi(double d) {
+    if (fabs(d) < 0.5) {
+        double p = 1.0 / 518918400.0;
+        p = fma(p, d, 1.0 / 43545600.0);
+        p = fma(p, d, 1.0 / 3991680.0);
+        p = fma(p, d, 1.0 / 403200.0);
+        p = fma(p, d, 1.0 / 45360.0);
+        p = fma(p, d, 1.0 / 5760.0);
+        p = fma(p, d, 1.0 / 840.0);
+        p = fma(p, d, 1.0 / 144.0);
+        p = fma(p, d, 1.0 / 30.0);
+        p = fma(p, d, 0.125);
+        p = fma(p, d, 1.0 / 3.0);
+        p = fma(p, d, 0.5);
+        return p * d * d;
+    }
+    if (d < -708.0) return 1.0;
+    const double em = obe_expm1_lean(d);
+    return fma(d, em + 1.0, -em);
+}
+
+#define OBE_INFO_ARRAYS 6            // per warp: [6][K] doubles of shared memory
+// One warp per setting.  The lanes evaluate the K outputs, pick the reference, build the windows (sorted by rank,
+// merged by lane 0), then walk the union with a fixed assignment (lane l takes the l-th, (l+32)-th, ... value of y,
+// each summing its own terms in order) and reduce in the fixed xor tree of obe_warp_sum: the same bits whatever the
+// grid.  The argmax contract is obe_utility_body's.
+template <class Model, class Pmf>
+__device__ void obe_info_gain_body(const ObeUtilityArgs& a) {
+    extern __shared__ double obe_smem[];
+    double* sdraw = obe_smem;  // [K][NP]
+    __shared__ double bval[OBE_THREADS / 32];
+    __shared__ long long bidx[OBE_THREADS / 32];
+    __shared__ unsigned int is_last;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int K = a.k;
+    obe_grid_dep_wait();
+    for (int q = tid; q < K * Model::NP; q += blockDim.x) {
+        const int k = q / Model::NP, j = q % Model::NP;
+        sdraw[q] = a.draws[(long long)j * K + k];
+    }
+    __syncthreads();
+    const double n = a.var_noise[0];                     // binomial: the planned trials (the design aux)
+    const double kd = (double)K;
+    double* xa = sdraw + K * Model::NP + (long long)warp * OBE_INFO_ARRAYS * K;  // outputs, then A_k
+    double* xb = xa + K;          // cumulative counts of the merged windows
+    double* sl = xb + K;          // windows sorted by their start, then B_k
+    double* sh = sl + K;
+    double* ml = sh + K;          // windows of the K draws, then the merged union
+    double* mh = ml + K;
+    double best = 0.0;
+    long long besti = -1;
+    const int wpb = (int)(blockDim.x >> 5);
+    for (long long s = (long long)blockIdx.x * wpb + warp; s < a.n_settings; s += (long long)gridDim.x * wpb) {
+        double st[Model::NS > 0 ? Model::NS : 1], yv[Model::NCH];
+#pragma unroll
+        for (int j = 0; j < Model::NS; ++j) st[j] = a.settings[j * a.lds + s];
+        for (int k = lane; k < K; k += 32) {
+            Model::eval(st, sdraw + k * Model::NP, a.cons, yv);
+            xa[k] = yv[0];
+        }
+        __syncwarp();
+        const double x0 = xa[0];
+        bool ok = true, same = true;
+        double xsum = 0.0;
+        for (int k = lane; k < K; k += 32) {
+            const double x = xa[k];
+            ok = ok & Pmf::ok(x);
+            same = same & (x == x0);
+            xsum += x;
+        }
+        ok = __all_sync(0xffffffffu, ok);
+        same = __all_sync(0xffffffffu, same);
+        double u = 0.0;
+        if (ok && !same) {
+            // the reference: the interior output closest to the mean, lowest k among equals
+            const double mean = obe_warp_sum(xsum) / kd;
+            double bd = 0.0;
+            int bk = K;                                  // (K: no interior draw seen)
+            double m0 = 0.0;                             // (point masses at 0, for a binomial without interior draws)
+            for (int k = lane; k < K; k += 32) {
+                const double x = xa[k];
+                const double dist = fabs(x - mean);
+                if (Pmf::interior(x) && (bk == K || dist < bd)) { bd = dist; bk = k; }
+                m0 += x == 0.0 ? 1.0 : 0.0;
+            }
+#pragma unroll
+            for (int m = 16; m >= 1; m >>= 1) {
+                const double od = __shfl_xor_sync(0xffffffffu, bd, m);
+                const int ok2 = __shfl_xor_sync(0xffffffffu, bk, m);
+                if (ok2 != K && (bk == K || od < bd || (od == bd && ok2 < bk))) { bd = od; bk = ok2; }
+            }
+            if (bk == K) {
+                // every draw a point mass at 0 or n (binomial), not all at the same one: the entropy of the split
+                const double c0 = obe_warp_sum(m0), f0 = c0 / kd, f1 = (kd - c0) / kd;
+                u = -(f0 * log(f0) + f1 * log(f1));
+            } else {
+                const double xr = xa[bk];
+                // windows, then their rank by start (ties by k) places them in sl/sh
+                for (int k = lane; k < K; k += 32) {
+                    double mu, var;
+                    Pmf::moments(xa[k], n, mu, var);
+                    const double t = var > 0.0 ? sqrt(79.0 * var) + 27.0 : 0.0;
+                    ml[k] = fmax(ceil(mu - t), 0.0);
+                    mh[k] = fmin(floor(mu + t), Pmf::top(n));
+                }
+                __syncwarp();
+                for (int k = lane; k < K; k += 32) {
+                    const double lo = ml[k];
+                    int rank = 0;
+                    for (int j = 0; j < K; ++j) {
+                        const double lj = ml[j];
+                        rank += (lj < lo || (lj == lo && j < k)) ? 1 : 0;
+                    }
+                    sl[rank] = lo;
+                    sh[rank] = mh[k];
+                }
+                __syncwarp();
+                double wtot = 0.0;
+                if (lane == 0) {                         // merge into ml/mh, cumulative counts into xb
+                    double clo = sl[0], chi = sh[0], cum = 0.0;
+                    int nb = 0;
+                    for (int i = 1; i < K; ++i) {
+                        const double lo = sl[i], hi = sh[i];
+                        if (lo <= chi + 1.0) {
+                            chi = fmax(chi, hi);
+                        } else {
+                            ml[nb] = clo; mh[nb] = chi; xb[nb] = cum;
+                            cum += chi - clo + 1.0;
+                            ++nb;
+                            clo = lo; chi = hi;
+                        }
+                    }
+                    ml[nb] = clo; mh[nb] = chi; xb[nb] = cum;
+                    wtot = cum + (chi - clo + 1.0);
+                }
+                wtot = __shfl_sync(0xffffffffu, wtot, 0);
+                __syncwarp();
+                for (int k = lane; k < K; k += 32) {
+                    double A, B;
+                    Pmf::coef(xa[k], xr, n, A, B);
+                    xa[k] = A;
+                    sl[k] = B;
+                }
+                __syncwarp();
+                double acc = 0.0;
+                int b = 0;
+                for (double j = (double)lane; j < wtot; j += 32.0) {
+                    while (j >= xb[b] + (mh[b] - ml[b] + 1.0)) ++b;
+                    const double y = ml[b] + (j - xb[b]);
+                    double M = 0.0;                      // (delta_r = 0)
+                    for (int k = 0; k < K; ++k) M = fmax(M, Pmf::delta(y, n, xa[k], sl[k]));
+                    double sm = 0.0;
+                    for (int k = 0; k < K; ++k) sm += obe_expm1_lean(Pmf::delta(y, n, xa[k], sl[k]) - M);
+                    const double L = log1p(sm / kd);
+                    double f = 0.0;
+                    for (int k = 0; k < K; ++k) f += obe_info_phi((Pmf::delta(y, n, xa[k], sl[k]) - M) - L);
+                    const double w = obe_exp_nonpos(fmin((Pmf::logpmf(y, xr, n) + M) + L, 0.0));
+                    acc = fma(w, f, acc);
+                }
+                u = obe_warp_sum(acc) / kd;
+            }
+        }
+        if (a.cost) u = obe_div(u, a.cost[s]);
+        u = ok ? u : 0.0;
+        if (lane == 0) {
+            a.utility[s] = u;
+            obe_argmax_take(best, besti, u, s);
+        }
+        __syncwarp();
+    }
+    // ---- block argmax (lowest index among equals), then the last block combines the per-block results
+    obe_block_argmax(best, besti, bval, bidx);
+    if (tid == 0) {
+        a.part_val[blockIdx.x] = best;
+        a.part_idx[blockIdx.x] = besti;
+        __threadfence();
+        is_last = (atomicAdd(a.counter, 1u) == gridDim.x - 1) ? 1u : 0u;
+    }
+    __syncthreads();
+    if (!is_last) return;
+    __threadfence();
+    best = 0.0; besti = -1;
+    for (unsigned int b = tid; b < gridDim.x; b += blockDim.x)
+        obe_argmax_take(best, besti, __ldcg(a.part_val + b), __ldcg(a.part_idx + b));
+    __syncthreads();
+    obe_block_argmax(best, besti, bval, bidx);
+    if (tid == 0) {
+        *a.best_idx = besti;
+        *a.best_val = best;
+        if (a.best_out2) {
+            a.best_out2[0] = besti;
+            reinterpret_cast<double*>(a.best_out2)[1] = best;
+            if (a.seq_out2) {
+                __threadfence_system();
+                *reinterpret_cast<volatile unsigned long long*>(a.seq_out2) = a.seq_val;
+            }
+        }
+        *a.counter = 0u;
+    }
+}
+// (the kernel of a handle without a pmf is empty: obe_utility refuses method 4 there)
+template <class Model, class Pmf>
+__device__ __forceinline__ void obe_info_gain_entry(const ObeUtilityArgs& a) {
+    if constexpr (Pmf::EXACT) obe_info_gain_body<Model, Pmf>(a);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -2192,13 +2484,17 @@ struct ObeNoModel {
     }
 
 // The utility of a likelihood-aware design (design_noise='likelihood'): var_noise[c] is the design aux a_c and NOISE
-// the likelihood's noise-variance policy.  Compiled by NVRTC per handle, beside OBE_DEFINE_LIK_KERNELS.
+// the likelihood's noise-variance policy, NOISE::Info its pmf for the information gain (obe_k_utility_info, method 4).
+// Compiled by NVRTC per handle, beside OBE_DEFINE_LIK_KERNELS.
 #define OBE_DEFINE_DESIGN_KERNELS(MODEL, NOISE)                                                               \
     extern "C" __global__ void __launch_bounds__(OBE_THREADS) obe_k_utility_design(const ObeUtilityArgs a) {  \
         obe_utility_body<MODEL, NOISE>(a);                                                                    \
     }                                                                                                         \
     extern "C" __global__ void __launch_bounds__(OBE_THREADS) obe_k_evals_design(const ObeEvalArgs a) {       \
         obe_eval_settings_body<MODEL>(a);                                                                     \
+    }                                                                                                         \
+    extern "C" __global__ void __launch_bounds__(OBE_THREADS) obe_k_utility_info(const ObeUtilityArgs a) {    \
+        obe_info_gain_entry<MODEL, NOISE::Info>(a);                                                              \
     }
 
 #define OBE_DEFINE_GRID_KERNELS(MODEL, SUFFIX)                                                             \

@@ -48,6 +48,32 @@ class LazyDeviceArray:
         return f'LazyDeviceArray({self._getter()!r})'
 
 
+def _information_gain_aux_problem(aux):
+    """Why the binomial trial counts ``aux`` cannot be the information gain's (None if they can)."""
+    a = np.asarray(aux, dtype=np.float64).reshape(-1)
+    if not (np.all(np.isfinite(a)) and np.all(a >= 1.0) and np.all(a == np.floor(a))):
+        return ("utility_method='information_gain' with a binomial likelihood needs design_aux, the planned number of "
+                f'trials, to be an integer >= 1, got {aux!r}')
+    return None
+
+
+def _information_gain_problem(likelihood, design_lik, n_channels, aux):
+    """Why an engine cannot run the information-gain utility (None if it can)."""
+    if not (isinstance(likelihood, str) and likelihood in ('poisson', 'binomial')):
+        return ("utility_method='information_gain' needs likelihood_model='poisson' or 'binomial' (the sum over "
+                f'counts needs a known support), got {likelihood!r}')
+    if not design_lik:
+        return "utility_method='information_gain' needs design_noise='likelihood'"
+    if n_channels != 1:
+        return f"utility_method='information_gain' supports single-channel models, got {n_channels} channels"
+    if likelihood == 'binomial':
+        if aux is None:
+            return ("utility_method='information_gain' with a binomial likelihood needs design_aux, the planned "
+                    'number of trials')
+        return _information_gain_aux_problem(aux)
+    return None
+
+
 class OptBayesExpt(ParticlePDF):
     """Sequential Bayesian experiment design (obe_base.py:21-272).
 
@@ -77,6 +103,13 @@ class OptBayesExpt(ParticlePDF):
 
     ``design_aux`` is a scalar or one value per channel, finite and > 0, and may be reassigned between cycles.
     Overriding ``likelihood`` in Python raises ``TypeError``: it could not run inside the kernel.
+
+    ``utility_method='information_gain'`` ranks settings by the mutual information between the parameters and the
+    next count, in nats, for the parameters uniform over the K drawn sets:
+    ``I(s) = (1/K) sum_k sum_y p_k(y) log(p_k(y) / pbar(y))``, summed exactly over the counts the K draws make
+    possible (see :meth:`utility_information_gain`).  It needs ``likelihood_model='poisson'`` or ``'binomial'``,
+    ``design_noise='likelihood'``, a single-channel model and, for binomial, an integer ``design_aux >= 1`` (the
+    planned trials).  ``utility_log_form`` does not apply to it and is ignored; ``cost_estimate()`` divides it.
     """
 
     def __init__(self, measurement_model, setting_values, parameter_samples, constants,
@@ -110,6 +143,11 @@ class OptBayesExpt(ParticlePDF):
             measurement_model = measurement_model.with_likelihood(measurement_model.likelihood, 'likelihood')
         elif measurement_model.design_noise != 'fixed':
             measurement_model = measurement_model.with_likelihood(measurement_model.likelihood)
+        if utility_method == 'information_gain':
+            problem = _information_gain_problem(measurement_model.likelihood, self._design_lik,
+                                                measurement_model.n_channels, design_aux)
+            if problem:
+                raise ValueError(problem)
         #: 'gaussian', 'poisson', 'binomial' or a CudaLikelihood
         self.likelihood_model = measurement_model.likelihood
         if self.likelihood_model != 'gaussian':
@@ -144,9 +182,10 @@ class OptBayesExpt(ParticlePDF):
         self.n_channels = measurement_model.n_channels
         self.utility_y_space = np.array([])   # never materialised on the device path
         self.default_noise_std = np.ones((self.n_channels, 1)) * default_noise_std
+        self._utility_code = 4 if utility_method == 'information_gain' else None   # (read by the design_aux setter)
         self.design_aux = design_aux
 
-        utilitymethods = ['variance_approx', 'pseudo_utility', 'full_kld_utility', 'max_min']
+        utilitymethods = ['variance_approx', 'pseudo_utility', 'full_kld_utility', 'max_min', 'information_gain']
         if utility_method == 'variance_approx':
             self._utility_code = 0
         elif utility_method == 'max_min':
@@ -158,11 +197,13 @@ class OptBayesExpt(ParticlePDF):
             if self.n_channels != 1:
                 raise ValueError('full_kld_utility supports single-channel models (the reference broadcast '
                                  'of obe_base.py:719-720 only works for one channel)')
+        elif utility_method == 'information_gain':
+            self._utility_code = 4
         else:
             raise SyntaxError(f'Unknown utility method, {utility_method}. '
                               f'Valid utility methods are: {utilitymethods}')
         self.utility_method = utility_method
-        #: use log(1 + var/sigma^2) instead of the linear form of obe_base.py:654
+        #: use log(1 + var/sigma^2) instead of the linear form of obe_base.py:654 (the information gain ignores it)
         self.utility_log_form = False
 
         selection_methods = ['optimal', 'good', 'random']
@@ -953,6 +994,10 @@ class OptBayesExpt(ParticlePDF):
                 raise ValueError(f'design_aux needs a scalar or {self.n_channels} values, got {arr.size}')
             if not (np.all(np.isfinite(arr)) and np.all(arr > 0)):
                 raise ValueError(f'design_aux must be finite and > 0, got {value!r}')
+        if getattr(self, '_utility_code', None) == 4 and self.likelihood_model == 'binomial':
+            problem = _information_gain_aux_problem(arr)
+            if problem:
+                raise ValueError(problem)
         self._design_aux = value
         self._design_aux_arr = arr
 
@@ -1054,6 +1099,11 @@ class OptBayesExpt(ParticlePDF):
         if code == 3 and self._design_lik:
             raise ValueError("full_kld_utility is not available with design_noise='likelihood': its noise samples "
                              'are Gaussian draws')
+        if code == 4:
+            problem = _information_gain_problem(self.likelihood_model, self._design_lik, self.n_channels,
+                                                self._design_aux_arr)
+            if problem:
+                raise ValueError(problem)
         saved = self._utility_code
         self._utility_code = code
         try:
@@ -1076,6 +1126,19 @@ class OptBayesExpt(ParticlePDF):
     def utility_full_kld(self):
         """Full Kullback-Leibler utility (obe_base.py:688-720)."""
         return self._utility_as(3)
+
+    def utility_information_gain(self):
+        """Expected information gain of the next measurement at every setting, in nats: the mutual information
+        between the parameters (uniform over the K drawn sets) and the count,
+        ``I(s) = (1/K) sum_k sum_y p_k(y) log(p_k(y) / pbar(y))``, ``pbar = (1/K) sum_j p_j``, in ``[0, log K]``.
+
+        The sum over y is exact: it runs over the union of the draws' count windows, each wide enough that the
+        mass it leaves out is below 1e-17, so a setting costs about K times that many pmf terms.  A setting where
+        some draw's output is impossible for the likelihood gets 0, and identical draws give 0.  Divided by
+        ``cost_estimate()``; ``utility_log_form`` is ignored.  Raises ``ValueError`` unless the engine has a Poisson
+        or binomial likelihood with ``design_noise='likelihood'``, one channel and, for binomial, an integer
+        ``design_aux >= 1``."""
+        return self._utility_as(4)
 
     def opt_setting(self):
         """Setting with the maximum utility (obe_base.py:733-756)."""
