@@ -131,6 +131,19 @@ int obe_model_compile_likelihood_design(const char* builtin_name, const char* mo
                                         int n_channels, const char* likelihood, const char* likelihood_source,
                                         const char* likelihood_entry, const char* noise_var_entry, obe_model_t* out,
                                         char* log, size_t log_len);
+/* The design handle of obe_model_compile_likelihood_design for a "user" likelihood, with the information-gain
+ * utility (obe_utility method 4).  `window_entry` names a third function of `likelihood_source`,
+ *   __device__ void <window_entry>(double y_model, double aux, double* lo, double* hi),
+ * the integer count range [lo, hi] that holds one draw's distribution up to a negligible mass (1e-17 or less is
+ * recommended).  Declaring it declares that <likelihood_entry>(&y_model, &y, &aux, 1) is a normalised log-pmf over
+ * the integers y.  A window with NaN or non-integer bounds, lo < 0, lo > hi or hi > 2^53, a log-pmf NaN or +inf,
+ * or a union of the K windows of more than 2^20 counts gives the setting utility 0.  A window with a built-in
+ * likelihood is refused.  Compile errors are in `log`, as for the other compile entries. */
+int obe_model_compile_likelihood_window(const char* builtin_name, const char* model_source, const char* model_entry,
+                                        int n_settings, int n_params, int n_model_params, int n_constants,
+                                        int n_channels, const char* likelihood, const char* likelihood_source,
+                                        const char* likelihood_entry, const char* noise_var_entry,
+                                        const char* window_entry, obe_model_t* out, char* log, size_t log_len);
 int obe_model_info(obe_model_t m, int* n_settings, int* n_model_params, int* n_constants,
                    int* n_channels, int* n_params);
 void obe_model_free(obe_model_t m);
@@ -414,8 +427,9 @@ int obe_draw_strided(const obe_cloud_t* c, const double* u_host, int m, double* 
  * 3 = full KLD (obe_base.py:688-720; kld_noise_dev = (K, C) noise samples, single channel),
  * 4 = information gain: the mutual information I(theta; y | s) in nats between the K draws (uniform) and the next
  * count, exact over the union of the draws' count windows, for the design handle of a Poisson or binomial likelihood
- * (obe_model_compile_likelihood_design), single channel, 1 <= K <= 128, var_noise[0] the design aux (binomial: the
- * planned trials, an integer >= 1); log_form is ignored; a setting where some draw's output is invalid for the
+ * (obe_model_compile_likelihood_design) or of a user likelihood with a window (obe_model_compile_likelihood_window),
+ * single channel, 1 <= K <= 128, var_noise[0] the design aux (binomial: the planned trials, an integer >= 1; user:
+ * the aux of its functions); log_form is ignored; a setting where some draw's output is invalid for the
  * likelihood gets 0; obe_cycle_t.method = 4 runs it inside the cycle.
  * log_form=1 gives log(1 + var/sigma^2).  utility_dev (S) out; best_dev: int64 index then double
  * value (16 bytes). */

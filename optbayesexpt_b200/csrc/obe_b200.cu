@@ -2467,7 +2467,7 @@ struct obe_model {
     int lik;                // OBE_LIK_*: the measurement likelihood of the update kernels
     const void* f_update_y; // non-Gaussian handles: the update from a supplied y_model (OBE_SRC_Y)
     int design;             // f_utility is the likelihood-aware utility: obe_utility reads var_noise[c] as the aux a_c
-    const void* f_utility_info;  // Poisson / binomial design handles: the information-gain utility (method 4)
+    const void* f_utility_info;  // Poisson / binomial / windowed user design handles: the information gain (method 4)
 };
 #define OBE_LIK_GAUSS 0
 #define OBE_LIK_POISSON 1
@@ -2729,7 +2729,8 @@ int obe_model_compile(const char* cuda_source, const char* entry, int n_settings
 static int compile_likelihood(const char* builtin_name, const char* model_source, const char* model_entry,
                               int n_settings, int n_params, int n_model_params, int n_constants, int n_channels,
                               const char* likelihood, const char* likelihood_source, const char* likelihood_entry,
-                              int design, const char* noise_var_entry, obe_model_t* out, char* log, size_t log_len) {
+                              int design, const char* noise_var_entry, const char* window_entry, obe_model_t* out,
+                              char* log, size_t log_len) {
     if (log && log_len) log[0] = 0;
     if (!out || !likelihood || (!builtin_name && (!model_source || !model_entry)))
         return obe_fail("null argument%s%s");
@@ -2743,6 +2744,8 @@ static int compile_likelihood(const char* builtin_name, const char* model_source
         return obe_fail("a user likelihood needs its source and entry%s%s");
     if (design && kind == OBE_LIK_USER && !noise_var_entry)
         return obe_fail("a likelihood-aware design with a user likelihood needs its noise_var entry%s%s");
+    if (window_entry && kind != OBE_LIK_USER)
+        return obe_fail("a count window applies to a user likelihood only (the built-ins know their support)%s%s");
     obe_model tmp = {};
     std::string model_def;
     if (builtin_name) {
@@ -2779,6 +2782,22 @@ static int compile_likelihood(const char* builtin_name, const char* model_source
                "        return ";
         src += likelihood_entry;
         src += "(y, ym, q.aux, n);\n    }\n};\ntypedef ObeLogLik<ObeUserPmf> ObeUserLik;\n";
+        if (design && window_entry) {
+            // the information gain (obe_info_gain_user_body): a window declares that entry, called with
+            // y_meas = &y, aux = &a and one channel, is a normalised log-pmf over the integers
+            src += "struct ObeUserInfo {\n"
+                   "    static constexpr bool EXACT = false;\n"
+                   "    enum { USER = 1 };\n"
+                   "    __device__ static __forceinline__ bool ok(double x, double a) { return ";
+            src += noise_var_entry;
+            src += "(x, a) >= 0.0; }\n"
+                   "    __device__ static __forceinline__ void window(double x, double a, double& lo, double& hi) { ";
+            src += window_entry;
+            src += "(x, a, &lo, &hi); }\n"
+                   "    __device__ static __forceinline__ double logpmf(double y, double x, double a) { return ";
+            src += likelihood_entry;
+            src += "(&x, &y, &a, 1); }\n};\n";
+        }
         if (design) {
             src += "struct ObeUserNoise {\n"
                    "    static constexpr bool LIK = true;\n"
@@ -2788,7 +2807,9 @@ static int compile_likelihood(const char* builtin_name, const char* model_source
             src += "(y, a); }\n"
                    "    __device__ static __forceinline__ bool ok(double, double v) { return v >= 0.0; }\n"
                    "    __device__ static __forceinline__ double finish(double m, double) { return m; }\n"
-                   "    typedef ObeNoInfo Info;\n};\n";
+                   "    typedef ";
+            src += window_entry ? "ObeUserInfo" : "ObeNoInfo";
+            src += " Info;\n};\n";
         }
     }
     const char* noise_type = kind == OBE_LIK_POISSON ? "ObePoissonNoise"
@@ -2811,8 +2832,8 @@ static int compile_likelihood(const char* builtin_name, const char* model_source
     const char* kn[6] = {"obe_k_update_lik", "obe_k_updatey_lik", "obe_k_evalp_lik", "obe_k_utility_lik",
                          "obe_k_evals_lik", "obe_k_utility_info"};
     if (design) { kn[3] = "obe_k_utility_design"; kn[4] = "obe_k_evals_design"; }
-    // (the information gain needs a known support: Poisson and binomial design handles only)
-    const int nk = design && kind != OBE_LIK_USER ? 6 : 5;
+    // (the information gain needs a known support: Poisson and binomial design handles, and user ones with a window)
+    const int nk = design && (kind != OBE_LIK_USER || window_entry) ? 6 : 5;
     if (load_kernels(m, cubin, kn, k, nk)) return -1;
     m->f_update = k[0]; m->f_update_y = k[1]; m->f_evalp = k[2]; m->f_utility = k[3]; m->f_evals = k[4];
     if (nk == 6) m->f_utility_info = k[5];
@@ -2825,8 +2846,8 @@ int obe_model_compile_likelihood(const char* builtin_name, const char* model_sou
                                  const char* likelihood, const char* likelihood_source, const char* likelihood_entry,
                                  obe_model_t* out, char* log, size_t log_len) {
     return compile_likelihood(builtin_name, model_source, model_entry, n_settings, n_params, n_model_params,
-                              n_constants, n_channels, likelihood, likelihood_source, likelihood_entry, 0, nullptr, out,
-                              log, log_len);
+                              n_constants, n_channels, likelihood, likelihood_source, likelihood_entry, 0, nullptr,
+                              nullptr, out, log, log_len);
 }
 
 int obe_model_compile_likelihood_design(const char* builtin_name, const char* model_source, const char* model_entry,
@@ -2836,7 +2857,17 @@ int obe_model_compile_likelihood_design(const char* builtin_name, const char* mo
                                         char* log, size_t log_len) {
     return compile_likelihood(builtin_name, model_source, model_entry, n_settings, n_params, n_model_params,
                               n_constants, n_channels, likelihood, likelihood_source, likelihood_entry, 1,
-                              noise_var_entry, out, log, log_len);
+                              noise_var_entry, nullptr, out, log, log_len);
+}
+
+int obe_model_compile_likelihood_window(const char* builtin_name, const char* model_source, const char* model_entry,
+                                        int n_settings, int n_params, int n_model_params, int n_constants,
+                                        int n_channels, const char* likelihood, const char* likelihood_source,
+                                        const char* likelihood_entry, const char* noise_var_entry,
+                                        const char* window_entry, obe_model_t* out, char* log, size_t log_len) {
+    return compile_likelihood(builtin_name, model_source, model_entry, n_settings, n_params, n_model_params,
+                              n_constants, n_channels, likelihood, likelihood_source, likelihood_entry, 1,
+                              noise_var_entry, window_entry, out, log, log_len);
 }
 
 int obe_model_info(obe_model_t m, int* ns, int* npm, int* nc, int* nch, int* np) {
@@ -3756,9 +3787,12 @@ int obe_utility(obe_model_t m, const double* draws_dev, int k, const double* set
         return obe_fail("null argument%s%s");
     if (method < 0 || method > 4) return obe_fail("unknown utility method%s%s");
     if (method == 4) {
+        if (m->design && m->lik == OBE_LIK_USER && !m->f_utility_info)
+            return obe_fail("information gain utility: the user likelihood declares no count window (build the "
+                            "handle with obe_model_compile_likelihood_window)%s%s");
         if (!m->design || !m->f_utility_info)
             return obe_fail("information gain utility: needs the likelihood-aware design handle of a Poisson or "
-                            "binomial likelihood%s%s");
+                            "binomial likelihood, or of a user likelihood with a window%s%s");
         if (m->nch != 1) return obe_fail("information gain utility: single-channel models only%s%s");
         if (k < 1 || k > OBE_MAX_DRAWS) return obe_fail("information gain utility: 1 <= n_draws <= 128%s%s");
         if (!var_noise) return obe_fail("information gain utility: needs the design aux in var_noise%s%s");

@@ -1786,9 +1786,12 @@ __device__ void obe_utility_body(const ObeUtilityArgs& a) {
 // - pbar(y) = exp(log p_r(y) + M + L) is the only place lgamma enters.
 // An invalid output (ok() false) gives the setting 0; K bitwise-equal outputs give exactly 0.
 // Pmf: the likelihood's support, windows, reference log-pmf and the coefficients of delta_k(y).  n: the binomial trials.
-struct ObeNoInfo {                    // (a user likelihood: its support is unknown, so no information-gain kernel body)
+struct ObeNoInfo {                    // (a user likelihood without a window: its support is unknown, so no kernel body)
     static constexpr bool EXACT = false;
+    enum { USER = 0 };                // (an enum, not a static member: NVRTC would emit one as a global variable)
 };
+// (a user likelihood with a declared window: ObeUserInfo, generated with its source by compile_likelihood, is the
+// policy of obe_info_gain_user_body below: ok(x, a), window(x, a, lo, hi) and logpmf(y, x, a))
 // Poisson with mean x: delta_k(y) = y A_k - B_k, A_k = log1p((x_k - x_r) / x_r), B_k = x_k - x_r.
 struct ObePoissonInfo {
     static constexpr bool EXACT = true;
@@ -1873,6 +1876,46 @@ __device__ __forceinline__ double obe_info_phi(double d) {
 }
 
 #define OBE_INFO_ARRAYS 6            // per warp: [6][K] doubles of shared memory
+// The union of the K integer windows [ml_k, mh_k] of one warp: the windows ranked by start (ties by k) into sl/sh,
+// merged by lane 0 into the disjoint intervals ml/mh with the cumulative counts before each in xb.  Returns the
+// number of integers in the union, in every lane.  Call with the K windows visible to the warp (after __syncwarp).
+// (obe_info_gain_body keeps its own inline copy of these steps: calling this helper there changes the register
+// allocation and the SASS of the Poisson and binomial kernels.)
+__device__ __forceinline__ double obe_info_union(int K, int lane, double* ml, double* mh, double* sl, double* sh,
+                                                 double* xb) {
+    for (int k = lane; k < K; k += 32) {
+        const double lo = ml[k];
+        int rank = 0;
+        for (int j = 0; j < K; ++j) {
+            const double lj = ml[j];
+            rank += (lj < lo || (lj == lo && j < k)) ? 1 : 0;
+        }
+        sl[rank] = lo;
+        sh[rank] = mh[k];
+    }
+    __syncwarp();
+    double wtot = 0.0;
+    if (lane == 0) {                         // merge into ml/mh, cumulative counts into xb
+        double clo = sl[0], chi = sh[0], cum = 0.0;
+        int nb = 0;
+        for (int i = 1; i < K; ++i) {
+            const double lo = sl[i], hi = sh[i];
+            if (lo <= chi + 1.0) {
+                chi = fmax(chi, hi);
+            } else {
+                ml[nb] = clo; mh[nb] = chi; xb[nb] = cum;
+                cum += chi - clo + 1.0;
+                ++nb;
+                clo = lo; chi = hi;
+            }
+        }
+        ml[nb] = clo; mh[nb] = chi; xb[nb] = cum;
+        wtot = cum + (chi - clo + 1.0);
+    }
+    wtot = __shfl_sync(0xffffffffu, wtot, 0);
+    __syncwarp();
+    return wtot;
+}
 // One warp per setting.  The lanes evaluate the K outputs, pick the reference, build the windows (sorted by rank,
 // merged by lane 0), then walk the union with a fixed assignment (lane l takes the l-th, (l+32)-th, ... value of y,
 // each summing its own terms in order) and reduce in the fixed xor tree of obe_warp_sum: the same bits whatever the
@@ -2051,10 +2094,148 @@ __device__ void obe_info_gain_body(const ObeUtilityArgs& a) {
         *a.counter = 0u;
     }
 }
+// ---- information gain of a user likelihood with a declared window (cuda_likelihood(..., window=)) -------------
+// The same I(s), with the user's log-pmf and count windows in place of the built-in closed forms:
+// - draw k contributes the integers of its declared window [lo_k, hi_k]; y runs over the union of the K windows;
+// - there is no analytic reference, so at each y: l_k = log p(y | x_k, a), M = max_k l_k,
+//   L = log1p((1/K) sum_k expm1(l_k - M)), d_k = l_k - M - L = log(p_k / pbar), pbar = exp(M + L), and the term is
+//   pbar sum_k phi(d_k) >= 0 as above.  The per-y maximum (not a reference draw) keeps draws whose supports do not
+//   overlap finite; a y where every l_k = -inf contributes 0.  d_k is a difference of two user log-pmfs, so its
+//   absolute error is about one ulp of |l|: |dI| <~ 1e-8 I + 1e-14 sqrt(I) (DESIGN.md section 6b);
+// - l_k is recomputed, not stored (K doubles per lane per y do not fit beside 8 warps): the first pass over k keeps M
+//   and sum_k expm1(l_k - M) online -- when M rises to l the sum becomes sum + expm1(M - l) (sum + k), a sum of
+//   non-positive terms, so nothing cancels -- and the second pass sums phi(d_k): 2K log-pmf calls per y.
+// A setting gets exactly 0 when some draw is invalid: its noise variance negative or NaN (ok() false), its window
+// with NaN or non-integer bounds, lo < 0, lo > hi or hi > 2^53, some l_k NaN or +inf, or a union of more than
+// OBE_INFO_USER_MAX_COUNTS integers (a careless window would otherwise hold the GPU for hours); K bitwise-equal outputs
+// give exactly 0.  Same fixed lane assignment, xor-tree reduction and argmax contract as obe_info_gain_body.
+#define OBE_INFO_USER_MAX_COUNTS 1048576.0
+template <class Model, class Info>
+__device__ void obe_info_gain_user_body(const ObeUtilityArgs& a) {
+    extern __shared__ double obe_smem[];
+    double* sdraw = obe_smem;  // [K][NP]
+    __shared__ double bval[OBE_THREADS / 32];
+    __shared__ long long bidx[OBE_THREADS / 32];
+    __shared__ unsigned int is_last;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int K = a.k;
+    obe_grid_dep_wait();
+    for (int q = tid; q < K * Model::NP; q += blockDim.x) {
+        const int k = q / Model::NP, j = q % Model::NP;
+        sdraw[q] = a.draws[(long long)j * K + k];
+    }
+    __syncthreads();
+    const double aux = a.var_noise[0];                   // the design aux, passed to the user's functions
+    const double inf = __longlong_as_double(0x7ff0000000000000LL);
+    const double kd = (double)K;
+    double* xa = sdraw + K * Model::NP + (long long)warp * OBE_INFO_ARRAYS * K;  // outputs
+    double* xb = xa + K;          // cumulative counts of the merged windows
+    double* sl = xb + K;          // windows sorted by their start
+    double* sh = sl + K;
+    double* ml = sh + K;          // windows of the K draws, then the merged union
+    double* mh = ml + K;
+    double best = 0.0;
+    long long besti = -1;
+    const int wpb = (int)(blockDim.x >> 5);
+    for (long long s = (long long)blockIdx.x * wpb + warp; s < a.n_settings; s += (long long)gridDim.x * wpb) {
+        double st[Model::NS > 0 ? Model::NS : 1], yv[Model::NCH];
+#pragma unroll
+        for (int j = 0; j < Model::NS; ++j) st[j] = a.settings[j * a.lds + s];
+        for (int k = lane; k < K; k += 32) {
+            Model::eval(st, sdraw + k * Model::NP, a.cons, yv);
+            xa[k] = yv[0];
+        }
+        __syncwarp();
+        const double x0 = xa[0];
+        bool ok = true, same = true;
+        for (int k = lane; k < K; k += 32) {
+            const double x = xa[k];
+            double lo = 0.0, hi = -1.0;
+            Info::window(x, aux, lo, hi);
+            ok = ok & Info::ok(x, aux) & (lo >= 0.0) & (lo <= hi) & (hi <= 9007199254740992.0) &
+                 (lo == floor(lo)) & (hi == floor(hi));
+            same = same & (x == x0);
+            ml[k] = lo;
+            mh[k] = hi;
+        }
+        ok = __all_sync(0xffffffffu, ok);
+        same = __all_sync(0xffffffffu, same);
+        double u = 0.0;
+        if (ok && !same) {
+            __syncwarp();
+            const double wtot = obe_info_union(K, lane, ml, mh, sl, sh, xb);
+            if (!(wtot <= OBE_INFO_USER_MAX_COUNTS)) {
+                ok = false;
+            } else {
+                double acc = 0.0;
+                bool bad = false;
+                int b = 0;
+                for (double j = (double)lane; j < wtot; j += 32.0) {
+                    while (j >= xb[b] + (mh[b] - ml[b] + 1.0)) ++b;
+                    const double y = ml[b] + (j - xb[b]);
+                    double M = -inf, sm = 0.0;           // sm = sum_{j < k} expm1(l_j - M); -1 per l_j = -inf
+                    for (int k = 0; k < K; ++k) {
+                        const double l = Info::logpmf(y, xa[k], aux);
+                        bad = bad | !(l < inf);          // NaN or +inf
+                        if (l == -inf) sm -= 1.0;
+                        else if (l > M) { sm = fma(obe_expm1_lean(M - l), sm + (double)k, sm); M = l; }
+                        else sm += obe_expm1_lean(l - M);
+                    }
+                    if (M == -inf) continue;             // (no draw reaches y)
+                    const double L = log1p(sm / kd);
+                    double f = 0.0;
+                    for (int k = 0; k < K; ++k) f += obe_info_phi((Info::logpmf(y, xa[k], aux) - M) - L);
+                    const double w = obe_exp_nonpos(fmin(M + L, 0.0));
+                    acc = fma(w, f, acc);
+                }
+                ok = !__any_sync(0xffffffffu, bad);
+                u = obe_warp_sum(acc) / kd;
+            }
+        }
+        if (a.cost) u = obe_div(u, a.cost[s]);
+        u = ok ? u : 0.0;
+        if (lane == 0) {
+            a.utility[s] = u;
+            obe_argmax_take(best, besti, u, s);
+        }
+        __syncwarp();
+    }
+    // ---- block argmax (lowest index among equals), then the last block combines the per-block results
+    obe_block_argmax(best, besti, bval, bidx);
+    if (tid == 0) {
+        a.part_val[blockIdx.x] = best;
+        a.part_idx[blockIdx.x] = besti;
+        __threadfence();
+        is_last = (atomicAdd(a.counter, 1u) == gridDim.x - 1) ? 1u : 0u;
+    }
+    __syncthreads();
+    if (!is_last) return;
+    __threadfence();
+    best = 0.0; besti = -1;
+    for (unsigned int b = tid; b < gridDim.x; b += blockDim.x)
+        obe_argmax_take(best, besti, __ldcg(a.part_val + b), __ldcg(a.part_idx + b));
+    __syncthreads();
+    obe_block_argmax(best, besti, bval, bidx);
+    if (tid == 0) {
+        *a.best_idx = besti;
+        *a.best_val = best;
+        if (a.best_out2) {
+            a.best_out2[0] = besti;
+            reinterpret_cast<double*>(a.best_out2)[1] = best;
+            if (a.seq_out2) {
+                __threadfence_system();
+                *reinterpret_cast<volatile unsigned long long*>(a.seq_out2) = a.seq_val;
+            }
+        }
+        *a.counter = 0u;
+    }
+}
+
 // (the kernel of a handle without a pmf is empty: obe_utility refuses method 4 there)
 template <class Model, class Pmf>
 __device__ __forceinline__ void obe_info_gain_entry(const ObeUtilityArgs& a) {
     if constexpr (Pmf::EXACT) obe_info_gain_body<Model, Pmf>(a);
+    else if constexpr (Pmf::USER) obe_info_gain_user_body<Model, Pmf>(a);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -97,7 +97,11 @@ class DeviceModel:
                     b'user' if user else self.likelihood.encode(),
                     self.likelihood.source.encode() if user else None,
                     self.likelihood.entry.encode() if user else None)
-            if self.design_noise == 'likelihood':
+            if self.design_noise == 'likelihood' and user and self.likelihood.window is not None:
+                rc = lib.obe_model_compile_likelihood_window(*args, self.likelihood.noise_var.encode(),
+                                                             self.likelihood.window.encode(), C.byref(h), log,
+                                                             len(log))
+            elif self.design_noise == 'likelihood':
                 nv = self.likelihood.noise_var.encode() if user else None
                 rc = lib.obe_model_compile_likelihood_design(*args, nv, C.byref(h), log, len(log))
             else:
@@ -182,21 +186,25 @@ DESIGN_NOISES = ('fixed', 'likelihood')
 class CudaLikelihood:
     """A measurement likelihood as CUDA source: see :func:`cuda_likelihood`."""
 
-    def __init__(self, source, entry, noise_var=None):
+    def __init__(self, source, entry, noise_var=None, window=None):
         self.source = source
         self.entry = entry
         self.noise_var = noise_var
+        self.window = window
+
+    def _key(self):
+        return (self.source, self.entry, self.noise_var, self.window)
 
     def __eq__(self, other):
-        return isinstance(other, CudaLikelihood) and \
-            (self.source, self.entry, self.noise_var) == (other.source, other.entry, other.noise_var)
+        return isinstance(other, CudaLikelihood) and self._key() == other._key()
 
     def __hash__(self):
-        return hash((self.source, self.entry, self.noise_var))
+        return hash(self._key())
 
     def __repr__(self):
         nv = '' if self.noise_var is None else f', noise_var={self.noise_var!r}'
-        return f'cuda_likelihood(entry={self.entry!r}{nv})'
+        win = '' if self.window is None else f', window={self.window!r}'
+        return f'cuda_likelihood(entry={self.entry!r}{nv}{win})'
 
 
 def non_gaussian(measurement_model, likelihood_model=None):
@@ -206,7 +214,7 @@ def non_gaussian(measurement_model, likelihood_model=None):
     return isinstance(measurement_model, DeviceModel) and measurement_model.likelihood != 'gaussian'
 
 
-def cuda_likelihood(source, entry, noise_var=None):
+def cuda_likelihood(source, entry, noise_var=None, window=None):
     """User measurement likelihood for ``OptBayesExpt(..., likelihood_model=...)``, compiled by NVRTC with the model.
 
     ``source`` must define ``__device__ double <entry>(const double* y_model, const double* y_meas,
@@ -220,8 +228,19 @@ def cuda_likelihood(source, entry, noise_var=None):
     double aux)``: the variance of one channel's measurement given its model output and the design aux.  It is
     what ``OptBayesExpt(..., design_noise='likelihood')`` divides the utility by (averaged over the draws), and
     that mode requires it.  A negative or NaN value marks the output as impossible: the setting's utility is 0.
+
+    ``window`` (optional) names a third function of ``source``, ``__device__ void <window>(double y_model,
+    double aux, double* lo, double* hi)``: the integer count range ``[lo, hi]`` that holds the distribution of one
+    measurement given its model output and the design aux, up to a negligible mass (1e-17 or less is
+    recommended, as the built-in likelihoods use).  Declaring it also declares that ``entry``, called with
+    ``y_meas = &y``, ``aux = &design_aux`` and ``n_channels = 1``, is a normalised log-pmf over the integers y.
+    With it, ``OptBayesExpt(..., utility_method='information_gain', design_noise='likelihood')`` runs for this
+    likelihood (single-channel models): the exact sum over counts runs over the union of the K draws' windows, at
+    about 2 K calls of ``entry`` per count.  A window with NaN or non-integer bounds, ``lo < 0``, ``lo > hi`` or
+    ``hi > 2**53``, a log-pmf that is NaN or +inf, or a union of windows of more than 2**20 counts gives the
+    setting utility 0.
     """
-    return CudaLikelihood(source, entry, noise_var)
+    return CudaLikelihood(source, entry, noise_var, window)
 
 
 def builtin(name):

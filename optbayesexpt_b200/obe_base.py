@@ -14,7 +14,7 @@ import math
 import numpy as np
 
 from . import _lib
-from .models import DESIGN_NOISES, DeviceModel, builtin
+from .models import DESIGN_NOISES, CudaLikelihood, DeviceModel, builtin
 from .particlepdf import ParticlePDF
 
 DEFAULT_N_DRAWS = 30
@@ -59,9 +59,11 @@ def _information_gain_aux_problem(aux):
 
 def _information_gain_problem(likelihood, design_lik, n_channels, aux):
     """Why an engine cannot run the information-gain utility (None if it can)."""
-    if not (isinstance(likelihood, str) and likelihood in ('poisson', 'binomial')):
-        return ("utility_method='information_gain' needs likelihood_model='poisson' or 'binomial' (the sum over "
-                f'counts needs a known support), got {likelihood!r}')
+    user_window = isinstance(likelihood, CudaLikelihood) and likelihood.window is not None
+    if not (user_window or (isinstance(likelihood, str) and likelihood in ('poisson', 'binomial'))):
+        return ("utility_method='information_gain' needs likelihood_model='poisson' or 'binomial', or a "
+                'cuda_likelihood with a window (the sum over counts needs a known support), got '
+                f'{likelihood!r}')
     if not design_lik:
         return "utility_method='information_gain' needs design_noise='likelihood'"
     if n_channels != 1:
@@ -107,9 +109,11 @@ class OptBayesExpt(ParticlePDF):
     ``utility_method='information_gain'`` ranks settings by the mutual information between the parameters and the
     next count, in nats, for the parameters uniform over the K drawn sets:
     ``I(s) = (1/K) sum_k sum_y p_k(y) log(p_k(y) / pbar(y))``, summed exactly over the counts the K draws make
-    possible (see :meth:`utility_information_gain`).  It needs ``likelihood_model='poisson'`` or ``'binomial'``,
-    ``design_noise='likelihood'``, a single-channel model and, for binomial, an integer ``design_aux >= 1`` (the
-    planned trials).  ``utility_log_form`` does not apply to it and is ignored; ``cost_estimate()`` divides it.
+    possible (see :meth:`utility_information_gain`).  It needs ``likelihood_model='poisson'`` or ``'binomial'``, or
+    a ``cuda_likelihood`` with a ``window`` (its entry is then a normalised log-pmf, called with ``aux =
+    design_aux``), ``design_noise='likelihood'``, a single-channel model and, for binomial, an integer
+    ``design_aux >= 1`` (the planned trials).  ``utility_log_form`` does not apply to it and is ignored;
+    ``cost_estimate()`` divides it.
     """
 
     def __init__(self, measurement_model, setting_values, parameter_samples, constants,
@@ -1135,9 +1139,10 @@ class OptBayesExpt(ParticlePDF):
         The sum over y is exact: it runs over the union of the draws' count windows, each wide enough that the
         mass it leaves out is below 1e-17, so a setting costs about K times that many pmf terms.  A setting where
         some draw's output is impossible for the likelihood gets 0, and identical draws give 0.  Divided by
-        ``cost_estimate()``; ``utility_log_form`` is ignored.  Raises ``ValueError`` unless the engine has a Poisson
-        or binomial likelihood with ``design_noise='likelihood'``, one channel and, for binomial, an integer
-        ``design_aux >= 1``."""
+        ``cost_estimate()``; ``utility_log_form`` is ignored.  For a ``cuda_likelihood`` with a ``window`` the sum
+        runs over the union of the declared windows (see :func:`~optbayesexpt_b200.cuda_likelihood`).  Raises
+        ``ValueError`` unless the engine has a Poisson or binomial likelihood, or a cuda_likelihood with a window,
+        with ``design_noise='likelihood'``, one channel and, for binomial, an integer ``design_aux >= 1``."""
         return self._utility_as(4)
 
     def opt_setting(self):
