@@ -185,6 +185,20 @@ int obe_update_from_likelihood(const obe_cloud_t* c, const double* likelihood_de
  * (yvar_noise_model, obe_noiseparam.py:132-136). */
 int obe_refresh(const obe_cloud_t* c, uint32_t mask_le, uint32_t mask_lt, const int32_t* noise_index,
                 int n_noise, const double* pivot, int renormalise, void* stream);
+/* Time-varying parameters: one Gaussian random-walk step of every live particle, in place,
+ *   x <- x + F z,  z ~ N(0, I_d),  F F^T = Q  (the covariance of one step).
+ * factor_host: F, (d, d) row-major, lower-triangular (a non-zero above the diagonal or a non-finite entry is
+ * refused).  Rows of F that are all zero are neither read back nor written: those parameters keep their bits.
+ * A step that would leave the region of the constraint masks (bit j of mask_le: x_j <= 0, of mask_lt: x_j < 0, as in
+ * obe_refresh) is not taken: the particle keeps its previous position exactly.  The weights, tile sums, CDF prefix,
+ * normaliser, N_eff and the implicit-weight word are not touched; the pass rewrites the moments of the moved cloud
+ * (M1, M2 and PIVOT = pivot, plus NOISE of the noise_index rows) with the reductions of obe_update.
+ * Normals: Philox4x32-10 per particle slot i, ctr = (i_lo, i_hi, 0x40000000 | c, epoch), key = seed ^
+ * 0x9E3779B97F4A7C15, c = 0 .. (d-1)/4, each call two float32 Box-Muller pairs (coordinates 4c .. 4c+3).
+ * z_out_dev: optional (d, ld), the normals of every live slot. */
+int obe_drift(const obe_cloud_t* c, const double* factor_host, uint32_t mask_le, uint32_t mask_lt,
+              const int32_t* noise_index, int n_noise, const double* pivot, uint64_t seed, uint32_t epoch,
+              double* z_out_dev, void* stream);
 /* Copy the stats block to host memory (synchronises the stream). */
 int obe_fetch_stats(const obe_cloud_t* c, double* stats_host, void* stream);
 /* After a systematic resample the weights are IMPLICIT (stats[62] = 1/n_total > 0 and weights_dev is
@@ -399,6 +413,13 @@ typedef struct obe_cycle {
      * appears (the update kernel wrote it, or its copy was enqueued ahead of the selection). */
     uint64_t seq;
     void* seq_host;
+    /* drift != 0: obe_drift on the live cloud after the update, the resample and the constraint refresh, before the
+     * draws, with drift_factor (d*d row-major, lower-triangular), drift_mask_le / drift_mask_lt, seed, drift_epoch,
+     * pivot and the noise_index rows of n_noise.  stats_host then receives the block of the drift pass (its FIRED word
+     * is still the update's decision).  The K draws come from the drifted cloud: no early select.  Whole clouds only. */
+    int32_t drift;
+    uint32_t drift_epoch, drift_mask_le, drift_mask_lt;
+    double drift_factor[OBE_MAX_PARAMS * OBE_MAX_PARAMS];
 } obe_cycle_t;
 int obe_cycle(const obe_cycle_t* c);
 /* cudaStreamSynchronize(stream): what a closed loop waits on before it reads best_host / stats_host

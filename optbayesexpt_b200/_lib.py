@@ -72,7 +72,9 @@ class Cycle(C.Structure):
                 ('stream', C.c_void_p), ('side_stream', C.c_void_p),
                 ('resample_threshold', C.c_double), ('stats_host', C.c_void_p), ('stats_src_dev', C.c_void_p),
                 ('best_host', C.c_void_p), ('phase', C.c_int32), ('pad1', C.c_int32),
-                ('seq', C.c_uint64), ('seq_host', C.c_void_p)]
+                ('seq', C.c_uint64), ('seq_host', C.c_void_p),
+                ('drift', C.c_int32), ('drift_epoch', C.c_uint32), ('drift_mask_le', C.c_uint32),
+                ('drift_mask_lt', C.c_uint32), ('drift_factor', C.c_double * (MAX_PARAMS * MAX_PARAMS))]
 
 
 _PD = C.POINTER(C.c_double)
@@ -113,6 +115,8 @@ SIGNATURES = {
                                           C.c_double, _PD, _VP]),
     'obe_update_from_likelihood': (C.c_int, [_PCLOUD, _VP, _PD, _VP]),
     'obe_refresh': (C.c_int, [_PCLOUD, C.c_uint32, C.c_uint32, _PI32, C.c_int, _PD, C.c_int, _VP]),
+    'obe_drift': (C.c_int, [_PCLOUD, _PD, C.c_uint32, C.c_uint32, _PI32, C.c_int, _PD, C.c_uint64, C.c_uint32, _VP,
+                            _VP]),
     'obe_fetch_stats': (C.c_int, [_PCLOUD, _PD, _VP]),
     'obe_materialize_weights': (C.c_int, [_PCLOUD, _VP]),
     'obe_normalized_weights': (C.c_int, [_PCLOUD, _VP, _VP]),

@@ -142,13 +142,19 @@ static cudaError_t set_max_smem(const void* f, size_t smem) {
     if (e == cudaSuccess && dev >= 0 && n_cached < 96) cache[n_cached++] = Ent{f, smem, dev};
     return e;
 }
-// q: the per-record data of a non-Gaussian likelihood, the second argument of its update kernels
+// the random-walk drift (obe_drift): the update body's pipeline and reductions with the likelihood replaced by the step
+template <int D>
+__global__ void __launch_bounds__(OBE_UPDATE_THREADS, 1) k_drift(const ObeUpdateArgs a, const ObeDriftParams q) {
+    obe_update_body<ObeNoModel, D, OBE_SRC_DRIFT, ObeDrift>(a, ObeDrift{q});
+}
+// q: the second argument of the update kernels that take one (ObeLikParams of a non-Gaussian likelihood,
+// ObeDriftParams of the drift)
 static int launch_update_kernel(const void* f, int d, int src, const ObeUpdateArgs& a, int grid, cudaStream_t st,
-                                const ObeLikParams* q = nullptr) {
+                                const void* q = nullptr) {
     const size_t smem = update_smem_bytes(d, src);
     cudaError_t e = set_max_smem(f, smem);
     if (e != cudaSuccess) return obe_fail("cudaFuncSetAttribute(max dynamic smem): %s%s", cudaGetErrorString(e));
-    void* params[2] = {const_cast<ObeUpdateArgs*>(&a), const_cast<ObeLikParams*>(q)};
+    void* params[2] = {const_cast<ObeUpdateArgs*>(&a), const_cast<void*>(q)};
     e = cudaLaunchKernel(f, dim3(grid), dim3(OBE_UPDATE_THREADS), params, smem, st);
     if (e != cudaSuccess) return obe_fail("launch update kernel: %s%s", cudaGetErrorString(e));
     return 0;
@@ -3086,6 +3092,64 @@ int obe_refresh(const obe_cloud_t* c, uint32_t mask_le, uint32_t mask_lt, const 
     return finish_update(c, renormalise, st);
 }
 
+// One random-walk step of every live particle (see obe_drift in the header).  gate / gate_on / gate_not: the gated
+// launches of obe_cycle (resample == 2); stats_out: optional copy of the finished stats block (pinned host memory
+// under UVA, or device memory).
+static int drift_impl(const obe_cloud_t* c, const double* factor, uint32_t mask_le, uint32_t mask_lt,
+                      const int32_t* noise_index, int n_noise, const double* pivot, uint64_t seed, uint32_t epoch,
+                      double* z_out_dev, const double* gate, int gate_on, double* gate_not, double* stats_out,
+                      cudaStream_t st) {
+    if (check_cloud(c)) return -1;
+    if (!factor) return obe_fail("obe_drift: null factor%s%s");
+    if (n_noise < 0 || n_noise > OBE_MAX_CH) return obe_fail("obe_drift: n_noise out of range%s%s");
+    const int d = c->d;
+    ObeDriftParams q;
+    memset(&q, 0, sizeof(q));
+    for (int j = 0; j < d; ++j)
+        for (int k = 0; k < d; ++k) {
+            const double v = factor[j * d + k];
+            if (!std::isfinite(v)) return obe_fail("obe_drift: the factor must be finite%s%s");
+            if (k > j && v != 0.0) return obe_fail("obe_drift: the factor must be lower-triangular%s%s");
+            if (k <= j) {
+                q.f[j * (j + 1) / 2 + k] = v;
+                if (v != 0.0) q.rows |= 1u << j;
+            }
+        }
+    q.particles = c->particles_dev; q.z_out = z_out_dev;
+    q.gate = gate; q.gate_on = gate_on; q.gate_not = gate_not;
+    q.seed = seed; q.epoch = epoch;
+    ObeUpdateArgs a;
+    base_update_args(c, a, pivot);
+    a.scale_in = 0; a.write_weights = 0; a.renormalise = 0;
+    a.mask_le = mask_le; a.mask_lt = mask_lt;
+    a.stats_out2 = stats_out;
+    if (noise_index)
+        for (int j = 0; j < n_noise; ++j) {
+            if (noise_index[j] < 0 || noise_index[j] >= d) return obe_fail("obe_drift: noise_index out of range%s%s");
+            a.noise_idx[j] = noise_index[j]; a.n_noise = j + 1;
+        }
+    const void* f = nullptr;
+    switch (d) {
+        case 1: f = (const void*)k_drift<1>; break;
+        case 2: f = (const void*)k_drift<2>; break;
+        case 3: f = (const void*)k_drift<3>; break;
+        case 4: f = (const void*)k_drift<4>; break;
+        case 5: f = (const void*)k_drift<5>; break;
+        case 6: f = (const void*)k_drift<6>; break;
+        case 7: f = (const void*)k_drift<7>; break;
+        case 8: f = (const void*)k_drift<8>; break;
+        default: return obe_fail("n_params must be 1..8%s%s");
+    }
+    return launch_update_kernel(f, d, OBE_SRC_DRIFT, a, update_grid(c), st, &q);
+}
+
+int obe_drift(const obe_cloud_t* c, const double* factor_host, uint32_t mask_le, uint32_t mask_lt,
+              const int32_t* noise_index, int n_noise, const double* pivot, uint64_t seed, uint32_t epoch,
+              double* z_out_dev, void* stream) {
+    return drift_impl(c, factor_host, mask_le, mask_lt, noise_index, n_noise, pivot, seed, epoch, z_out_dev, nullptr,
+                      0, nullptr, nullptr, (cudaStream_t)stream);
+}
+
 int obe_fetch_stats(const obe_cloud_t* c, double* stats_host, void* stream) {
     if (!c || !stats_host) return obe_fail("null argument%s%s");
     cudaStream_t st = (cudaStream_t)stream;
@@ -3607,6 +3671,52 @@ static int cycle_copy_out(const obe_cycle_t* c, const obe_cloud_t* updated, void
     return 0;
 }
 
+// The drift pass of a cycle on `cloud` (drift != 0).  Two spare words regions of the live cloud's scratch serve the
+// gated cycle: [0, 64) the stats block for a caller whose stats_host is not device-visible, [64] "not fired".
+static double* cycle_words(const obe_cloud_t* c) {
+    return scratch_of(c).partials + (size_t)OBE_MAX_GRID * OBE_NACC_MAX - 72;
+}
+static int cycle_drift(const obe_cycle_t* c, const obe_cloud_t* cloud, const double* gate, int gate_on, double* gate_not,
+                       double* stats_out) {
+    return drift_impl(cloud, c->drift_factor, c->drift_mask_le, c->drift_mask_lt, c->n_noise > 0 ? c->noise_index : nullptr,
+                      c->n_noise, c->pivot, c->seed, c->drift_epoch, nullptr, gate, gate_on, gate_not, stats_out,
+                      (cudaStream_t)c->stream);
+}
+
+// resample == 2 with the drift: the K draws cannot come from the resample plan (they would miss the step), so the
+// resample is emitted at once, the drift runs on alt gated on the test and on the cloud gated on its complement, and
+// the plain draws follow on whichever cloud is live (the alt pass leaves the complement in a word for the draw kernel).
+static int cycle_auto_drift(const obe_cycle_t* c, const CycleZeroCopy& z) {
+    void* st = c->stream;
+    const obe_cloud_t* live = c->cloud;
+    const double* fired = live->stats_dev + OBE_ST_FIRED;
+    double* words = cycle_words(live);
+    double* stats_dst = z.stats ? z.stats : words;
+    g_gate_on = fired;
+    int rc = obe_resample_systematic(live, c->alt, c->u0, nullptr, nullptr, c->seed, c->epoch, c->a_param, c->scale,
+                                     nullptr, nullptr, st);
+    g_gate_on = nullptr;
+    if (rc) return -1;
+    if (cycle_drift(c, c->alt, fired, 1, words + 64, stats_dst) || cycle_drift(c, live, fired, 0, nullptr, stats_dst))
+        return -1;
+    if (c->stats_host && !z.stats)
+        OBE_CUDA(cudaMemcpyAsync(c->stats_host, words, OBE_STATS_LEN * sizeof(double), cudaMemcpyDeviceToHost,
+                                 (cudaStream_t)st));
+    g_gate_off = words + 64;
+    rc = obe_draw(c->alt, c->u, c->k, c->draws_dev, nullptr, st);
+    g_gate_off = fired;
+    if (!rc) rc = obe_draw(live, c->u, c->k, c->draws_dev, nullptr, st);
+    g_gate_off = nullptr;
+    if (rc) return -1;
+    g_utility_best_out = z.best; g_utility_seq_out = z.seq; g_utility_seq_val = c->seq;
+    rc = obe_utility(c->model, c->draws_dev, c->k, c->settings_dev, c->lds, c->n_settings, c->constants, c->var_noise,
+                     nullptr, c->cost_dev, c->method, c->log_form, c->kld_noise_dev, c->utility_dev, c->best_dev,
+                     c->select_scratch_dev, st);
+    g_utility_best_out = nullptr; g_utility_seq_out = nullptr;
+    if (rc) return -1;
+    return cycle_copy_out(c, live, st, z, 1);
+}
+
 // resample == 2: the resample test runs on the device.  The update's finishing block writes stats[FIRED]; plan, pick
 // and the streaming resample are launched gated on it, the plain K-draw kernel gated on its complement, and the
 // utility pass reads whichever draws were produced -- one stream, no host decision, the caller learns the outcome
@@ -3635,6 +3745,7 @@ static int cycle_auto(const obe_cycle_t* c) {
         if (rc_u) return -1;
         if (c->phase == 1) return 0;
     }
+    if (c->drift) return cycle_auto_drift(c, z);
     const double* fired = live->stats_dev + OBE_ST_FIRED;
     g_gate_on = fired;
     obe_resample_defer(1);
@@ -3672,7 +3783,9 @@ int obe_cycle(const obe_cycle_t* c) {
     g_utility_best_out = nullptr; g_utility_seq_out = nullptr;
     g_update_stats_out = nullptr;
     if (rc) return -1;
-    return copied ? 0 : cycle_copy_out(c, c->cloud, c->stream, z);
+    // with the drift the block to deliver is the one its pass wrote, on the resampled cloud if there was a resample
+    const obe_cloud_t* delivered = (c->drift && c->resample) ? c->alt : c->cloud;
+    return copied ? 0 : cycle_copy_out(c, delivered, c->stream, z);
 }
 
 static int cycle_body(const obe_cycle_t* c, bool& copied, const CycleZeroCopy& z) {
@@ -3680,6 +3793,7 @@ static int cycle_body(const obe_cycle_t* c, bool& copied, const CycleZeroCopy& z
     const obe_cloud_t* live = c->cloud;
     const int sharded = c->plan_dev != nullptr;
     if (sharded && !c->peer_bufs) return obe_fail("obe_cycle: a sharded cycle needs the peer exchange%s%s");
+    if (sharded && c->drift) return obe_fail("obe_cycle: the drift is for a whole (unsharded) cloud%s%s");
     if (c->phase != 2) {
         g_update_stats_out = z.stats;
         const int rc_u = obe_update(c->model, live, c->setting, c->constants, c->y_meas, c->has_sigma ? c->sigma : nullptr,
@@ -3695,7 +3809,7 @@ static int cycle_body(const obe_cycle_t* c, bool& copied, const CycleZeroCopy& z
         return -1;
     const bool masks = (c->mask_le | c->mask_lt) != 0u;
     const bool early = c->resample && c->select && !masks && !c->noise_from_stats && c->side_stream && c->method != 3 &&
-                       c->k >= 1 && c->k <= OBE_MAX_DRAWS && g_resample_fused;
+                       c->k >= 1 && c->k <= OBE_MAX_DRAWS && g_resample_fused && !c->drift;
     const double* stats_for_utility = nullptr;
     if (c->resample) {
         if (!c->alt) return obe_fail("obe_cycle: resample needs the second buffer%s%s");
@@ -3737,6 +3851,7 @@ static int cycle_body(const obe_cycle_t* c, bool& copied, const CycleZeroCopy& z
                 return -1;
         }
     }
+    if (c->drift && cycle_drift(c, live, nullptr, 0, nullptr, z.stats)) return -1;
     if (!c->select) return 0;
     if (c->noise_from_stats) stats_for_utility = live->stats_dev;
     if (sharded) {

@@ -80,6 +80,7 @@
 #define OBE_SRC_Y 1      /* y_model supplied (pdf_update(..., y_model_data)) */
 #define OBE_SRC_LIK 2    /* likelihood supplied (ParticlePDF.bayesian_update) */
 #define OBE_SRC_NONE 3   /* no likelihood: moments / tile sums / constraint mask only */
+#define OBE_SRC_DRIFT 4  /* no likelihood: the random-walk step of the particles (obe_drift), then their moments */
 
 struct ObeUpdateArgs {
     const double* particles;
@@ -518,7 +519,7 @@ __device__ __forceinline__ void obe_update_vec(const ObeUpdateArgs& a, const dou
     const double* r_y = BATCHED ? rec + OBE_REC_Y : a.y_meas;
     const double* r_isig = BATCHED ? rec + OBE_REC_ISIG : a.inv_sigma;
     const double* r_piv = BATCHED ? rec + OBE_REC_PIVOT : a.pivot;
-    if (SRC == OBE_SRC_NONE) {
+    if (SRC == OBE_SRC_NONE || SRC == OBE_SRC_DRIFT) {
 #pragma unroll
         for (int e = 0; e < NE; ++e) t[e] = w_in[e];
     } else {
@@ -807,6 +808,9 @@ __device__ void obe_update_body(const ObeUpdateArgs& a, const Lik& likf = Lik())
 
     const int tid = threadIdx.x;
     const int warp = tid >> 5, lane = tid & 31;
+    if constexpr (SRC == OBE_SRC_DRIFT) {
+        if (!likf.gate_open()) return;           // (uniform over the grid: no block has touched anything yet)
+    }
     const long long n = a.n_dev ? *a.n_dev : a.n;
     const long long n_tiles = (n + OBE_TILE - 1) / OBE_TILE;
     // implicit uniform weights (left by a systematic resample): the weight row is neither copied nor read
@@ -940,6 +944,7 @@ __device__ void obe_update_body(const ObeUpdateArgs& a, const Lik& likf = Lik())
                     for (int c = 0; c < OBE_MAX_CH; ++c) yge[e][c] = (SRC == OBE_SRC_Y) ? yv[SRC == OBE_SRC_Y ? c : 0][e] : 0.0;
                     lke[e] = (SRC == OBE_SRC_LIK) ? lv[e] : 1.0;
                 }
+                if constexpr (SRC == OBE_SRC_DRIFT) likf.template move<D, EPT>(a, pe, valid, base, ct, n_valid);
                 obe_update_vec<Model, D, SRC, EPT, false, false, Lik>(a, pe, wv, yge, lke, valid, invS, acc, nullptr, te, likf);
 #pragma unroll
                 for (int e = 0; e < EPT; ++e) tsum += te[e];
@@ -956,14 +961,16 @@ __device__ void obe_update_body(const ObeUpdateArgs& a, const Lik& likf = Lik())
         // tile sum: warp partials -> one named barrier among the consumers -> fixed-order sum.  (A barrier-free
         // variant -- ring of partial slots, the last warp to arrive sums -- and a select-free path for full stages
         // were measured on top of the interleaved exp and changed nothing: 0.586 vs 0.590 ms at 1e8.)
-        tsum = obe_warp_sum(tsum);
-        if (lane == 0) red[tile_par][cwarp] = tsum;
-        obe_named_bar(1, OBE_CONSUMER_THREADS);
-        if (ct == 0) {
-            double s = red[tile_par][0];
+        if constexpr (SRC != OBE_SRC_DRIFT) {     // (the drift leaves the weights, hence the tile sums, as they are)
+            tsum = obe_warp_sum(tsum);
+            if (lane == 0) red[tile_par][cwarp] = tsum;
+            obe_named_bar(1, OBE_CONSUMER_THREADS);
+            if (ct == 0) {
+                double s = red[tile_par][0];
 #pragma unroll
-            for (int w = 1; w < OBE_CONSUMER_WARPS; ++w) s += red[tile_par][w];
-            a.tile_sums[tile] = s;
+                for (int w = 1; w < OBE_CONSUMER_WARPS; ++w) s += red[tile_par][w];
+                a.tile_sums[tile] = s;
+            }
         }
     }
 
@@ -1003,6 +1010,23 @@ __device__ void obe_update_body(const ObeUpdateArgs& a, const Lik& likf = Lik())
         if (lane == 0) fin[v] = sv;
     }
     obe_named_bar(1, OBE_CONSUMER_THREADS);
+    if constexpr (SRC == OBE_SRC_DRIFT) {
+        // only the moments move: totals, normaliser, N_eff, the implicit-weight word and the tile prefix stay
+        if (ct == 0) {
+            for (int j = 0; j < D; ++j) { a.stats[OBE_ST_M1 + j] = fin[3 + j]; a.stats[OBE_ST_PIVOT + j] = a.pivot[j]; }
+            for (int j = 0; j < NM2; ++j) a.stats[OBE_ST_M2 + j] = fin[3 + D + j];
+            for (int c = 0; c < OBE_MAX_CH; ++c)
+                if (a.noise_idx[c] >= 0) a.stats[OBE_ST_NOISE + c] = fin[3 + D + NM2 + c];
+            *a.counter = 0u;
+        }
+        if (a.stats_out2) {
+            obe_named_bar(1, OBE_CONSUMER_THREADS);
+            // the FIRED word of the copy is the update's decision, which this (gated) pass ran under
+            if (ct < OBE_STATS_LEN)
+                a.stats_out2[ct] = (ct == OBE_ST_FIRED && likf.q.gate) ? *likf.q.gate : __ldcg(a.stats + ct);
+        }
+        return;
+    }
     if (ct == 0) {
         a.stats[OBE_ST_SUMSQ] = fin[0];
         a.stats[OBE_ST_SUMT] = fin[1];
@@ -1394,6 +1418,116 @@ __device__ __forceinline__ void device_normals(long long slot, unsigned long lon
         }
     }
 }
+
+// ---------------------------------------------------------------------------------------------
+// Random-walk drift of the parameters between measurements (obe_drift): x <- x + F z, z ~ N(0, I), F F^T = Q
+// ---------------------------------------------------------------------------------------------
+// Normals of particle slot `slot` in drift step `epoch`: the per-slot layout of device_normals (call c gives four
+// 24-bit uniforms -> two float32 Box-Muller pairs for coordinates 4c .. 4c+3) with ctr = (slot_lo, slot_hi,
+// 0x40000000 | c, epoch) and key = seed ^ OBE_DRIFT_KEY, so the stream shares neither counters nor key with the
+// Liu-West jitter of the same seed.  Restated in oracle/obe_oracle.py:drift_normals.
+#define OBE_DRIFT_CTR 0x40000000u
+#define OBE_DRIFT_KEY 0x9E3779B97F4A7C15ull
+template <int D>
+__device__ __forceinline__ void obe_drift_normals(long long slot, unsigned long long seed, unsigned int epoch,
+                                                  double (&z)[D]) {
+    const unsigned long long key = seed ^ OBE_DRIFT_KEY;
+#pragma unroll
+    for (int c = 0; c < (D + 3) / 4; ++c) {
+        unsigned int r[4];
+        philox4x32_10((unsigned int)(slot & 0xffffffffll), (unsigned int)((unsigned long long)slot >> 32),
+                      OBE_DRIFT_CTR | (unsigned int)c, epoch, (unsigned int)(key & 0xffffffffull),
+                      (unsigned int)(key >> 32), r);
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+            if (4 * c + 2 * h < D) {
+                const float rad = obe_sqrt_approx(-2.0f * __logf(u24(r[2 * h])));
+                float sn, cs;
+                __sincosf(6.2831853071795865f * u24(r[2 * h + 1]), &sn, &cs);
+                z[4 * c + 2 * h] = (double)(rad * cs);
+                if (4 * c + 2 * h + 1 < D) z[4 * c + 2 * h + 1] = (double)(rad * sn);
+            }
+        }
+    }
+}
+
+// The by-value second argument of k_drift<D>.
+struct ObeDriftParams {
+    double f[OBE_MAX_DIMS * (OBE_MAX_DIMS + 1) / 2];   // F, lower triangle packed row-major: F[j][k] at j(j+1)/2 + k
+    double* particles;        // the cloud's rows, moved in place (ObeUpdateArgs::particles is the same memory)
+    double* z_out;            // optional (d, ld): the normals of every live slot
+    const double* gate;       // optional: the pass runs only when (*gate != 0) == gate_on (obe_cycle, resample == 2)
+    double* gate_not;         // optional: block 0 stores (*gate == 0) here before the pass starts or is skipped
+    unsigned long long seed;
+    unsigned int epoch;
+    unsigned int rows;        // bit j: row j of F is not all zero (the other rows are neither moved nor stored)
+    int gate_on;
+};
+
+// The drift as the "likelihood" of obe_update_body<ObeNoModel, D, OBE_SRC_DRIFT>: the body stages the weights and the
+// particle rows, move() steps the particles of a consumer's stage and stores the moved rows, and the body then
+// accumulates the moments of the moved cloud with the weights as they are (t = w, like the refresh pass).
+// The constraint masks of ObeUpdateArgs reject a step: the particle keeps its previous position exactly.
+struct ObeDrift {
+    static constexpr bool GAUSS = false;
+    ObeDriftParams q;
+    __device__ __forceinline__ bool gate_open() const {
+        if (!q.gate) return true;
+        const bool fired = *q.gate != 0.0;
+        if (q.gate_not && blockIdx.x == 0 && threadIdx.x == 0) *q.gate_not = fired ? 0.0 : 1.0;
+        return fired == (q.gate_on != 0);
+    }
+    template <int D, int NE>
+    __device__ __forceinline__ void move(const ObeUpdateArgs& a, double (&p)[NE][D], const bool (&valid)[NE],
+                                         long long base, int ct, int n_valid) const {
+#pragma unroll
+        for (int e = 0; e < NE; ++e) {
+            if (!valid[e]) continue;
+            const long long slot = base + ((NE >= 2) ? 2 * (ct + (e >> 1) * OBE_CONSUMER_THREADS) + (e & 1) : ct);
+            double z[D], x[D];
+            obe_drift_normals<D>(slot, q.seed, q.epoch, z);
+            if (q.z_out) {
+#pragma unroll
+                for (int j = 0; j < D; ++j) q.z_out[j * a.ld + slot] = z[j];
+            }
+            bool ok = true;
+#pragma unroll
+            for (int j = 0; j < D; ++j) {
+                x[j] = p[e][j];
+                if ((q.rows >> j) & 1u) {
+                    double nud = 0.0;
+#pragma unroll
+                    for (int k = 0; k <= j; ++k) nud = fma(q.f[j * (j + 1) / 2 + k], z[k], nud);
+                    x[j] += nud;
+                }
+                if (((a.mask_le >> j) & 1u) && x[j] <= 0.0) ok = false;
+                if (((a.mask_lt >> j) & 1u) && x[j] < 0.0) ok = false;
+            }
+            if (ok) {
+#pragma unroll
+                for (int j = 0; j < D; ++j) p[e][j] = x[j];
+            }
+        }
+#pragma unroll
+        for (int j = 0; j < D; ++j) {
+            if (!((q.rows >> j) & 1u)) continue;
+            double* row = q.particles + j * a.ld + base;
+#pragma unroll
+            for (int u = 0; u < (NE >= 2 ? NE / 2 : 1); ++u) {
+                const int e0 = (NE >= 2 ? 2 * (ct + u * OBE_CONSUMER_THREADS) : ct);
+                if (NE >= 2 && e0 + 1 < n_valid) obe_st2(row + e0, make_double2(p[2 * u][j], p[2 * u + 1][j]));
+                else if (e0 < n_valid) row[e0] = p[NE >= 2 ? 2 * u : 0][j];
+            }
+        }
+    }
+    // (never called: obe_update_vec takes the likelihood-free branch for OBE_SRC_DRIFT)
+    template <int D, int NE, int NY>
+    __device__ __forceinline__ void operator()(const ObeUpdateArgs&, const double (&)[NE][D], const double (&)[NE][NY],
+                                               const double*, const double*, double (&lik)[NE]) const {
+#pragma unroll
+        for (int e = 0; e < NE; ++e) lik[e] = 1.0;
+    }
+};
 
 // uniform double in (0,1) from two Philox words
 __device__ __forceinline__ double obe_u53(unsigned int lo, unsigned int hi) {

@@ -14,6 +14,7 @@ import math
 import numpy as np
 
 from . import _lib
+from .drift import drift_factor
 from .models import DESIGN_NOISES, CudaLikelihood, DeviceModel, builtin
 from .particlepdf import ParticlePDF
 
@@ -114,12 +115,26 @@ class OptBayesExpt(ParticlePDF):
     design_aux``), ``design_noise='likelihood'``, a single-channel model and, for binomial, an integer
     ``design_aux >= 1`` (the planned trials).  ``utility_log_form`` does not apply to it and is ignored;
     ``cost_estimate()`` divides it.
+
+    ``drift`` makes the parameters time-varying: after every update (and after the resample, if one ran) each
+    particle takes one Gaussian random-walk step ``x <- x + F z``, ``z ~ N(0, I)``, ``F F^T = Q``, on the device.
+    ``drift`` is the per-parameter standard deviation of one step (a scalar or ``n_dims`` values) or its
+    ``(n_dims, n_dims)`` covariance ``Q`` (symmetric positive semidefinite; zero variance keeps a parameter fixed
+    bit for bit), ``None`` (the default) for static parameters.  It may be reassigned between cycles, e.g.
+    ``eng.drift = Q_per_unit_time * dt_next`` for irregular time steps.  A step that would leave the region of the
+    engine's constraints (the positive noise parameters of OptBayesExptNoiseParameter) is not taken.  The weights
+    are not changed.  The normals are Philox normals keyed by the engine seed, the particle slot and the drift step,
+    also with ``resampling='multinomial'``.  See :meth:`pdf_update` for what the summaries describe.
     """
+    #: why a subclass does not take ``drift`` (None: it does)
+    _drift_refusal = None
 
     def __init__(self, measurement_model, setting_values, parameter_samples, constants,
                  n_draws=DEFAULT_N_DRAWS, choke=None, use_jit=True, utility_method='variance_approx',
                  selection_method='optimal', pickiness=15, default_noise_std=1.0, likelihood_model=None,
-                 design_noise='fixed', design_aux=None, **kwargs):
+                 design_noise='fixed', design_aux=None, drift=None, **kwargs):
+        if drift is not None and self._drift_refusal:
+            raise ValueError(self._drift_refusal)
         if isinstance(measurement_model, str):
             measurement_model = builtin(measurement_model)
         if not isinstance(measurement_model, DeviceModel):
@@ -280,6 +295,42 @@ class OptBayesExpt(ParticlePDF):
         self._best_copied = False         # the argmax of the prepared selection is on its way to _cy_best_np
         self._async_pending = False
         self._dt_cache = None
+        self._drift_epoch = 0             # drift steps taken: the epoch word of their normals
+        self.drift = drift
+
+    # ------------------------------------------------------------------------------------------
+    # time-varying parameters
+    # ------------------------------------------------------------------------------------------
+    @property
+    def drift(self):
+        """Standard deviations or covariance of one random-walk step of the parameters per update (None: static)."""
+        return self._drift
+
+    @drift.setter
+    def drift(self, value):
+        if value is not None and self._drift_refusal:
+            raise ValueError(self._drift_refusal)
+        factor = drift_factor(value, self.n_dims)
+        self._drift = value
+        self._drift_F = factor
+        self._drift_arr = None if factor is None else _lib.darr(factor.reshape(-1), _lib.MAX_PARAMS * _lib.MAX_PARAMS)
+        self._dt_cache = None
+
+    def _apply_drift(self, pivot):
+        """One random-walk step of the live cloud (obe_drift); its moments are then valid on the device."""
+        self._drift_epoch += 1
+        ni = self._noise_index
+        le, lt = self._constraint_masks()
+        self._check(self._lib.obe_drift(self._cs(), self._drift_arr, le, lt, self._noise_iarr(ni),
+                                        0 if ni is None else len(ni), _lib.darr(pivot, _lib.MAX_PARAMS),
+                                        self._philox_seed, self._drift_epoch & 0xffffffff, None, self._stream()))
+        self._after_drift()
+
+    def _after_drift(self):
+        self._invalidate(particles=True)
+        self._cloud_version += 1
+        self._stats = None
+        self._moments_valid = True
 
     # -- the reference rebinds `parameters` to `particles` in pdf_update (obe_base.py:185,395);
     #    here it is a live alias, which removes the stale-alias quirk after resample()/set_pdf()
@@ -308,6 +359,8 @@ class OptBayesExpt(ParticlePDF):
         ParticlePDF.set_pdf(self, samples, weights)
         self._noise_index = noise_index
         self._model = self.model_function.handle(self.n_dims)
+        if self._drift is not None:
+            self.drift = self._drift          # (checks the shape against the new cloud)
 
     # ------------------------------------------------------------------------------------------
     # model evaluation in both orientations (obe_base.py:298-338)
@@ -426,6 +479,11 @@ class OptBayesExpt(ParticlePDF):
 
         Returns ``(particles, particle_weights)`` as lazy, numpy-convertible handles: nothing is
         copied off the GPU unless the caller looks at them.
+
+        With a ``drift`` the random-walk step is the last thing the update does, on every path: after it the cloud
+        and therefore ``mean()``, ``std()``, ``covariance()``, ``quantile()``, ``histogram()``, ``randdraw()`` and
+        the draws of the next ``opt_setting()`` are one step ahead -- the predictive distribution of the parameters
+        at the next measurement, not the posterior at this one.
         """
         if self._pending_cycle:
             self._settle()
@@ -439,6 +497,7 @@ class OptBayesExpt(ParticlePDF):
         y_meas, sigma, noise_index, n_lik = self._likelihood_spec(measurement_record)
         use_choke = 0 if self.choke is None else 1
         choke = 0.0 if self.choke is None else float(self.choke)
+        update_pivot = self._pivot
         pivot = self._a_pivot.fill(self._pivot)
         if y_model_data is None and getattr(self, '_prefetched', None) is not None:
             y_model_data = self._take_prefetched(onesetting)
@@ -471,6 +530,13 @@ class OptBayesExpt(ParticlePDF):
         self._after_update()
         if self.just_resampled:
             self.enforce_parameter_constraints()
+        if self._drift_F is not None:
+            # (moments around the update's pivot, and the next pivot from the step's moments: what the cycle entry
+            # does, so that every path computes the same bits)
+            self._apply_drift(update_pivot)
+            mean = self._mean_from(self._fetch_stats())
+            if np.all(np.isfinite(mean)):
+                self._pivot = mean
         return (LazyDeviceArray(lambda: self.particles), LazyDeviceArray(lambda: self.particle_weights))
 
     # ---- pdf_update without a host synchronisation ------------------------------------------------
@@ -507,7 +573,10 @@ class OptBayesExpt(ParticlePDF):
         return (LazyDeviceArray(lambda: self.particles), LazyDeviceArray(lambda: self.particle_weights))
 
     def _async_stats_source(self, resample):
-        """Device block holding the stats of the update that just ran (the resample swapped the buffers)."""
+        """Device block holding the stats of the update that just ran (the resample swapped the buffers), or of the
+        drift step that followed it on the live cloud."""
+        if self._drift_F is not None:
+            return self._buf.stats
         return (self._alt if resample else self._buf).stats
 
     def _post_async_stats(self, resample):
@@ -581,13 +650,14 @@ class OptBayesExpt(ParticlePDF):
         tp = self.tuning_parameters
         # the answer only changes with these switches: one tuple compare per update instead of seven method calls
         key = (self.device_resample_test, self.eager_select, self.resampling, tp['resample_threshold'], self.early_select,
-               self.use_cycle_entry, self.N_DRAWS, self._utility_code, self._stream_override)
+               self.use_cycle_entry, self.N_DRAWS, self._utility_code, self._stream_override, self._drift_F is None)
         cached = self._dt_cache
         if cached is not None and cached[0] == key:
             return cached[1]
+        # (with a drift the cycle draws from the drifted cloud instead of the resample plan, under the same conditions)
         ok = bool(self.device_resample_test and self.eager_select and self.resampling == 'systematic'
                   and 0.0 <= tp['resample_threshold'] <= 1.0 and self._constraint_masks() == (0, 0)
-                  and not self._noise_from_stats() and self._early_select_ok() and self._cycle_c_ok(True, True))
+                  and not self._noise_from_stats() and self._early_select_possible() and self._cycle_c_ok(True, True))
         # (a subclass with its own cost model can change its mind between calls: do not cache for it)
         if type(self).cost_estimate is OptBayesExpt.cost_estimate:
             self._dt_cache = (key, ok)
@@ -647,7 +717,7 @@ class OptBayesExpt(ParticlePDF):
         self._after_cycle_c(fired)
         self._select_ready, self._best_copied = ready, copied     # (the prepared selection belongs to this outcome)
         self._just_resampled = fired
-        if not fired:
+        if not fired or self._cy.drift:
             self._stats = st                    # the live cloud's stats block, already on the host
         self._adopt_stats(st)
         return True
@@ -790,7 +860,14 @@ class OptBayesExpt(ParticlePDF):
             if not cy.noise_from_stats:
                 vn = np.asarray(self._design_var_noise(), dtype=np.float64).reshape(-1)
                 self._cy_vn[:min(len(vn), _lib.MAX_CHANNELS)] = vn[:_lib.MAX_CHANNELS]
-        if self.early_select and resample and select:
+        if self._drift_F is not None:
+            self._drift_epoch += 1
+            cy.drift, cy.drift_epoch, cy.seed = 1, self._drift_epoch & 0xffffffff, self._philox_seed
+            cy.drift_mask_le, cy.drift_mask_lt = self._constraint_masks()
+            C.memmove(C.addressof(cy) + _lib.Cycle.drift_factor.offset, self._drift_arr, C.sizeof(self._drift_arr))
+        else:
+            cy.drift = 0
+        if self.early_select and resample and select and self._drift_F is None:
             # (small clouds: same early order on the main stream -- the fork / join cost more than the overlap hides)
             cy.side_stream = (self._side_stream()[1].value if self._n_total_for_test() >= self.two_stream_min_particles
                               else cy.stream)
@@ -840,6 +917,8 @@ class OptBayesExpt(ParticlePDF):
                 self._moments_valid = True
                 self._weights_uniform = False
                 self._weights_lazy = True
+        if self._cy.drift:
+            self._after_drift()
 
     def resample_select_async(self, resample=True, select=True):
         """The part of run_cycle_async after the update: (forced) resample and selection, enqueued without a host
@@ -858,14 +937,21 @@ class OptBayesExpt(ParticlePDF):
             self.resample()
             self.just_resampled = True
             self._enforce_constraints_async()
+        if self._drift_F is not None:
+            self._apply_drift(self._pivot)
         if select:
             self._utility_dev_run()
 
     # ---- early select -------------------------------------------------------------------------
     def _early_select_ok(self):
-        """Can the selection be taken from the resample plan?  Needs the one-kernel systematic resample, offspring
-        that keep their uniform weights (no constraint mask), a utility that reads nothing the resample changes
-        (no noise parameter), and no host-side upload inside the utility call (full KLD noise)."""
+        """Can the selection be taken from the resample plan?  Not with a drift, whose step comes after the
+        resample; otherwise see _early_select_possible."""
+        return self._drift_F is None and self._early_select_possible()
+
+    def _early_select_possible(self):
+        """Needs the one-kernel systematic resample, offspring that keep their uniform weights (no constraint mask), a
+        utility that reads nothing the resample changes (no noise parameter), and no host-side upload inside the
+        utility call (full KLD noise)."""
         if not self.early_select or self.resampling != 'systematic' or self._utility_code == 3:
             return False
         if not (1 <= self.N_DRAWS <= _lib.MAX_DRAWS) or self._noise_from_stats():

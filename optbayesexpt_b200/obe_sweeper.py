@@ -26,8 +26,13 @@ class OptBayesExptSweeper(OptBayesExptNoiseParameter):
     ``cost_of_new_sweep`` (5.0).
     """
 
+    _drift_refusal = ('OptBayesExptSweeper does not take drift: its fused multi-point update would need a transition '
+                      'between the points of a sweep')
+
     def __init__(self, model_function, setting_values, parameter_samples, constants, noise_parameter_index,
                  **kwargs):
+        if kwargs.get('drift') is not None:           # (before anything reaches the device)
+            raise ValueError(self._drift_refusal)
         OptBayesExptNoiseParameter.__init__(self, model_function, setting_values, parameter_samples, constants,
                                             noise_parameter_index=noise_parameter_index, **kwargs)
         self.sweep_settings = np.asarray(setting_values[0])

@@ -262,9 +262,14 @@ class ShardedOptBayesExpt(OptBayesExpt):
     reference-shaped ``pdf_update``/``opt_setting`` fetch the plan block only to take the
     resample decision and to return the argmax."""
 
+    _drift_refusal = ('ShardedOptBayesExpt does not take drift: its normals would have to be keyed by the global '
+                      'particle slot to keep the cloud independent of the number of ranks')
+
     def __init__(self, measurement_model, setting_values, parameter_samples, constants, group=None,
                  slack=0.25, seed=0, peer_exchange=None, **kwargs):
         import torch
+        if kwargs.get('drift') is not None:           # (before the process group is touched)
+            raise ValueError(self._drift_refusal)
         if non_gaussian(measurement_model, kwargs.get('likelihood_model')):
             raise ValueError('ShardedOptBayesExpt supports the Gaussian likelihood only; use OptBayesExpt for '
                              'likelihood_model=\'poisson\' | \'binomial\' | cuda_likelihood(...)')
