@@ -552,6 +552,25 @@ int obe_batch_simulate(obe_model_t m, const obe_batch_t* b, const double* settin
                        const double* true_params_dev, int64_t ld_true, const double* constants,
                        const double* noise_level, const double* noise_level_dev, uint64_t seed,
                        uint32_t cycle, int write_sigma, void* stream);
+/* Time-varying parameters of the batched engines: one Gaussian random-walk step of every live particle of every
+ * instance, in place, x <- x + F_b z (obe_drift per instance).  Exactly one of
+ *   factor_host: F, (d, d) row-major, lower-triangular and finite (else refused), shared by all instances;
+ *   factor_dev:  (n_inst, d, d) row-major on the device, one F per instance (only the lower triangle is read).
+ * Rows of F that are all zero are neither read back nor written.  A step that would leave the region of the
+ * constraint masks (as in obe_batch_refresh) is not taken: the particle keeps its previous position exactly.  The
+ * weight buffers, cur, tile sums, prefix rows, TOTAL / INVS / SUMSQ / N_eff / SUMT / NZERO / UNIFORM, flag, epoch,
+ * last_idx and the record are not touched; the pass rewrites M1, M2, PIVOT and the NOISE sums of the noise_index rows
+ * of every instance with the reductions of the batched refresh, and moves its pivot to the drifted mean.
+ * Normals: Philox4x32-10 per slot i of instance b, ctr = (i, b, 0x40000000 | c, step), key = seed ^
+ * 0x9E3779B97F4A7C15 (obe_drift's keying with slot = b << 32 | i). */
+int obe_batch_drift(const obe_batch_t* b, const double* factor_host, const double* factor_dev, uint32_t mask_le,
+                    uint32_t mask_lt, const int32_t* noise_index, int n_noise, uint64_t seed, uint32_t step,
+                    void* stream);
+/* One random-walk step of the true parameters of the on-device simulator: column b of truth_dev (n_params, ld_true)
+ * SoA moves by F_b z, with factor_host / factor_dev as in obe_batch_drift over n_params and no constraint.
+ * Normals: ctr = (b_lo, b_hi, 0x50000000 | c, step), key = seed ^ 0xD1B54A32D192ED03. */
+int obe_batch_truth_drift(double* truth_dev, int64_t ld_true, int64_t n_inst, int n_params, const double* factor_host,
+                          const double* factor_dev, uint64_t seed, uint32_t step, void* stream);
 
 #ifdef __cplusplus
 }

@@ -180,6 +180,9 @@ SIGNATURES = {
     'obe_batch_refresh': (C.c_int, [_PBATCH, C.c_uint32, C.c_uint32, _PI32, C.c_int, _VP]),
     'obe_batch_select': (C.c_int, [_VP, _PBATCH, _VP, C.c_int64, C.c_int64, _PD, C.c_int, _PD, C.c_double,
                                    C.c_uint64, C.c_uint32, C.c_int, C.c_int, _VP, _VP]),
+    'obe_batch_drift': (C.c_int, [_PBATCH, _PD, _VP, C.c_uint32, C.c_uint32, _PI32, C.c_int, C.c_uint64, C.c_uint32,
+                                  _VP]),
+    'obe_batch_truth_drift': (C.c_int, [_VP, C.c_int64, C.c_int64, C.c_int, _PD, _VP, C.c_uint64, C.c_uint32, _VP]),
     'obe_eval_parameters': (C.c_int, [_VP, _PCLOUD, _PD, _PD, _VP, C.c_int64, _VP]),
     'obe_eval_settings': (C.c_int, [_VP, _VP, C.c_int64, C.c_int64, _PD, _PD, _VP, C.c_int64, _VP]),
 }

@@ -10,22 +10,42 @@ one launch over all instances and the whole closed loop stays on the device:
 Same model functors, same kernels' arithmetic, same constraint/cost/noise-parameter options as the
 single engines; instance b reproduces a single engine that is fed the same uniforms
 (tests/test_gpu_batched.py).
+
+``drift`` gives every instance time-varying parameters, as ``OptBayesExpt(drift=...)`` does: at the end of every
+update each particle takes a Gaussian random-walk step ``x <- x + F z`` with ``F F^T = Q`` (``optbayesexpt_b200.drift``).
+``set_simulator(..., drift=...)`` lets the simulated experiment's true parameters take the same kind of step after
+every simulated measurement, so a closed loop of drifting instruments runs on the device.
 """
 import ctypes as C
 
 import numpy as np
 
 from . import _lib
+from .drift import batched_drift_factors
 from .models import DeviceModel, builtin, non_gaussian
 
 
 class BatchedOptBayesExpt:
+    """``drift``: the random-walk step every instance's cloud takes at the end of every update (after the resample
+    of the instances that resampled), or None (the default: static parameters).  It takes every form of
+    ``OptBayesExpt``'s ``drift`` -- a standard deviation, ``n_dims`` of them or an ``(n_dims, n_dims)`` covariance
+    ``Q`` -- applied to all instances, or an ``(n_instances, n_dims, n_dims)`` array with one covariance per instance
+    (per-instance standard deviations as diagonal covariances).  It is also a property: ``beng.drift = Q * dt`` takes
+    effect at the next update, in stream order and without a host synchronisation; ``beng.drift = None`` stops the
+    steps.  The weights are never changed, and a step that would leave the region of the constraint masks (such as
+    a positive noise parameter) is not taken.  The summaries and the next design therefore describe the parameters
+    at the next measurement.  The normals are Philox normals keyed by the engine seed, the instance, the particle
+    slot and the engine's count of drift steps, so no step reuses another's numbers."""
+
     def __init__(self, measurement_model, setting_values, parameter_samples, constants, n_draws=30, choke=None,
                  default_noise_std=1.0, noise_parameter_index=None, constraint_le=(), constraint_lt=(),
                  cost_of_changing_setting=None, a_param=0.98, resample_threshold=0.5, auto_resample=True,
-                 scale=True, seed=0, utility_method='variance_approx', device=None):
+                 scale=True, seed=0, utility_method='variance_approx', device=None, drift=None):
         import torch
         self._torch = torch
+        shape = tuple(parameter_samples.shape) if hasattr(parameter_samples, 'shape') else np.shape(parameter_samples)
+        # (drift is checked before the device is: (B, d, n) is all it needs)
+        drift_factors = batched_drift_factors(drift, shape[0], shape[1]) if len(shape) == 3 else None
         self._lib = _lib.require_device()
         if isinstance(measurement_model, str):
             measurement_model = builtin(measurement_model)
@@ -113,6 +133,8 @@ class BatchedOptBayesExpt:
         self._check(self._lib.obe_batch_init(self._bs(), _lib.iarr(self._noise_index),
                                              0 if self._noise_index is None else len(self._noise_index),
                                              self._stream()))
+        self._drift_step = 0              # drift steps taken: the step word of their normals
+        self._install_drift(drift, drift_factors)
 
     # ---- plumbing
     def _stream(self):
@@ -124,6 +146,45 @@ class BatchedOptBayesExpt:
     @staticmethod
     def _check(rc):
         _lib.check(rc)
+
+    def _to_device(self, a):
+        """A new float64 device tensor holding ``a``, copied in stream order without a host synchronisation."""
+        host = self._torch.from_numpy(np.ascontiguousarray(a, dtype=np.float64)).pin_memory()
+        return host.to(self._dev, non_blocking=True)
+
+    def _factor_args(self, factors):
+        """(factor_host, factor_dev tensor) of the C drift entries: a shared F by value, per-instance F on the device."""
+        if factors is None:
+            return None, None
+        if factors.ndim == 2:
+            return _lib.darr(factors.reshape(-1)), None
+        return None, self._to_device(factors)
+
+    @staticmethod
+    def _ptr(t):
+        return None if t is None else C.c_void_p(t.data_ptr())
+
+    # ---- time-varying parameters
+    @property
+    def drift(self):
+        """The random-walk step of every instance's cloud per update (see the class docstring), or None."""
+        return self._drift
+
+    @drift.setter
+    def drift(self, value):
+        self._install_drift(value, batched_drift_factors(value, self.n_instances, self.n_dims))
+
+    def _install_drift(self, value, factors):
+        self._drift = value
+        self._drift_arr, self._drift_dev = self._factor_args(factors)
+
+    def _apply_drift(self):
+        """One random-walk step of every instance's live cloud (obe_batch_drift); its moments follow on the device."""
+        self._drift_step += 1
+        ni = self._noise_index
+        self._check(self._lib.obe_batch_drift(self._bs(), self._drift_arr, self._ptr(self._drift_dev), self._mask_le,
+                                              self._mask_lt, _lib.iarr(ni), 0 if ni is None else len(ni),
+                                              self._seed_normal, self._drift_step & 0xffffffff, self._stream()))
 
     # ---- design half
     def opt_setting(self, want_utility=False, sync=True):
@@ -195,15 +256,23 @@ class BatchedOptBayesExpt:
                                                      self._mask_lt, _lib.iarr(self._noise_index),
                                                      0 if self._noise_index is None else len(self._noise_index),
                                                      self._stream()))
+        if self._drift is not None:
+            self._apply_drift()
         self.cycle += 1
 
     # ---- on-device MeasurementSimulator (obe_utils.py:8-53), SURVEY 8(f) row 4
-    def set_simulator(self, true_params, noise_level, seed=12345):
+    def set_simulator(self, true_params, noise_level, seed=12345, drift=None):
         """Install the simulated experiment of every instance: ``true_params`` (B, n_model_params) (or one
-        set for all), ``noise_level`` a scalar, one value per channel, or (B,) per instance."""
+        set for all), ``noise_level`` a scalar, one value per channel, or (B,) per instance.
+
+        ``drift``: the true parameters of every instance take one Gaussian random-walk step on the device after each
+        simulated measurement, so measurement t sees the truth after t steps (``simulator_truth()`` returns the
+        current one).  It takes the forms of the engine's ``drift`` over the model's ``n_model_params``; None (the
+        default) keeps the truths fixed.  No constraint applies to the truth."""
         torch = self._torch
         B = self.n_instances
         npm = self.model_function.n_model_params
+        sim_factors = batched_drift_factors(drift, B, npm)
         tp = np.asarray(true_params, dtype=np.float64)
         if tp.ndim == 1:
             tp = np.broadcast_to(tp[:npm], (B, npm))
@@ -218,6 +287,15 @@ class BatchedOptBayesExpt:
         else:
             self._sim_noise = _lib.darr(np.broadcast_to(nl, (self.n_channels,)), _lib.MAX_CHANNELS)
         self._sim_seed = int(seed)
+        self._sim_drift_arr, self._sim_drift_dev = self._factor_args(sim_factors)
+        self._sim_drift = drift
+        self._truth_step = 0
+
+    def simulator_truth(self):
+        """(B, n_model_params): the simulator's current true parameters of every instance."""
+        if getattr(self, '_sim_true', None) is None:
+            raise RuntimeError('call set_simulator(true_params, noise_level) first')
+        return self._sim_true.T.cpu().numpy()
 
     def simulate_measurement(self):
         """Instance b measures at the setting it chose last; the record rows are written on the device.
@@ -229,12 +307,19 @@ class BatchedOptBayesExpt:
             C.c_void_p(self._sim_true.data_ptr()), self.n_instances, self._cons_arr, self._sim_noise,
             None if self._sim_noise_dev is None else C.c_void_p(self._sim_noise_dev.data_ptr()),
             self._sim_seed, self.cycle, 1 if self._noise_index is None else 0, self._stream()))
+        if self._sim_drift is not None:
+            self._truth_step += 1
+            self._check(self._lib.obe_batch_truth_drift(
+                C.c_void_p(self._sim_true.data_ptr()), self.n_instances, self.n_instances,
+                self.model_function.n_model_params, self._sim_drift_arr, self._ptr(self._sim_drift_dev),
+                self._sim_seed, self._truth_step & 0xffffffff, self._stream()))
         return self._record
 
     def closed_loop_cycle(self, force_resample=False):
         """opt_setting -> simulated measurement -> pdf_update of every instance, without any host
         round trip (no synchronisation, no H2D/D2H): the fit_vs_obe study's inner loop
-        (demos/fit_vs_obe/fit_vs_obe_makedata.py:149-194) for all runs at once."""
+        (demos/fit_vs_obe/fit_vs_obe_makedata.py:149-194) for all runs at once.  With a ``drift`` the cloud steps at
+        the end of the update, and with a simulator ``drift`` the truth steps after the simulated measurement."""
         self.opt_setting(sync=False)
         self.simulate_measurement()
         self._update_from_record(1, self.n_channels, force_resample)

@@ -2444,6 +2444,31 @@ template <int D>
 __global__ void __launch_bounds__(OBE_UPDATE_THREADS, 1) k_brefresh(const ObeBatchArgs a) {
     obe_update_batched_body<ObeNoModel, D, OBE_SRC_NONE>(a);
 }
+// the batched random-walk drift (obe_batch_drift): the refresh body with the step as its move policy; PER: one factor
+// per instance from device memory, otherwise the shared factor of the by-value parameters
+template <int D, bool PER>
+__global__ void __launch_bounds__(OBE_UPDATE_THREADS, 1) k_bdrift(const ObeBatchArgs a, const ObeBDriftParams q) {
+    obe_update_batched_body<ObeNoModel, D, OBE_SRC_DRIFT, ObeBDrift<PER>>(a, ObeBDrift<PER>{q});
+}
+// one random-walk step of the batched simulator's true parameters (obe_batch_truth_drift): thread b moves column b
+// of the (npm, ld) SoA truth by F z, z = obe_drift_normals keyed by OBE_TRUTH_CTR / OBE_TRUTH_KEY
+__global__ void __launch_bounds__(OBE_THREADS) k_btruth_drift(double* __restrict__ truth, long long ld, long long n_inst,
+                                                              int npm, const double* __restrict__ f_dev,
+                                                              const ObeBDriftParams q) {
+    const long long b = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= n_inst) return;
+    double z[OBE_MAX_DIMS];
+    obe_drift_normals<OBE_MAX_DIMS, OBE_TRUTH_CTR, OBE_TRUTH_KEY>(b, q.seed, q.step, z);
+#pragma unroll
+    for (int j = 0; j < OBE_MAX_DIMS; ++j) {
+        if (j >= npm) break;
+        double nud = 0.0;
+#pragma unroll
+        for (int k = 0; k <= j; ++k)
+            nud = fma(f_dev ? f_dev[(b * npm + j) * npm + k] : q.f[j * (j + 1) / 2 + k], z[k], nud);
+        truth[j * ld + b] += nud;
+    }
+}
 template <class M>
 __global__ void __launch_bounds__(OBE_THREADS) k_bselect_model(const ObeBSelectArgs a) {
     obe_bselect_body<M>(a);
@@ -4266,6 +4291,82 @@ int obe_batch_select(obe_model_t m, const obe_batch_t* b, const double* settings
     // than the second evaluation for this FP64-latency-bound body)
     const size_t smem = (size_t)(OBE_TILE + k * (m->np_model > 0 ? m->np_model : 1)) * sizeof(double);
     return launch_kernel(m->f_bselect, (int)g, smem, (cudaStream_t)stream, &a);
+}
+
+// The factor arguments of the two batched drift entries: exactly one of factor_host (d*d, row-major,
+// lower-triangular, finite: packed into q.f with its non-zero rows in q.rows) and factor_dev.
+static int batch_drift_factor(const char* who, const double* factor_host, const double* factor_dev, int d,
+                              ObeBDriftParams& q) {
+    memset(&q, 0, sizeof(q));
+    if (!factor_host == !factor_dev) return obe_fail("%s: pass exactly one of factor_host and factor_dev%s", who, "");
+    q.f_dev = factor_dev;
+    if (factor_host)
+        for (int j = 0; j < d; ++j)
+            for (int k = 0; k < d; ++k) {
+                const double v = factor_host[j * d + k];
+                if (!std::isfinite(v)) return obe_fail("%s: the factor must be finite%s", who, "");
+                if (k > j && v != 0.0) return obe_fail("%s: the factor must be lower-triangular%s", who, "");
+                if (k <= j) {
+                    q.f[j * (j + 1) / 2 + k] = v;
+                    if (v != 0.0) q.rows |= 1u << j;
+                }
+            }
+    return 0;
+}
+
+int obe_batch_drift(const obe_batch_t* b, const double* factor_host, const double* factor_dev, uint32_t mask_le,
+                    uint32_t mask_lt, const int32_t* noise_index, int n_noise, uint64_t seed, uint32_t step,
+                    void* stream) {
+    if (check_batch(b)) return -1;
+    ObeBDriftParams q;
+    if (batch_drift_factor("obe_batch_drift", factor_host, factor_dev, b->d, q)) return -1;
+    if (n_noise < 0 || n_noise > OBE_MAX_CH || (n_noise > 0 && !noise_index))
+        return obe_fail("obe_batch_drift: n_noise out of range%s%s");
+    q.particles[0] = b->particles_dev[0]; q.particles[1] = b->particles_dev[1];
+    q.seed = seed; q.step = step;
+    ObeBatchArgs a;
+    fill_batch_args(b, a);
+    a.u.scale_in = 0; a.u.write_weights = 0;
+    a.u.mask_le = mask_le; a.u.mask_lt = mask_lt;
+    a.flag = nullptr;
+    for (int j = 0; j < n_noise; ++j) {
+        if (noise_index[j] < 0 || noise_index[j] >= b->d) return obe_fail("obe_batch_drift: noise_index out of range%s%s");
+        a.u.noise_idx[j] = noise_index[j]; a.u.n_noise = j + 1;
+    }
+    const bool per = factor_dev != nullptr;
+    const void* f = nullptr;
+#define OBE_BDRIFT_CASE(D) \
+    case D: f = per ? (const void*)k_bdrift<D, true> : (const void*)k_bdrift<D, false>; break;
+    switch (b->d) {
+        OBE_BDRIFT_CASE(1) OBE_BDRIFT_CASE(2) OBE_BDRIFT_CASE(3) OBE_BDRIFT_CASE(4)
+        OBE_BDRIFT_CASE(5) OBE_BDRIFT_CASE(6) OBE_BDRIFT_CASE(7) OBE_BDRIFT_CASE(8)
+        default: return obe_fail("n_params must be 1..8%s%s");
+    }
+#undef OBE_BDRIFT_CASE
+    const size_t smem = update_smem_bytes(b->d, OBE_SRC_MODEL);
+    cudaError_t e = set_max_smem(f, smem);
+    if (e != cudaSuccess) return obe_fail("cudaFuncSetAttribute(max dynamic smem): %s%s", cudaGetErrorString(e));
+    int64_t g = obe_sms();
+    if (g > b->n_inst) g = b->n_inst;
+    void* params[2] = {&a, &q};
+    e = cudaLaunchKernel(f, dim3((unsigned)g), dim3(OBE_UPDATE_THREADS), params, smem, (cudaStream_t)stream);
+    if (e != cudaSuccess) return obe_fail("launch k_bdrift: %s%s", cudaGetErrorString(e));
+    return 0;
+}
+
+int obe_batch_truth_drift(double* truth_dev, int64_t ld_true, int64_t n_inst, int n_params, const double* factor_host,
+                          const double* factor_dev, uint64_t seed, uint32_t step, void* stream) {
+    if (!truth_dev) return obe_fail("obe_batch_truth_drift: null truth%s%s");
+    if (n_inst < 1 || n_params < 1 || n_params > OBE_MAX_DIMS || ld_true < n_inst)
+        return obe_fail("obe_batch_truth_drift: need n_inst >= 1, 1 <= n_params <= 8, ld_true >= n_inst%s%s");
+    ObeBDriftParams q;
+    if (batch_drift_factor("obe_batch_truth_drift", factor_host, factor_dev, n_params, q)) return -1;
+    if (obe_sms() <= 0) return obe_fail("no CUDA device: this library has no CPU fallback%s%s");
+    q.seed = seed; q.step = step;
+    const int blocks = (int)((n_inst + OBE_THREADS - 1) / OBE_THREADS);
+    k_btruth_drift<<<blocks, OBE_THREADS, 0, (cudaStream_t)stream>>>(truth_dev, ld_true, n_inst, n_params, factor_dev, q);
+    OBE_LAUNCH_CHECK("k_btruth_drift");
+    return 0;
 }
 
 }  // extern "C"

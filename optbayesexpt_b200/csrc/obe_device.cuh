@@ -605,7 +605,8 @@ __device__ __forceinline__ void obe_update_vec(const ObeUpdateArgs& a, const dou
             for (int e = 0; e < NE; ++e) t[e] = obe_nan_to_num_fast(t[e]);
         }
     }
-    if ((SRC == OBE_SRC_NONE || BATCHED) && (a.mask_le | a.mask_lt)) {   // constraint masks: refresh pass / batched
+    // constraint masks: refresh pass / batched update (the batched drift rejects steps in its move instead)
+    if ((SRC == OBE_SRC_NONE || (BATCHED && SRC != OBE_SRC_DRIFT)) && (a.mask_le | a.mask_lt)) {
 #pragma unroll
         for (int e = 0; e < NE; ++e) {
             bool bad = false;
@@ -1076,8 +1077,12 @@ struct ObeBatchArgs {
     const int* n_list;            // ... and its length (device)
 };
 
-template <class Model, int D, int SRC>
-__device__ void obe_update_batched_body(const ObeBatchArgs& a) {
+// The move policy of the batched body.  Every kernel but the batched drift (SRC == OBE_SRC_DRIFT, ObeBDrift) runs
+// with this one, which is never called.
+struct ObeNoMove {};
+
+template <class Model, int D, int SRC, class Mv = ObeNoMove>
+__device__ void obe_update_batched_body(const ObeBatchArgs& a, const Mv& mv = Mv()) {
     constexpr int NROWS = 1 + D;
     using ST = ObeStage<NROWS>;
     constexpr int SE = ST::ELEMS, NST = ST::NSTAGES, SUB = ST::SUB, EPT = ST::EPT;
@@ -1154,6 +1159,7 @@ __device__ void obe_update_batched_body(const ObeBatchArgs& a) {
             }
             rec[ct] = v;
         }
+        if constexpr (SRC == OBE_SRC_DRIFT) mv.template load<D>(b, (int)(ii & 1), ct);
         obe_named_bar(1, OBE_CONSUMER_THREADS);
         const double invS = rec[OBE_REC_INVS];
         ObeAcc<D> acc;
@@ -1178,15 +1184,24 @@ __device__ void obe_update_batched_body(const ObeBatchArgs& a) {
                 obe_mbar_wait(full_bar + s, k & 1u);
                 const double* src = stage_base + (size_t)s * (NROWS * SE);
                 double wv[EPT], pv[D][EPT];
+                // ONE1: a stage of one element per thread (EPT == 1, D = 8).  Only the drift pass handles it; the
+                // update and refresh instantiations keep their code (DESIGN §7).
+                constexpr bool ONE1 = SRC == OBE_SRC_DRIFT && EPT == 1;
+                if constexpr (ONE1) {
+                    wv[0] = src[ct];
 #pragma unroll
-                for (int q = 0; q < EPT / 2; ++q) {
-                    const int e = 2 * (ct + q * OBE_CONSUMER_THREADS);
-                    const double2 w2 = *reinterpret_cast<const double2*>(src + e);
-                    wv[2 * q] = w2.x; wv[2 * q + 1] = w2.y;
+                    for (int j = 0; j < D; ++j) pv[j][0] = src[(1 + j) * SE + ct];
+                } else {
 #pragma unroll
-                    for (int j = 0; j < D; ++j) {
-                        const double2 p2 = *reinterpret_cast<const double2*>(src + (1 + j) * SE + e);
-                        pv[j][2 * q] = p2.x; pv[j][2 * q + 1] = p2.y;
+                    for (int q = 0; q < EPT / 2; ++q) {
+                        const int e = 2 * (ct + q * OBE_CONSUMER_THREADS);
+                        const double2 w2 = *reinterpret_cast<const double2*>(src + e);
+                        wv[2 * q] = w2.x; wv[2 * q + 1] = w2.y;
+#pragma unroll
+                        for (int j = 0; j < D; ++j) {
+                            const double2 p2 = *reinterpret_cast<const double2*>(src + (1 + j) * SE + e);
+                            pv[j][2 * q] = p2.x; pv[j][2 * q + 1] = p2.y;
+                        }
                     }
                 }
                 __syncwarp();
@@ -1196,17 +1211,19 @@ __device__ void obe_update_batched_body(const ObeBatchArgs& a) {
                     bool valid[EPT];
 #pragma unroll
                     for (int e = 0; e < EPT; ++e) {
-                        valid[e] = 2 * (ct + (e >> 1) * OBE_CONSUMER_THREADS) + (e & 1) < n_valid;
+                        valid[e] = (ONE1 ? ct : 2 * (ct + (e >> 1) * OBE_CONSUMER_THREADS) + (e & 1)) < n_valid;
 #pragma unroll
                         for (int j = 0; j < D; ++j) pe[e][j] = pv[j][e];
 #pragma unroll
                         for (int c = 0; c < OBE_MAX_CH; ++c) yge[e][c] = 0.0;
                         lke[e] = 1.0;
                     }
+                    if constexpr (SRC == OBE_SRC_DRIFT)
+                        mv.template move<D, EPT>(a.u, pe, valid, b, cb, loc, base, (int)(ii & 1), ct, n_valid);
                     obe_update_vec<Model, D, SRC, EPT, true>(a.u, pe, wv, yge, lke, valid, invS, acc, rec, te);
 #pragma unroll
                     for (int e = 0; e < EPT; ++e) tsum += te[e];
-                    if (write_weights) {
+                    if (SRC != OBE_SRC_DRIFT && write_weights) {
 #pragma unroll
                         for (int q = 0; q < EPT / 2; ++q) {
                             const int e0 = 2 * (ct + q * OBE_CONSUMER_THREADS);
@@ -1216,15 +1233,17 @@ __device__ void obe_update_batched_body(const ObeBatchArgs& a) {
                     }
                 }
             }
-            tsum = obe_warp_sum(tsum);
-            if (lane == 0) red[tile_par][cwarp] = tsum;
-            obe_named_bar(1, OBE_CONSUMER_THREADS);
-            if (ct == 0) {
-                double s = red[tile_par][0];
+            if constexpr (SRC != OBE_SRC_DRIFT) {     // (the drift leaves the weights, hence the tile sums, as they are)
+                tsum = obe_warp_sum(tsum);
+                if (lane == 0) red[tile_par][cwarp] = tsum;
+                obe_named_bar(1, OBE_CONSUMER_THREADS);
+                if (ct == 0) {
+                    double s = red[tile_par][0];
 #pragma unroll
-                for (int w = 1; w < OBE_CONSUMER_WARPS; ++w) s += red[tile_par][w];
-                a.tile_sums[b * T + t] = s;
-                tsum_s[t] = s;
+                    for (int w = 1; w < OBE_CONSUMER_WARPS; ++w) s += red[tile_par][w];
+                    a.tile_sums[b * T + t] = s;
+                    tsum_s[t] = s;
+                }
             }
         }
         // ---- instance epilogue: stats block, CDF prefix row, resample flag, next pivot
@@ -1243,6 +1262,27 @@ __device__ void obe_update_batched_body(const ObeBatchArgs& a) {
         }
         obe_named_bar(1, OBE_CONSUMER_THREADS);
         double* st = a.stats + b * OBE_STATS_LEN;
+        if constexpr (SRC == OBE_SRC_DRIFT) {
+            // only the moments move: totals, normaliser, N_eff, SUMT, NZERO, the tile sums, the prefix row and the
+            // flag stay; the pivot of the next pass becomes the drifted mean, as after a refresh
+            if (ct < NACC) {
+                double sv = accsm[0][ct];
+#pragma unroll
+                for (int w = 1; w < OBE_CONSUMER_WARPS; ++w) sv += accsm[w][ct];
+                if (ct >= 3 && ct < 3 + D) st[OBE_ST_M1 + (ct - 3)] = sv;
+                else if (ct >= 3 + D && ct < 3 + D + NM2) st[OBE_ST_M2 + (ct - 3 - D)] = sv;
+                else if (ct >= 3 + D + NM2 && a.u.noise_idx[ct - 3 - D - NM2] >= 0) st[OBE_ST_NOISE + (ct - 3 - D - NM2)] = sv;
+                accsm[0][ct] = sv;
+            }
+            obe_named_bar(1, OBE_CONSUMER_THREADS);
+            if (ct < D) {
+                st[OBE_ST_PIVOT + ct] = rec[OBE_REC_PIVOT + ct];
+                const double sumt = accsm[0][1];
+                if (sumt > 0.0) a.pivot[b * OBE_MAX_DIMS + ct] = rec[OBE_REC_PIVOT + ct] + accsm[0][3 + ct] / sumt;
+            }
+            obe_named_bar(1, OBE_CONSUMER_THREADS);
+            continue;
+        }
         if (ct < NACC) {
             double sv = accsm[0][ct];
 #pragma unroll
@@ -1428,15 +1468,19 @@ __device__ __forceinline__ void device_normals(long long slot, unsigned long lon
 // Liu-West jitter of the same seed.  Restated in oracle/obe_oracle.py:drift_normals.
 #define OBE_DRIFT_CTR 0x40000000u
 #define OBE_DRIFT_KEY 0x9E3779B97F4A7C15ull
-template <int D>
+// The random walk of the batched simulator's true parameters (obe_batch_truth_drift) draws the same way with its own
+// counter word and key: ctr = (instance_lo, instance_hi, 0x50000000 | c, step), key = seed ^ OBE_TRUTH_KEY.
+#define OBE_TRUTH_CTR 0x50000000u
+#define OBE_TRUTH_KEY 0xD1B54A32D192ED03ull
+template <int D, unsigned int CTR = OBE_DRIFT_CTR, unsigned long long KEY = OBE_DRIFT_KEY>
 __device__ __forceinline__ void obe_drift_normals(long long slot, unsigned long long seed, unsigned int epoch,
                                                   double (&z)[D]) {
-    const unsigned long long key = seed ^ OBE_DRIFT_KEY;
+    const unsigned long long key = seed ^ KEY;
 #pragma unroll
     for (int c = 0; c < (D + 3) / 4; ++c) {
         unsigned int r[4];
         philox4x32_10((unsigned int)(slot & 0xffffffffll), (unsigned int)((unsigned long long)slot >> 32),
-                      OBE_DRIFT_CTR | (unsigned int)c, epoch, (unsigned int)(key & 0xffffffffull),
+                      CTR | (unsigned int)c, epoch, (unsigned int)(key & 0xffffffffull),
                       (unsigned int)(key >> 32), r);
 #pragma unroll
         for (int h = 0; h < 2; ++h) {
@@ -1526,6 +1570,99 @@ struct ObeDrift {
                                                const double*, const double*, double (&lik)[NE]) const {
 #pragma unroll
         for (int e = 0; e < NE; ++e) lik[e] = 1.0;
+    }
+};
+
+// ---- batched drift (obe_batch_drift): the batched refresh body with ObeBDrift as its move policy ----------------
+#define OBE_DRIFT_NF (OBE_MAX_DIMS * (OBE_MAX_DIMS + 1) / 2)
+// The by-value second argument of k_bdrift<D, PER>.
+struct ObeBDriftParams {
+    double f[OBE_DRIFT_NF];   // PER == false: the F of every instance, lower triangle packed row-major
+    const double* f_dev;      // PER == true: (n_inst, d, d) row-major, one F per instance (the lower triangle is read)
+    double* particles[2];     // the two cloud buffers, moved in place (ObeBatchArgs::particles is the same memory)
+    unsigned long long seed;
+    unsigned int step;
+    unsigned int rows;        // PER == false: bit j: row j of F is not all zero
+};
+
+// The factor of the instance a CTA is on (PER == true), staged by load() next to the record; two buffers, like rec_s.
+struct ObeBDriftSmem {
+    double f[2][OBE_DRIFT_NF];
+    unsigned int nz[2][OBE_MAX_DIMS];   // row j of F is not all zero
+};
+
+// Instance b's slot i steps with obe_drift_normals(slot = (b << 32) | i): ctr = (i, b, 0x40000000 | c, step), the
+// single engine's keying with the instance in the high slot word.  A step that would leave the region of the
+// constraint masks is not taken; rows of F that are all zero are neither moved nor stored.
+template <bool PER>
+struct ObeBDrift {
+    ObeBDriftParams q;
+    __device__ static __forceinline__ ObeBDriftSmem& smem() {
+        __shared__ ObeBDriftSmem s;
+        return s;
+    }
+    template <int D>
+    __device__ __forceinline__ void load(long long b, int buf, int ct) const {
+        if constexpr (PER) {
+            if (ct < D) {
+                const double* row = q.f_dev + (b * D + ct) * D;
+                ObeBDriftSmem& s = smem();
+                bool nz = false;
+                for (int k = 0; k <= ct; ++k) {
+                    const double v = row[k];
+                    s.f[buf][ct * (ct + 1) / 2 + k] = v;
+                    nz |= v != 0.0;
+                }
+                s.nz[buf][ct] = nz ? 1u : 0u;
+            }
+        }
+    }
+    template <int D, int NE>
+    __device__ __forceinline__ void move(const ObeUpdateArgs& a, double (&p)[NE][D], const bool (&valid)[NE],
+                                         long long b, int cb, long long loc, long long base, int buf, int ct,
+                                         int n_valid) const {
+        const double* f = PER ? smem().f[buf] : q.f;
+        unsigned int rows = q.rows;
+        if constexpr (PER) {
+            rows = 0u;
+#pragma unroll
+            for (int j = 0; j < D; ++j) rows |= smem().nz[buf][j] << j;
+        }
+#pragma unroll
+        for (int e = 0; e < NE; ++e) {
+            if (!valid[e]) continue;
+            const long long slot = (b << 32) + loc + ((NE >= 2) ? 2 * (ct + (e >> 1) * OBE_CONSUMER_THREADS) + (e & 1) : ct);
+            double z[D], x[D];
+            obe_drift_normals<D>(slot, q.seed, q.step, z);
+            bool ok = true;
+#pragma unroll
+            for (int j = 0; j < D; ++j) {
+                x[j] = p[e][j];
+                if ((rows >> j) & 1u) {
+                    double nud = 0.0;
+#pragma unroll
+                    for (int k = 0; k <= j; ++k) nud = fma(f[j * (j + 1) / 2 + k], z[k], nud);
+                    x[j] += nud;
+                }
+                if (((a.mask_le >> j) & 1u) && x[j] <= 0.0) ok = false;
+                if (((a.mask_lt >> j) & 1u) && x[j] < 0.0) ok = false;
+            }
+            if (ok) {
+#pragma unroll
+                for (int j = 0; j < D; ++j) p[e][j] = x[j];
+            }
+        }
+#pragma unroll
+        for (int j = 0; j < D; ++j) {
+            if (!((rows >> j) & 1u)) continue;
+            double* row = q.particles[cb] + j * a.ld + base;
+#pragma unroll
+            for (int u = 0; u < (NE >= 2 ? NE / 2 : 1); ++u) {
+                const int e0 = (NE >= 2 ? 2 * (ct + u * OBE_CONSUMER_THREADS) : ct);
+                if (NE >= 2 && e0 + 1 < n_valid) obe_st2(row + e0, make_double2(p[2 * u][j], p[2 * u + 1][j]));
+                else if (e0 < n_valid) row[e0] = p[NE >= 2 ? 2 * u : 0][j];
+            }
+        }
     }
 };
 

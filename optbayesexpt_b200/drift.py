@@ -63,3 +63,29 @@ def drift_factor(drift, n_dims):
     if scale > 0.0 and np.linalg.eigvalsh(q)[0] < -PSD_TOL * scale:
         raise ValueError('the drift covariance must be positive semidefinite')
     return semidefinite_cholesky(q)
+
+
+def batched_drift_factors(drift, n_instances, n_dims):
+    """The factors of a batched engine's ``drift``: None for ``drift=None``, one ``(n_dims, n_dims)`` F shared by all
+    instances for every form ``drift_factor`` takes, or ``(n_instances, n_dims, n_dims)`` factors for an
+    ``(n_instances, n_dims, n_dims)`` array of covariances (per-instance standard deviations are passed as diagonal
+    covariances).  Each slice is validated like the single engine's ``drift``; ``ValueError`` names the instance."""
+    if drift is None:
+        return None
+    try:
+        a = np.array(drift, dtype=np.float64)
+    except (TypeError, ValueError) as exc:
+        raise ValueError(f'drift must be a number, {n_dims} standard deviations, an ({n_dims}, {n_dims}) covariance or '
+                         f'({n_instances}, {n_dims}, {n_dims}) covariances, got {drift!r}') from exc
+    if a.ndim < 3:
+        return drift_factor(a, n_dims)
+    if a.shape != (n_instances, n_dims, n_dims):
+        raise ValueError(f'per-instance drift covariances must have shape ({n_instances}, {n_dims}, {n_dims}), got '
+                         f'{a.shape}')
+    out = np.empty_like(a)
+    for b in range(n_instances):
+        try:
+            out[b] = drift_factor(a[b], n_dims)
+        except ValueError as exc:
+            raise ValueError(f'drift of instance {b}: {exc}') from None
+    return out
