@@ -108,8 +108,9 @@ int obe_model_compile(const char* cuda_source, const char* entry, int n_settings
  *               returning log L of the record (y_meas = its second element, aux = its third).
  * The weight factor is exp(choke * log L).  obe_update / obe_cycle / obe_update_from_y_model take such a
  * handle: y_meas carries the counts (the measured values), sigma the third element of the record
- * (trial counts, aux; may be NULL for Poisson), noise_index must be NULL.  The batched and multi-point
- * entries refuse it. */
+ * (trial counts, aux; may be NULL for Poisson), noise_index must be NULL.  The batched entries take it too
+ * (obe_batch_update, obe_batch_select, and obe_batch_simulate for "poisson" / "binomial"); only
+ * obe_update_multi refuses it. */
 int obe_model_compile_likelihood(const char* builtin_name, const char* model_source, const char* model_entry,
                                  int n_settings, int n_params, int n_model_params, int n_constants,
                                  int n_channels, const char* likelihood, const char* likelihood_source,
@@ -524,7 +525,11 @@ typedef struct obe_batch {
 int obe_batch_init(const obe_batch_t* b, const int32_t* noise_index, int n_noise, void* stream);
 /* pdf_update of every instance (obe_base.py:381-394) with its own record; use_last=1 takes each
  * instance's setting from settings_dev[:, last_idx[b]] (closed loop without a host round-trip).
- * Writes flag_dev[b] = resample decision of particlepdf.py:243-258 (or 1 when force_resample). */
+ * Writes flag_dev[b] = resample decision of particlepdf.py:243-258 (or 1 when force_resample).
+ * With a handle of obe_model_compile_likelihood(_design/_window) the record's [4:8) holds the counts (the measured
+ * values) and [8:12) the third element (binomial trial counts, a user likelihood's aux; ignored for Poisson), not
+ * sigma; the log-factorial constants are computed per instance on the device (counts are not validated there: a
+ * NaN count zeroes that instance's weights, as a NaN measurement does), and noise_index must be NULL. */
 int obe_batch_update(obe_model_t m, const obe_batch_t* b, const double* settings_dev, int64_t lds, int use_last,
                      const double* constants, const int32_t* noise_index, int n_lik_channels, int use_choke,
                      double choke, double resample_threshold, int force_resample, void* stream);
@@ -538,7 +543,9 @@ int obe_batch_refresh(const obe_batch_t* b, uint32_t mask_le, uint32_t mask_lt, 
                       void* stream);
 /* opt_setting of every instance (obe_base.py:733-756): K draws (uniforms 0..K-1 of the instance's
  * stream in this cycle), variance utility, argmax -> last_idx_dev / best_val_dev.  cost_change > 0
- * applies the sticky cost of demos/lockin/lockin_of_coil.py:135-152. */
+ * applies the sticky cost of demos/lockin/lockin_of_coil.py:135-152.  A likelihood-aware design handle
+ * (obe_model_compile_likelihood_design) reads var_noise[c] as the design aux a_c and runs obe_utility's
+ * likelihood-aware variance utility (binomial: a_c must be an integer >= 1, else refused). */
 int obe_batch_select(obe_model_t m, const obe_batch_t* b, const double* settings_dev, int64_t lds, int64_t n_settings,
                      const double* constants, int k, const double* var_noise, double cost_change, uint64_t uniform_seed,
                      uint32_t cycle, int method, int log_form, double* utility_dev, void* stream);
@@ -547,7 +554,13 @@ int obe_batch_select(obe_model_t m, const obe_batch_t* b, const double* settings
  * library's Philox/Box-Muller normals (counter b, key seed, epoch cycle), and its record row is filled in
  * on the device (setting, y, and sigma = noise level when write_sigma != 0).  true_params_dev: (np_model,
  * ld_true) SoA; noise_level: host array of n_channels, or noise_level_dev: (B) per instance.  Followed by
- * obe_batch_update(use_last = 1) a closed loop never touches the host. */
+ * obe_batch_update(use_last = 1) a closed loop never touches the host.
+ * A "poisson" handle draws y_c ~ Poisson(model_c) and ignores the noise level (may be NULL); a "binomial" handle
+ * draws y_c ~ Binomial(n, model_c) with n the noise level (the trial count), which write_sigma writes into the
+ * third element.  Counts come from Philox4x32-10 with ctr = (b, cycle, 0x60000000 | c, attempt), key seed: inversion
+ * below a mean of 10, transformed rejection (PTRS / BTRS) at or above it.  An invalid model output (lambda < 0 or
+ * not finite, p outside [0, 1] or NaN) or trial count (negative, non-integer, above 2^31) gives a NaN count.  A
+ * "user" handle is refused: it has no sampler. */
 int obe_batch_simulate(obe_model_t m, const obe_batch_t* b, const double* settings_dev, int64_t lds,
                        const double* true_params_dev, int64_t ld_true, const double* constants,
                        const double* noise_level, const double* noise_level_dev, uint64_t seed,

@@ -15,6 +15,18 @@ single engines; instance b reproduces a single engine that is fed the same unifo
 update each particle takes a Gaussian random-walk step ``x <- x + F z`` with ``F F^T = Q`` (``optbayesexpt_b200.drift``).
 ``set_simulator(..., drift=...)`` lets the simulated experiment's true parameters take the same kind of step after
 every simulated measurement, so a closed loop of drifting instruments runs on the device.
+
+``likelihood_model``, ``design_noise`` and ``design_aux`` mean what they mean for ``OptBayesExpt``: the update of every
+instance uses a Poisson, binomial or ``cuda_likelihood`` measurement likelihood, and ``design_noise='likelihood'``
+divides each instance's utility by the likelihood's own noise variance.  ``set_simulator`` then draws counts on the
+device (Poisson, or binomial with ``trials``), so a design study of counting measurements runs thousands of seeds in
+one closed loop::
+
+    beng = BatchedOptBayesExpt('lorentzian_hwhm', (np.linspace(1.5, 4.5, 241),), priors, (0.3,),
+                               likelihood_model='poisson', design_noise='likelihood')
+    beng.set_simulator(truths)                       # (B, 3) true parameters; counts ~ Poisson(model)
+    for _ in range(150):
+        beng.closed_loop_cycle()                     # no host round trip
 """
 import ctypes as C
 
@@ -22,7 +34,8 @@ import numpy as np
 
 from . import _lib
 from .drift import batched_drift_factors
-from .models import DeviceModel, builtin, non_gaussian
+from .models import DeviceModel, builtin
+from .obe_base import design_aux_array, resolve_likelihood
 
 
 class BatchedOptBayesExpt:
@@ -35,25 +48,48 @@ class BatchedOptBayesExpt:
     steps.  The weights are never changed, and a step that would leave the region of the constraint masks (such as
     a positive noise parameter) is not taken.  The summaries and the next design therefore describe the parameters
     at the next measurement.  The normals are Philox normals keyed by the engine seed, the instance, the particle
-    slot and the engine's count of drift steps, so no step reuses another's numbers."""
+    slot and the engine's count of drift steps, so no step reuses another's numbers.
+
+    ``likelihood_model`` ('poisson', 'binomial' or a ``cuda_likelihood``; None keeps the model's own, Gaussian by
+    default), ``design_noise`` ('fixed' or 'likelihood') and ``design_aux`` are ``OptBayesExpt``'s and apply to every
+    instance: instance b reproduces a single ``OptBayesExpt`` with the same likelihood fed the same counts.  With a
+    count likelihood ``pdf_update(counts, aux)`` takes the record's third element as its second argument (ignored for
+    Poisson, the trials of a binomial, the aux of a ``cuda_likelihood``), a noise parameter is refused, and a binomial
+    ``design_aux`` with ``design_noise='likelihood'`` must be an integer >= 1.  Only the variance utility is
+    implemented for batched engines."""
 
     def __init__(self, measurement_model, setting_values, parameter_samples, constants, n_draws=30, choke=None,
                  default_noise_std=1.0, noise_parameter_index=None, constraint_le=(), constraint_lt=(),
                  cost_of_changing_setting=None, a_param=0.98, resample_threshold=0.5, auto_resample=True,
-                 scale=True, seed=0, utility_method='variance_approx', device=None, drift=None):
+                 scale=True, seed=0, utility_method='variance_approx', device=None, drift=None, likelihood_model=None,
+                 design_noise='fixed', design_aux=1):
         import torch
         self._torch = torch
         shape = tuple(parameter_samples.shape) if hasattr(parameter_samples, 'shape') else np.shape(parameter_samples)
-        # (drift is checked before the device is: (B, d, n) is all it needs)
-        drift_factors = batched_drift_factors(drift, shape[0], shape[1]) if len(shape) == 3 else None
-        self._lib = _lib.require_device()
+        # (the cloud's shape, drift and the likelihood are checked before the device is)
+        if len(shape) != 3:
+            raise ValueError(f'parameter_samples must have shape (n_instances, n_dims, n_particles), got {shape}: every '
+                             'instance has a cloud of its own, whatever its likelihood (Gaussian, Poisson, binomial '
+                             'or cuda_likelihood); one (n_dims, n_particles) cloud is an OptBayesExpt')
+        drift_factors = batched_drift_factors(drift, shape[0], shape[1])
         if isinstance(measurement_model, str):
             measurement_model = builtin(measurement_model)
         if not isinstance(measurement_model, DeviceModel):
             raise TypeError('measurement_model must be a DeviceModel; there is no CPU fallback')
-        if non_gaussian(measurement_model):
-            raise ValueError('BatchedOptBayesExpt supports the Gaussian likelihood only; use OptBayesExpt for '
-                             'a Poisson, binomial or cuda_likelihood model')
+        if utility_method not in ('variance_approx',):
+            raise NotImplementedError('batched engines implement the variance utility')
+        measurement_model, self._design_lik = resolve_likelihood(measurement_model, likelihood_model, design_noise,
+                                                                 design_aux, utility_method)
+        #: 'gaussian', 'poisson', 'binomial' or a CudaLikelihood
+        self.likelihood_model = measurement_model.likelihood
+        #: 'fixed' or 'likelihood': the noise variance of the utility
+        self.design_noise = design_noise
+        if self.likelihood_model != 'gaussian' and noise_parameter_index is not None:
+            raise ValueError('a noise parameter is the sigma of the Gaussian likelihood: '
+                             f'{type(self).__name__} takes no other likelihood_model')
+        self.n_channels = measurement_model.n_channels
+        self.design_aux = design_aux
+        self._lib = _lib.require_device()
         self.model_function = measurement_model
         from .models import resolve_device
         dev = resolve_device(device)
@@ -93,7 +129,6 @@ class BatchedOptBayesExpt:
                                  self._list.data_ptr(), self._n_list.data_ptr(), self._epoch.data_ptr(),
                                  B, n, self._np, ld, d, T)
         self._model = measurement_model.handle(d)
-        self.n_channels = measurement_model.n_channels
         # setting grid (obe_base.py:174-180)
         self.allsettings = np.array([s.flatten() for s in
                                      np.meshgrid(*[np.asarray(v, dtype=np.float64) for v in setting_values],
@@ -123,8 +158,6 @@ class BatchedOptBayesExpt:
         self.cost_of_changing_setting = cost_of_changing_setting
         self.tuning_parameters = {'a_param': a_param, 'resample_threshold': resample_threshold,
                                   'auto_resample': auto_resample, 'scale': scale}
-        if utility_method not in ('variance_approx',):
-            raise NotImplementedError('batched engines implement the variance utility')
         self.utility_log_form = False
         self._seed_uniform = int(seed)
         self._seed_normal = int(np.random.default_rng(seed).integers(0, 2 ** 62))
@@ -187,6 +220,21 @@ class BatchedOptBayesExpt:
                                               self._seed_normal, self._drift_step & 0xffffffff, self._stream()))
 
     # ---- design half
+    @property
+    def design_aux(self):
+        """Per-channel aux of the likelihood-aware utility (``design_noise='likelihood'``): the planned trials of the
+        next binomial measurement, the ``aux`` of a cuda_likelihood's ``noise_var``.  It travels by value in every
+        selection launch, so reassigning it between cycles needs no synchronisation."""
+        return self._design_aux
+
+    @design_aux.setter
+    def design_aux(self, value):
+        arr = design_aux_array(value, self._design_lik, self.likelihood_model, self.n_channels)
+        if self._design_lik and self.likelihood_model == 'binomial' and not np.all(arr == np.floor(arr)):
+            raise ValueError(f'a binomial design_aux is the planned number of trials, an integer >= 1, got {value!r}')
+        self._design_aux = value
+        self._design_aux_arr = arr
+
     def opt_setting(self, want_utility=False, sync=True):
         """argmax-utility setting of every instance -> (indices (B,), settings (s, B))."""
         torch = self._torch
@@ -197,7 +245,9 @@ class BatchedOptBayesExpt:
                                                 device=self._dev)
             util_ptr = C.c_void_p(self._utility_dev.data_ptr())
         var_noise = None
-        if self._noise_index is None:
+        if self._design_lik:
+            var_noise = _lib.darr(self._design_aux_arr, _lib.MAX_CHANNELS)
+        elif self._noise_index is None:
             var_noise = _lib.darr((self.default_noise_std ** 2).reshape(-1), _lib.MAX_CHANNELS)
         cost = float(self.cost_of_changing_setting) if self.cost_of_changing_setting is not None else 0.0
         self._check(self._lib.obe_batch_select(self._model, self._bs(), C.c_void_p(self._settings_dev.data_ptr()),
@@ -221,20 +271,29 @@ class BatchedOptBayesExpt:
     def pdf_update(self, y_meas, sigma=None, settings=None, force_resample=False):
         """Bayesian update of every instance from its own measurement, then the resample of the
         instances whose N_eff dropped below the threshold.  y_meas (B, C); sigma (B, C) or scalar for
-        known-sigma models; settings (B, s) or None to use each instance's last chosen setting."""
+        known-sigma models; settings (B, s) or None to use each instance's last chosen setting.
+        With a non-Gaussian likelihood y_meas holds the counts (the measured values of a cuda_likelihood) and
+        ``sigma`` the record's third element: ignored for Poisson, ``n_trials`` for binomial, the aux of a
+        cuda_likelihood (a scalar, (B,) or (B, C)); the records are checked before anything reaches the device."""
         torch = self._torch
         B = self.n_instances
         rec = np.zeros((B, 12))
-        y = np.asarray(y_meas, dtype=np.float64).reshape(B, -1)
-        n_lik = min(self.n_channels, y.shape[1])
-        rec[:, 4:4 + n_lik] = y[:, :n_lik]
-        if self._noise_index is None:
-            if sigma is None:
-                raise ValueError('sigma is required: this engine has no noise_parameter_index (known-sigma model)')
-            sg = np.asarray(sigma, dtype=np.float64)
-            if sg.ndim == 1 and sg.shape[0] == B:
-                sg = sg.reshape(B, 1)
-            rec[:, 8:8 + n_lik] = np.broadcast_to(sg, (B, n_lik))
+        if self.likelihood_model != 'gaussian':
+            y, aux = count_record(self.likelihood_model, y_meas, sigma, B, self.n_channels)
+            n_lik = y.shape[1]
+            rec[:, 4:4 + n_lik] = y
+            rec[:, 8:8 + n_lik] = aux
+        else:
+            y = np.asarray(y_meas, dtype=np.float64).reshape(B, -1)
+            n_lik = min(self.n_channels, y.shape[1])
+            rec[:, 4:4 + n_lik] = y[:, :n_lik]
+            if self._noise_index is None:
+                if sigma is None:
+                    raise ValueError('sigma is required: this engine has no noise_parameter_index (known-sigma model)')
+                sg = np.asarray(sigma, dtype=np.float64)
+                if sg.ndim == 1 and sg.shape[0] == B:
+                    sg = sg.reshape(B, 1)
+                rec[:, 8:8 + n_lik] = np.broadcast_to(sg, (B, n_lik))
         if settings is not None:
             st = np.asarray(settings, dtype=np.float64).reshape(B, -1)
             rec[:, :st.shape[1]] = st
@@ -261,9 +320,15 @@ class BatchedOptBayesExpt:
         self.cycle += 1
 
     # ---- on-device MeasurementSimulator (obe_utils.py:8-53), SURVEY 8(f) row 4
-    def set_simulator(self, true_params, noise_level, seed=12345, drift=None):
+    def set_simulator(self, true_params, noise_level=None, seed=12345, drift=None, trials=None):
         """Install the simulated experiment of every instance: ``true_params`` (B, n_model_params) (or one
         set for all), ``noise_level`` a scalar, one value per channel, or (B,) per instance.
+
+        With a count likelihood the simulator draws counts on the device instead of adding Gaussian noise: Poisson
+        counts with mean the model output (no ``noise_level``: passing one raises), or binomial counts of ``trials``
+        trials (required: a scalar, one per channel, or (B,) per instance; integers in [0, 2^31]) with success
+        probability the model output; the trials become the record's third element.  A cuda_likelihood has no
+        sampler and raises.  An instance whose model output is invalid for the likelihood gets a NaN count.
 
         ``drift``: the true parameters of every instance take one Gaussian random-walk step on the device after each
         simulated measurement, so measurement t sees the truth after t steps (``simulator_truth()`` returns the
@@ -272,6 +337,7 @@ class BatchedOptBayesExpt:
         torch = self._torch
         B = self.n_instances
         npm = self.model_function.n_model_params
+        noise_level = simulator_noise(self.model_function.likelihood, noise_level, trials)
         sim_factors = batched_drift_factors(drift, B, npm)
         tp = np.asarray(true_params, dtype=np.float64)
         if tp.ndim == 1:
@@ -299,7 +365,7 @@ class BatchedOptBayesExpt:
 
     def simulate_measurement(self):
         """Instance b measures at the setting it chose last; the record rows are written on the device.
-        Returns the device record tensor (B, 12): [0:4) setting, [4:8) y, [8:12) sigma."""
+        Returns the device record tensor (B, 12): [0:4) setting, [4:8) y, [8:12) sigma (a binomial's trials)."""
         if getattr(self, '_sim_true', None) is None:
             raise RuntimeError('call set_simulator(true_params, noise_level) first')
         self._check(self._lib.obe_batch_simulate(
@@ -378,3 +444,56 @@ class BatchedOptBayesExpt:
         lo = b * self._np
         w = self._w[cb][lo:lo + self.n_particles].cpu().numpy()
         return w * float(self._stats[b, _lib.ST_INVS].item())
+
+
+def simulator_noise(likelihood, noise_level, trials):
+    """The per-channel / per-instance value the simulator reads (the Gaussian noise level, the binomial trials, 0 for
+    Poisson) of ``set_simulator``'s arguments; raises ValueError for an argument the likelihood does not take."""
+    if likelihood == 'gaussian':
+        if noise_level is None:
+            raise ValueError('the Gaussian simulator needs noise_level')
+        if trials is not None:
+            raise ValueError('trials applies to a binomial likelihood; the Gaussian simulator takes noise_level')
+        return noise_level
+    if not isinstance(likelihood, str):
+        raise ValueError('a cuda_likelihood has no sampler: simulate its measurements on the host and pass them to '
+                         'pdf_update')
+    if noise_level is not None:
+        raise ValueError(f'a {likelihood} simulator draws its own noise and takes no noise_level'
+                         + (' (pass trials=)' if likelihood == 'binomial' else ''))
+    if likelihood == 'poisson':
+        if trials is not None:
+            raise ValueError('trials applies to a binomial likelihood')
+        return 0.0
+    if trials is None:
+        raise ValueError('a binomial simulator needs trials: a scalar, one per channel, or one per instance')
+    n = np.asarray(trials, dtype=np.float64)
+    if not (np.all(np.isfinite(n)) and np.all(n >= 0) and np.all(n <= 2.0 ** 31) and np.all(n == np.floor(n))):
+        raise ValueError(f'trials must be integers in [0, 2^31], got {trials!r}')
+    return n
+
+
+def count_record(likelihood, y_meas, aux, n_instances, n_channels):
+    """(y (B, n_lik), third element (B, n_lik)) of the batched records of a non-Gaussian likelihood, checked as the
+    single engine checks one record: Poisson counts finite non-negative integers (aux ignored), binomial integers
+    0 <= k <= n_trials with ``aux`` the trials, a cuda_likelihood's values and aux as given (aux required).  ``aux``
+    is a scalar, (B,) or (B, C).  Raises ValueError."""
+    y = np.asarray(y_meas, dtype=np.float64).reshape(n_instances, -1)
+    n_lik = min(n_channels, y.shape[1])
+    y = y[:, :n_lik]
+    if likelihood == 'poisson':
+        if not (np.all(np.isfinite(y)) and np.all(y >= 0) and np.all(y == np.floor(y))):
+            raise ValueError('Poisson counts must be finite non-negative integers')
+        return y, np.zeros_like(y)
+    if aux is None:
+        raise ValueError('a binomial record needs n_trials' if likelihood == 'binomial'
+                         else 'a cuda_likelihood record needs its aux')
+    a = np.asarray(aux, dtype=np.float64)
+    if a.ndim == 1 and a.shape[0] == n_instances:
+        a = a.reshape(n_instances, 1)
+    a = np.array(np.broadcast_to(a if a.ndim < 2 else a[:, :n_lik], (n_instances, n_lik)))
+    if likelihood == 'binomial':
+        if not (np.all(np.isfinite(y)) and np.all(np.isfinite(a)) and np.all(y >= 0) and np.all(y <= a)
+                and np.all(y == np.floor(y)) and np.all(a == np.floor(a))):
+            raise ValueError('binomial records need integers 0 <= k <= n_trials')
+    return y, a

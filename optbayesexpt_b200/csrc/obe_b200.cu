@@ -2845,29 +2845,36 @@ static int compile_likelihood(const char* builtin_name, const char* model_source
     }
     const char* noise_type = kind == OBE_LIK_POISSON ? "ObePoissonNoise"
                              : (kind == OBE_LIK_BINOMIAL ? "ObeBinomialNoise" : "ObeUserNoise");
-    char tail[512];
+    char tail[768];
     if (design)
         snprintf(tail, sizeof(tail),
                  "OBE_DEFINE_LIK_KERNELS(ObeLikModel, %s, %d)\n"
-                 "OBE_DEFINE_DESIGN_KERNELS(ObeLikModel, %s)\n", lik_type, n_params, noise_type);
+                 "OBE_DEFINE_DESIGN_KERNELS(ObeLikModel, %s)\n"
+                 "OBE_DEFINE_LIK_BATCH_KERNELS(ObeLikModel, %s, %s, %d)\n", lik_type, n_params, noise_type, lik_type,
+                 noise_type, n_params);
     else
         snprintf(tail, sizeof(tail),
                  "OBE_DEFINE_LIK_KERNELS(ObeLikModel, %s, %d)\n"
-                 "OBE_DEFINE_GRID_KERNELS(ObeLikModel, lik)\n", lik_type, n_params);
+                 "OBE_DEFINE_GRID_KERNELS(ObeLikModel, lik)\n"
+                 "OBE_DEFINE_LIK_BATCH_KERNELS(ObeLikModel, %s, ObeFixedNoise, %d)\n", lik_type, n_params, lik_type,
+                 n_params);
     src += tail;
     std::vector<char> cubin;
     if (nvrtc_cubin(src, "obe_likelihood_model.cu", cubin, log, log_len)) return -1;
     obe_model* m = new obe_model(tmp);
     m->d = n_params; m->user = true; m->lik = kind; m->design = design ? 1 : 0;
-    const void* k[6];
-    const char* kn[6] = {"obe_k_update_lik", "obe_k_updatey_lik", "obe_k_evalp_lik", "obe_k_utility_lik",
-                         "obe_k_evals_lik", "obe_k_utility_info"};
+    const void* k[9];
+    const char* kn[9] = {"obe_k_update_lik", "obe_k_updatey_lik", "obe_k_evalp_lik", "obe_k_utility_lik",
+                         "obe_k_evals_lik", "obe_k_bupdate_lik", "obe_k_bselect_lik", "obe_k_bsim_lik",
+                         "obe_k_utility_info"};
     if (design) { kn[3] = "obe_k_utility_design"; kn[4] = "obe_k_evals_design"; }
     // (the information gain needs a known support: Poisson and binomial design handles, and user ones with a window)
-    const int nk = design && (kind != OBE_LIK_USER || window_entry) ? 6 : 5;
+    const int nk = design && (kind != OBE_LIK_USER || window_entry) ? 9 : 8;
     if (load_kernels(m, cubin, kn, k, nk)) return -1;
     m->f_update = k[0]; m->f_update_y = k[1]; m->f_evalp = k[2]; m->f_utility = k[3]; m->f_evals = k[4];
-    if (nk == 6) m->f_utility_info = k[5];
+    // (a user likelihood's simulator kernel is empty: obe_batch_simulate refuses such a handle)
+    m->f_bupdate = k[5]; m->f_bselect = k[6]; m->f_bsim = k[7];
+    if (nk == 9) m->f_utility_info = k[8];
     *out = m;
     return 0;
 }
@@ -4057,9 +4064,11 @@ int obe_batch_simulate(obe_model_t m, const obe_batch_t* b, const double* settin
                        const double* noise_level, const double* noise_level_dev, uint64_t seed, uint32_t cycle,
                        int write_sigma, void* stream) {
     if (!m || !b || !settings_dev || !true_params_dev) return obe_fail("null argument%s%s");
-    if (m->lik != OBE_LIK_GAUSS)
-        return obe_fail("obe_batch_simulate: the model handle has a non-Gaussian likelihood (only the single-cloud update takes one)%s%s");
-    if (!noise_level && !noise_level_dev) return obe_fail("simulate: need a noise level%s%s");
+    if (m->lik == OBE_LIK_USER)
+        return obe_fail("obe_batch_simulate: a user likelihood has no count sampler; simulate its measurements "
+                        "elsewhere and pass them to obe_batch_update%s%s");
+    if (m->lik != OBE_LIK_POISSON && !noise_level && !noise_level_dev)
+        return obe_fail("simulate: need a noise level (the trial counts of a binomial likelihood)%s%s");
     if (ld_true < b->n_inst) return obe_fail("simulate: ld_true < n_inst%s%s");
     if (obe_sms() <= 0) return obe_fail("no CUDA device: this library has no CPU fallback%s%s");
     ObeBSimArgs a;
@@ -4216,8 +4225,8 @@ int obe_batch_update(obe_model_t m, const obe_batch_t* b, const double* settings
                      const double* constants, const int32_t* noise_index, int n_lik_channels, int use_choke,
                      double choke, double resample_threshold, int force_resample, void* stream) {
     if (!m) return obe_fail("null model%s%s");
-    if (m->lik != OBE_LIK_GAUSS)
-        return obe_fail("obe_batch_update: the model handle has a non-Gaussian likelihood (only the single-cloud update takes one)%s%s");
+    if (m->lik != OBE_LIK_GAUSS && noise_index)
+        return obe_fail("obe_batch_update: a noise parameter needs the Gaussian likelihood%s%s");
     if (check_batch(b)) return -1;
     if (m->d != b->d) return obe_fail("model was built for a different n_params%s%s");
     if (use_last && !settings_dev) return obe_fail("use_last needs the setting grid%s%s");
@@ -4268,10 +4277,19 @@ int obe_batch_select(obe_model_t m, const obe_batch_t* b, const double* settings
                      const double* constants, int k, const double* var_noise, double cost_change, uint64_t uniform_seed,
                      uint32_t cycle, int method, int log_form, double* utility_dev, void* stream) {
     if (!m || !settings_dev) return obe_fail("null argument%s%s");
-    if (m->lik != OBE_LIK_GAUSS)
-        return obe_fail("obe_batch_select: the model handle has a non-Gaussian likelihood (only the single-cloud update takes one)%s%s");
     if (check_batch(b)) return -1;
     if (k < 1 || k > OBE_MAX_DRAWS) return obe_fail("n_draws must be 1..128 for batched engines%s%s");
+    if (m->design) {
+        if (!var_noise) return obe_fail("a likelihood-aware design handle needs the design aux in var_noise%s%s");
+        for (int c = 0; c < m->nch; ++c)
+            if (m->lik == OBE_LIK_BINOMIAL && !(var_noise[c] >= 1.0 && var_noise[c] <= 9007199254740992.0 &&
+                                                var_noise[c] == floor(var_noise[c]))) {
+                char got[64];
+                snprintf(got, sizeof(got), "%.17g", var_noise[c]);
+                return obe_fail("obe_batch_select: the binomial trial count (design aux) must be an integer >= 1, "
+                                "got %s%s", got);
+            }
+    }
     ObeBSelectArgs a;
     memset(&a, 0, sizeof(a));
     a.particles[0] = b->particles_dev[0]; a.particles[1] = b->particles_dev[1];

@@ -360,6 +360,7 @@ struct ObeUpdateEval {
 #define OBE_REC_PIVOT 12   /* [8] pivot          */
 #define OBE_REC_INVS 20
 #define OBE_REC_LEN 24
+#define OBE_REC_LCONST 24  /* [4] count likelihoods only: log-factorial constants of the record (ObeBLik) */
 
 // NE elements at once, in one basic block: the per-element chains (reciprocal refinement, the 14-deep exp
 // polynomial, ...) are independent, and written this way ptxas interleaves them, which is what hides the
@@ -1081,7 +1082,10 @@ struct ObeBatchArgs {
 // with this one, which is never called.
 struct ObeNoMove {};
 
-template <class Model, int D, int SRC, class Mv = ObeNoMove>
+// Lik: ObeGaussLik (the record's third element is sigma), or ObeBLik of a count / user likelihood (NVRTC modules only:
+// the third element is the aux, and the record's log-factorial constants are computed here, per instance, because
+// in a closed loop the counts are written on the device).
+template <class Model, int D, int SRC, class Mv = ObeNoMove, class Lik = ObeGaussLik>
 __device__ void obe_update_batched_body(const ObeBatchArgs& a, const Mv& mv = Mv()) {
     constexpr int NROWS = 1 + D;
     using ST = ObeStage<NROWS>;
@@ -1094,7 +1098,8 @@ __device__ void obe_update_batched_body(const ObeBatchArgs& a, const Mv& mv = Mv
     unsigned long long* empty_bar = full_bar + NST;
     __shared__ double red[2][OBE_CONSUMER_WARPS];
     __shared__ double accsm[OBE_CONSUMER_WARPS][OBE_NACC_MAX];
-    __shared__ double rec_s[2][OBE_REC_LEN];
+    constexpr int RECN = Lik::GAUSS ? OBE_REC_LEN : OBE_REC_LCONST + OBE_MAX_CH;
+    __shared__ double rec_s[2][RECN];
     __shared__ double tsum_s[64];
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const long long n = a.u.n;                     // real particles per instance
@@ -1142,7 +1147,7 @@ __device__ void obe_update_batched_body(const ObeBatchArgs& a, const Mv& mv = Mv
         const int cb = a.cur[b];
         double* rec = rec_s[ii & 1];
         // ---- per-instance record into shared memory
-        if (ct < OBE_REC_LEN) {
+        if (ct < RECN) {
             double v = 0.0;
             if (ct < OBE_REC_Y) {
                 if (ct < a.n_set)
@@ -1151,11 +1156,17 @@ __device__ void obe_update_batched_body(const ObeBatchArgs& a, const Mv& mv = Mv
                 v = a.rec_in[b * 12 + ct];
             } else if (ct < OBE_REC_PIVOT) {
                 const double sg = a.rec_in[b * 12 + ct];
-                v = (sg != 0.0) ? 1.0 / sg : 1.0;
+                if constexpr (Lik::GAUSS) v = (sg != 0.0) ? 1.0 / sg : 1.0;
+                else v = sg;                                       // (the aux)
             } else if (ct < OBE_REC_INVS) {
                 v = a.pivot[b * OBE_MAX_DIMS + (ct - OBE_REC_PIVOT)];
             } else if (ct == OBE_REC_INVS) {
                 v = a.u.scale_in ? a.stats[b * OBE_STATS_LEN + OBE_ST_INVS] : 1.0;
+            } else if (ct >= OBE_REC_LCONST) {
+                if constexpr (!Lik::GAUSS) {
+                    const int c = ct - OBE_REC_LCONST;
+                    v = Lik::lconst(a.rec_in[b * 12 + OBE_REC_Y + c], a.rec_in[b * 12 + OBE_REC_ISIG + c]);
+                }
             }
             rec[ct] = v;
         }
@@ -1220,7 +1231,8 @@ __device__ void obe_update_batched_body(const ObeBatchArgs& a, const Mv& mv = Mv
                     }
                     if constexpr (SRC == OBE_SRC_DRIFT)
                         mv.template move<D, EPT>(a.u, pe, valid, b, cb, loc, base, (int)(ii & 1), ct, n_valid);
-                    obe_update_vec<Model, D, SRC, EPT, true>(a.u, pe, wv, yge, lke, valid, invS, acc, rec, te);
+                    obe_update_vec<Model, D, SRC, EPT, true, false, Lik>(a.u, pe, wv, yge, lke, valid, invS, acc, rec,
+                                                                          te);
 #pragma unroll
                     for (int e = 0; e < EPT; ++e) tsum += te[e];
                     if (SRC != OBE_SRC_DRIFT && write_weights) {
@@ -1678,6 +1690,156 @@ __device__ __forceinline__ double obe_batch_uniform(unsigned long long seed, uns
     philox4x32_10(q, cycle, b, 0x0B5E0001u, (unsigned int)(seed & 0xffffffffull), (unsigned int)(seed >> 32), r);
     return obe_u53(r[0], r[1]);
 }
+
+// ---------------------------------------------------------------------------------------------
+// Count likelihoods of the batched engines (NVRTC likelihood modules only)
+// ---------------------------------------------------------------------------------------------
+// The batched simulator's counts.  Draw c of instance b in cycle t takes attempt j's two 53-bit uniforms
+// u = u53(x0, x1), v = u53(x2, x3) of Philox4x32-10 with ctr = (b, t, OBE_COUNT_CTR | c, j) and key = the simulator
+// seed.  The counter words of the other streams: the Liu-West jitter and the Gaussian simulator (device_normals)
+// call word < 2, the packed normals 0x80000000 | D, the drift 0x40000000 | c, the truth walk 0x50000000 | c (both with
+// keys of their own), the batch uniforms ctr = (q, cycle, b, 0x0B5E0001); 0x60000000 | c is none of them.
+// Below a mean of 10 the count is the inversion of u through the pmf recurrence; at or above it, Hormann's
+// transformed rejection (PTRS for Poisson, as numpy; BTRS for binomial, with p > 1/2 by symmetry), at most
+// OBE_COUNT_TRIES attempts, NaN if every one is rejected rather than an unbounded loop on a shared GPU.
+// Invalid parameters give NaN.  Non-contracted operations throughout: oracle/batched_counts.py restates it bit for bit.
+#define OBE_COUNT_CTR 0x60000000u
+#define OBE_COUNT_TRIES 64
+#define OBE_COUNT_SWITCH 10.0
+#define OBE_COUNT_MAX_TRIALS 2147483648.0
+__device__ __forceinline__ void obe_count_uniforms(unsigned long long seed, long long b, unsigned int cycle, int c,
+                                                   int attempt, double& u, double& v) {
+    unsigned int r[4];
+    philox4x32_10((unsigned int)b, cycle, OBE_COUNT_CTR | (unsigned int)c, (unsigned int)attempt,
+                  (unsigned int)(seed & 0xffffffffull), (unsigned int)(seed >> 32), r);
+    u = obe_u53(r[0], r[1]);
+    v = obe_u53(r[2], r[3]);
+}
+__device__ double obe_poisson_draw(double lam, unsigned long long seed, long long b, unsigned int cycle, int c) {
+    const double qnan = __longlong_as_double(0x7ff8000000000000ll);
+    if (!(lam >= 0.0 && lam <= 1.7976931348623157e308)) return qnan;
+    double u, v;
+    if (lam < OBE_COUNT_SWITCH) {
+        obe_count_uniforms(seed, b, cycle, c, 0, u, v);
+        double k = 0.0, p = exp(-lam), F = p;
+        while (u > F && p > 0.0) {
+            k = obe_add(k, 1.0);
+            p = obe_mul(p, obe_div(lam, k));
+            F = obe_add(F, p);
+        }
+        return k;
+    }
+    const double slam = sqrt(lam), loglam = log(lam);
+    const double bb = obe_add(0.931, obe_mul(2.53, slam));
+    const double a = obe_add(-0.059, obe_mul(0.02483, bb));
+    const double linvalpha = log(obe_add(1.1239, obe_div(1.1328, obe_sub(bb, 3.4))));
+    const double vr = obe_sub(0.9277, obe_div(3.6224, obe_sub(bb, 2.0)));
+    for (int j = 0; j < OBE_COUNT_TRIES; ++j) {
+        obe_count_uniforms(seed, b, cycle, c, j, u, v);
+        const double U = obe_sub(u, 0.5), us = obe_sub(0.5, fabs(U));
+        const double k = floor(obe_add(obe_add(obe_mul(obe_add(obe_div(obe_mul(2.0, a), us), bb), U), lam), 0.43));
+        if (us >= 0.07 && v <= vr) return k;
+        if (k < 0.0 || (us < 0.013 && v > us)) continue;
+        const double lhs = obe_sub(obe_add(log(v), linvalpha), log(obe_add(obe_div(a, obe_mul(us, us)), bb)));
+        const double rhs = obe_sub(obe_add(-lam, obe_mul(k, loglam)), lgamma(obe_add(k, 1.0)));
+        if (lhs <= rhs) return k;
+    }
+    return qnan;
+}
+__device__ double obe_binomial_draw(double n, double p, unsigned long long seed, long long b, unsigned int cycle,
+                                    int c) {
+    const double qnan = __longlong_as_double(0x7ff8000000000000ll);
+    if (!(p >= 0.0 && p <= 1.0 && n >= 0.0 && n <= OBE_COUNT_MAX_TRIALS && n == floor(n))) return qnan;
+    const bool flip = p > 0.5;
+    const double q = flip ? obe_sub(1.0, p) : p;
+    double u, v, k = qnan;
+    if (obe_mul(n, q) < OBE_COUNT_SWITCH) {
+        obe_count_uniforms(seed, b, cycle, c, 0, u, v);
+        const double r = obe_div(q, obe_sub(1.0, q));
+        double pk = exp(obe_mul(n, log1p(-q))), F = pk;
+        k = 0.0;
+        while (u > F && pk > 0.0 && k < n) {
+            k = obe_add(k, 1.0);
+            pk = obe_mul(pk, obe_div(obe_mul(r, obe_add(obe_sub(n, k), 1.0)), k));
+            F = obe_add(F, pk);
+        }
+    } else {
+        const double qq = obe_sub(1.0, q);
+        const double spq = sqrt(obe_mul(obe_mul(n, q), qq));
+        const double bb = obe_add(1.15, obe_mul(2.53, spq));
+        const double a = obe_add(obe_add(-0.0873, obe_mul(0.0248, bb)), obe_mul(0.01, q));
+        const double cc = obe_add(obe_mul(n, q), 0.5);
+        const double alpha = obe_mul(obe_add(2.83, obe_div(5.1, bb)), spq);
+        const double vr = obe_sub(0.92, obe_div(4.2, bb));
+        const double m = floor(obe_mul(obe_add(n, 1.0), q));
+        const double lpq = log(obe_div(q, qq));
+        const double h = obe_add(lgamma(obe_add(m, 1.0)), lgamma(obe_add(obe_sub(n, m), 1.0)));
+        for (int j = 0; j < OBE_COUNT_TRIES; ++j) {
+            obe_count_uniforms(seed, b, cycle, c, j, u, v);
+            const double U = obe_sub(u, 0.5), us = obe_sub(0.5, fabs(U));
+            const double kk = floor(obe_add(obe_mul(obe_add(obe_div(obe_mul(2.0, a), us), bb), U), cc));
+            if (kk < 0.0 || kk > n) continue;
+            if (us >= 0.07 && v <= vr) { k = kk; break; }
+            const double lhs = log(obe_div(obe_mul(v, alpha), obe_add(obe_div(a, obe_mul(us, us)), bb)));
+            const double lg = obe_add(lgamma(obe_add(kk, 1.0)), lgamma(obe_add(obe_sub(n, kk), 1.0)));
+            const double rhs = obe_add(obe_sub(h, lg), obe_mul(obe_sub(kk, m), lpq));
+            if (lhs <= rhs) { k = kk; break; }
+        }
+    }
+    return flip ? obe_sub(n, k) : k;
+}
+
+// The per-record side of a likelihood (Pmf of ObeLogLik): the record constant lconst(k, aux) the update subtracts,
+// and the simulator's draw (COUNTS).  A user likelihood has neither: lconst 0, no simulator.
+template <class Pmf>
+struct ObeCounts {
+    static constexpr bool COUNTS = false;
+    __device__ static __forceinline__ double lconst(double, double) { return 0.0; }
+};
+template <>
+struct ObeCounts<ObePoissonPmf> {
+    static constexpr bool COUNTS = true;
+    __device__ static __forceinline__ double lconst(double k, double) { return lgamma(obe_add(k, 1.0)); }
+    __device__ static __forceinline__ double draw(double lam, double, unsigned long long seed, long long b,
+                                                  unsigned int cycle, int c) {
+        return obe_poisson_draw(lam, seed, b, cycle, c);
+    }
+};
+template <>
+struct ObeCounts<ObeBinomialPmf> {
+    static constexpr bool COUNTS = true;
+    __device__ static __forceinline__ double lconst(double k, double n) {
+        return obe_sub(obe_sub(lgamma(obe_add(n, 1.0)), lgamma(obe_add(k, 1.0))), lgamma(obe_add(obe_sub(n, k), 1.0)));
+    }
+    __device__ static __forceinline__ double draw(double p, double n, unsigned long long seed, long long b,
+                                                  unsigned int cycle, int c) {
+        return obe_binomial_draw(n, p, seed, b, cycle, c);
+    }
+};
+
+// The likelihood of the batched update (Lik of obe_update_batched_body): ObeLogLik<Pmf> with its per-record data
+// read from the instance's record in shared memory -- the aux in the third element's slots (r_aux), the constants
+// at OBE_REC_LCONST -- instead of from a by-value ObeLikParams.
+template <class L>
+struct ObeBLik;
+template <class Pmf>
+struct ObeBLik<ObeLogLik<Pmf>> {
+    static constexpr bool GAUSS = false;
+    typedef ObeCounts<Pmf> Counts;
+    __device__ static __forceinline__ double lconst(double k, double aux) { return Counts::lconst(k, aux); }
+    template <int D, int NE, int NY>
+    __device__ __forceinline__ void operator()(const ObeUpdateArgs& a, const double (&p)[NE][D],
+                                               const double (&y)[NE][NY], const double* r_y, const double* r_aux,
+                                               double (&lik)[NE]) const {
+        ObeLogLik<Pmf> f;
+#pragma unroll
+        for (int c = 0; c < OBE_MAX_CH; ++c) {
+            f.q.aux[c] = r_aux[c];
+            f.q.lconst[c] = r_aux[OBE_REC_LCONST - OBE_REC_ISIG + c];
+        }
+        f(a, p, y, r_y, r_aux, lik);
+    }
+};
 
 // ---------------------------------------------------------------------------------------------
 // Utility over the setting grid (obe_base.py:463-489, 628-655) fused with the argmax of
@@ -2536,7 +2698,10 @@ struct ObeBSelectArgs {
     double cons[OBE_MAX_CONS];
 };
 
-template <class Model>
+// Noise: ObeFixedNoise, or a likelihood policy (NVRTC modules: var_noise[c] is then the design aux a_c), with
+// obe_utility_body's arithmetic: nu summed beside the mean in the first pass, sequentially over k, and 0 for a setting
+// where some draw is invalid for the likelihood.
+template <class Model, class Noise = ObeFixedNoise>
 __device__ void obe_bselect_body(const ObeBSelectArgs& a) {
     extern __shared__ double obe_smem[];
     double* cn_s = obe_smem;                       // [OBE_TILE]
@@ -2606,10 +2771,23 @@ __device__ void obe_bselect_body(const ObeBSelectArgs& a) {
             double y[Model::NCH], mean[Model::NCH], ss[Model::NCH];
 #pragma unroll
             for (int c = 0; c < Model::NCH; ++c) { mean[c] = 0.0; ss[c] = 0.0; }
+            bool ok = true;
+            double nus[Noise::LIK ? Model::NCH : 1];
+            if constexpr (Noise::LIK) {
+#pragma unroll
+                for (int c = 0; c < Model::NCH; ++c) nus[c] = 0.0;
+            }
             for (int k = 0; k < K; ++k) {
                 Model::eval(st, sdraw + k * Model::NP, a.cons, y);
 #pragma unroll
-                for (int c = 0; c < Model::NCH; ++c) mean[c] = obe_add(mean[c], y[c]);
+                for (int c = 0; c < Model::NCH; ++c) {
+                    mean[c] = obe_add(mean[c], y[c]);
+                    if constexpr (Noise::LIK) {
+                        const double nu = Noise::nu(y[c], var_n[c]);
+                        if constexpr (!Noise::NU_IS_Y) nus[c] = obe_add(nus[c], nu);
+                        ok = ok & Noise::ok(y[c], nu);
+                    }
+                }
             }
 #pragma unroll
             for (int c = 0; c < Model::NCH; ++c) mean[c] = obe_div(mean[c], kd);
@@ -2624,10 +2802,17 @@ __device__ void obe_bselect_body(const ObeBSelectArgs& a) {
             double u = 0.0;
 #pragma unroll
             for (int c = 0; c < Model::NCH; ++c) {
-                const double r = obe_div(obe_div(ss[c], kd), var_n[c]);
+                double r;
+                if constexpr (Noise::LIK) {
+                    const double v = Noise::finish(Noise::NU_IS_Y ? mean[c] : obe_div(nus[c], kd), var_n[c]);
+                    r = obe_design_ratio(obe_div(ss[c], kd), v);
+                } else {
+                    r = obe_div(obe_div(ss[c], kd), var_n[c]);
+                }
                 u = obe_add(u, a.log_form ? log(obe_add(1.0, r)) : r);
             }
             if (a.cost_change > 0.0) u = obe_div(u, (s == prev_choice) ? 1.0 : a.cost_change);
+            if constexpr (Noise::LIK) u = ok ? u : 0.0;
             if (a.utility) a.utility[b * a.n_settings + s] = u;
             const bool unan = (u != u), bnan = (best != best);
             if (besti < 0 || (!bnan && (unan || u > best))) { best = u; besti = s; }
@@ -2723,7 +2908,10 @@ struct ObeBSimArgs {
     double cons[OBE_MAX_CONS];
 };
 
-template <class Model>
+// Cnt: ObeCounts<void> (Gaussian noise, above), or the ObeCounts of a Poisson / binomial pmf (NVRTC modules): then
+// y_c is a count drawn with mean model_c (Poisson, noise ignored) or of noise trials with success probability model_c
+// (binomial), and write_sigma writes the noise level -- the trials -- into the record's third element.
+template <class Model, class Cnt = ObeCounts<void>>
 __device__ void obe_bsimulate_body(const ObeBSimArgs& a) {
     const long long b = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= a.n_inst) return;
@@ -2736,6 +2924,17 @@ __device__ void obe_bsimulate_body(const ObeBSimArgs& a) {
 #pragma unroll
     for (int j = 0; j < Model::NP; ++j) p[j] = a.true_pars[j * a.ld_true + b];
     Model::eval(s, p, a.cons, y);
+    if constexpr (Cnt::COUNTS) {
+        double* rec = a.record + b * 12;
+#pragma unroll
+        for (int j = 0; j < Model::NS; ++j) rec[j] = s[j];
+        for (int c = 0; c < Model::NCH; ++c) {
+            const double nl = a.noise_dev ? a.noise_dev[b] : a.noise[c];
+            rec[4 + c] = Cnt::draw(y[c], nl, a.seed, b, a.cycle, c);
+            if (a.write_sigma) rec[8 + c] = nl;
+        }
+        return;
+    }
     device_normals<NCH>(b, a.seed, a.cycle, z);
     double* rec = a.record + b * 12;
 #pragma unroll
@@ -2921,7 +3120,8 @@ struct ObeNoModel {
     }
 
 // A model with a non-Gaussian likelihood LIK (compiled by NVRTC per handle): the model-evaluating update, the update
-// from a supplied y_model, and the model evaluation over the cloud.  No batched or multi-point kernels.
+// from a supplied y_model, and the model evaluation over the cloud.  No multi-point kernel; the batched ones are
+// OBE_DEFINE_LIK_BATCH_KERNELS.
 #define OBE_DEFINE_LIK_KERNELS(MODEL, LIK, D)                                                                  \
     extern "C" __global__ void __launch_bounds__(OBE_UPDATE_THREADS, 1) obe_k_update_lik(const ObeUpdateArgs a, \
                                                                                          const ObeLikParams q) { \
@@ -2933,6 +3133,24 @@ struct ObeNoModel {
     }                                                                                                          \
     extern "C" __global__ void __launch_bounds__(OBE_THREADS) obe_k_evalp_lik(const ObeEvalArgs a) {           \
         obe_eval_params_body<MODEL, D>(a);                                                                     \
+    }
+
+// The batched engine of a non-Gaussian likelihood LIK (compiled by NVRTC per handle, beside OBE_DEFINE_LIK_KERNELS):
+// the update reads the record's third element as the aux, the selection runs NOISE (ObeFixedNoise for a plain handle,
+// the likelihood's policy for a design handle), the simulator draws counts (empty for a user likelihood).
+template <class Model, class L>
+__device__ __forceinline__ void obe_bsim_lik_entry(const ObeBSimArgs& a) {
+    if constexpr (ObeBLik<L>::Counts::COUNTS) obe_bsimulate_body<Model, typename ObeBLik<L>::Counts>(a);
+}
+#define OBE_DEFINE_LIK_BATCH_KERNELS(MODEL, LIK, NOISE, D)                                                      \
+    extern "C" __global__ void __launch_bounds__(OBE_UPDATE_THREADS, 1) obe_k_bupdate_lik(const ObeBatchArgs a) { \
+        obe_update_batched_body<MODEL, D, OBE_SRC_MODEL, ObeNoMove, ObeBLik<LIK>>(a);                           \
+    }                                                                                                          \
+    extern "C" __global__ void __launch_bounds__(OBE_THREADS) obe_k_bselect_lik(const ObeBSelectArgs a) {       \
+        obe_bselect_body<MODEL, NOISE>(a);                                                                     \
+    }                                                                                                          \
+    extern "C" __global__ void __launch_bounds__(OBE_THREADS) obe_k_bsim_lik(const ObeBSimArgs a) {             \
+        obe_bsim_lik_entry<MODEL, LIK>(a);                                                                     \
     }
 
 // The utility of a likelihood-aware design (design_noise='likelihood'): var_noise[c] is the design aux a_c and NOISE

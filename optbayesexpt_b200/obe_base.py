@@ -77,6 +77,44 @@ def _information_gain_problem(likelihood, design_lik, n_channels, aux):
     return None
 
 
+def resolve_likelihood(measurement_model, likelihood_model, design_noise, design_aux, utility_method):
+    """(model variant, likelihood-aware design?) of an engine built with ``likelihood_model`` / ``design_noise`` /
+    ``design_aux`` (see :class:`OptBayesExpt`); raises ValueError for a combination no engine runs."""
+    if likelihood_model is not None:
+        measurement_model = measurement_model.with_likelihood(likelihood_model)
+    if design_noise not in DESIGN_NOISES:
+        raise ValueError(f'design_noise must be one of {list(DESIGN_NOISES)}, got {design_noise!r}')
+    # the likelihood-aware utility kernel runs only for a non-Gaussian likelihood
+    design_lik = design_noise == 'likelihood' and measurement_model.likelihood != 'gaussian'
+    if design_lik:
+        if utility_method == 'full_kld_utility':
+            raise ValueError("design_noise='likelihood' does not apply to full_kld_utility: its noise samples "
+                             'are Gaussian draws')
+        if measurement_model.likelihood == 'binomial' and design_aux is None:
+            raise ValueError("design_noise='likelihood' with a binomial likelihood needs design_aux, the planned "
+                             'number of trials of the next measurement')
+        measurement_model = measurement_model.with_likelihood(measurement_model.likelihood, 'likelihood')
+    elif measurement_model.design_noise != 'fixed':
+        measurement_model = measurement_model.with_likelihood(measurement_model.likelihood)
+    return measurement_model, design_lik
+
+
+def design_aux_array(value, design_lik, likelihood, n_channels):
+    """The per-channel array of a ``design_aux`` value (see :class:`OptBayesExpt`); raises ValueError."""
+    if value is None:
+        if design_lik and likelihood == 'binomial':
+            raise ValueError("design_noise='likelihood' with a binomial likelihood needs design_aux")
+        return np.ones(n_channels)
+    arr = np.asarray(value, dtype=np.float64).reshape(-1)
+    if arr.size == 1:
+        arr = np.full(n_channels, arr[0])
+    if arr.size != n_channels:
+        raise ValueError(f'design_aux needs a scalar or {n_channels} values, got {arr.size}')
+    if not (np.all(np.isfinite(arr)) and np.all(arr > 0)):
+        raise ValueError(f'design_aux must be finite and > 0, got {value!r}')
+    return arr
+
+
 class OptBayesExpt(ParticlePDF):
     """Sequential Bayesian experiment design (obe_base.py:21-272).
 
@@ -144,24 +182,10 @@ class OptBayesExpt(ParticlePDF):
             raise TypeError(f'{type(self).__name__} overrides likelihood() in Python, which the update kernel cannot '
                             'run: pass likelihood_model=\'poisson\' | \'binomial\' | '
                             'optbayesexpt_b200.cuda_likelihood(source, entry) instead')
-        if likelihood_model is not None:
-            measurement_model = measurement_model.with_likelihood(likelihood_model)
-        if design_noise not in DESIGN_NOISES:
-            raise ValueError(f'design_noise must be one of {list(DESIGN_NOISES)}, got {design_noise!r}')
+        measurement_model, self._design_lik = resolve_likelihood(measurement_model, likelihood_model, design_noise,
+                                                                 design_aux, utility_method)
         #: 'fixed' or 'likelihood': the noise variance of the utility (see the class documentation)
         self.design_noise = design_noise
-        # the likelihood-aware utility kernel runs only for a non-Gaussian likelihood
-        self._design_lik = design_noise == 'likelihood' and measurement_model.likelihood != 'gaussian'
-        if self._design_lik:
-            if utility_method == 'full_kld_utility':
-                raise ValueError("design_noise='likelihood' does not apply to full_kld_utility: its noise samples "
-                                 'are Gaussian draws')
-            if measurement_model.likelihood == 'binomial' and design_aux is None:
-                raise ValueError("design_noise='likelihood' with a binomial likelihood needs design_aux, the planned "
-                                 'number of trials of the next measurement')
-            measurement_model = measurement_model.with_likelihood(measurement_model.likelihood, 'likelihood')
-        elif measurement_model.design_noise != 'fixed':
-            measurement_model = measurement_model.with_likelihood(measurement_model.likelihood)
         if utility_method == 'information_gain':
             problem = _information_gain_problem(measurement_model.likelihood, self._design_lik,
                                                 measurement_model.n_channels, design_aux)
@@ -1072,18 +1096,7 @@ class OptBayesExpt(ParticlePDF):
 
     @design_aux.setter
     def design_aux(self, value):
-        if value is None:
-            if self._design_lik and self.likelihood_model == 'binomial':
-                raise ValueError("design_noise='likelihood' with a binomial likelihood needs design_aux")
-            arr = np.ones(self.n_channels)
-        else:
-            arr = np.asarray(value, dtype=np.float64).reshape(-1)
-            if arr.size == 1:
-                arr = np.full(self.n_channels, arr[0])
-            if arr.size != self.n_channels:
-                raise ValueError(f'design_aux needs a scalar or {self.n_channels} values, got {arr.size}')
-            if not (np.all(np.isfinite(arr)) and np.all(arr > 0)):
-                raise ValueError(f'design_aux must be finite and > 0, got {value!r}')
+        arr = design_aux_array(value, self._design_lik, self.likelihood_model, self.n_channels)
         if getattr(self, '_utility_code', None) == 4 and self.likelihood_model == 'binomial':
             problem = _information_gain_aux_problem(arr)
             if problem:
